@@ -13,6 +13,9 @@
  *                         (tagger.py:68-78 = sentence_lookup_as_begin_index + beam_search).
  *   lt_lattice / lt_beam  the same two stages on buffers already resident in HBM
  *                         (dictionary/lookup.py:344-369 ; beam/beam.py:5-61).
+ *   lt_pathset_eval    <- the score classes' `evaluate(seq)` hooks (beam/score_funcs.py) and
+ *                         SimpleTrigramEncoder.encode_sequence (features/feature.py:62-68) on given paths.
+ *   lt_perceptron_delta <- the trainer's epoch (trainer/train.py:61-65): phi(gold) - phi(predicted).
  *
  * Plain pointers and sizes only.  No function throws; each returns LT_OK or an LT_ERR_* code and
  * lt_last_error() returns the message of the calling thread's last failure.
@@ -27,7 +30,7 @@
 extern "C" {
 #endif
 
-#define LT_ABI_VERSION 3
+#define LT_ABI_VERSION 4
 
 /* return codes */
 #define LT_OK            0
@@ -299,6 +302,37 @@ int  lt_batch_timings(lt_batch* batch, lt_timings* out);
  * While they are recorded BETWEEN the kernels of a batch, the kernels are launched one strictly after the other;
  * without them each kernel is a programmatic dependent launch whose prologue overlaps its predecessor's tail.   */
 int  lt_batch_set_stage_timing(lt_batch* batch, int32_t on);
+
+/* Word paths given by the caller (a gold analysis, candidates from elsewhere), device-resident, tied to one
+ * lt_tables.  Path p is edges[path_off[p] .. path_off[p+1]), in order, BOS / EOS left out (path_off has
+ * n_paths + 1 entries, path_off[0] = 0).  Every edge is LT_EDGE_EXPLICIT: its strings 3*rule, 3*rule+1,
+ * 3*rule+2 of (str_chars, str_off) are word, morph0 and morph1 (empty when there is none), as in
+ * lt_lattice_import; they are hashed once, here.  Spans, Word.len and tags need not be anything the search
+ * could produce (tag ids below n_tags). */
+typedef struct lt_pathset lt_pathset;
+int  lt_pathset_create(lt_tables* tables, int32_t n_paths, const lt_edge* edges, const int64_t* path_off,
+                       const uint16_t* str_chars, const int64_t* str_off, int64_t n_strings, lt_pathset** out);
+void lt_pathset_destroy(lt_pathset* paths);
+
+/* scores[p] = the score of path p under the tables' score program, bit for bit what the beam computes for
+ * the path (BeamScoreFunctions over every transition, Sequence.add in word order; EOS adds nothing).
+ * With feat_off != NULL also the features of trigram scorer `func` that fire (SimpleTrigramEncoder.
+ * encode_sequence): word w (index over all words of the set) has feat_idx[feat_off[w] .. feat_off[w+1])
+ * (feat_off: n_words + 1 entries), indices in lt_tables_desc feature order, by template.  9 * n_words
+ * always suffices for feat_cap.  `func` is read only with feat_off.  Runs on the batch's stream; synchronous. */
+int  lt_pathset_eval(lt_batch* batch, const lt_pathset* paths, int32_t func, double* scores,
+                     int64_t* feat_off, int32_t* feat_idx, int64_t feat_cap);
+
+/* One perceptron step against the best paths of the batch's last lt_tag_batch_host / lt_beam, with gold path
+ * s for sentence s (gold->n_paths = the batch's sentences).  Sentence s differs when its status is not
+ * LT_SENT_OK or its best path is not gold path s word for word on (b, e, morph0, morph1, tag0, tag1);
+ * Word.len and is_l are not compared.  For every sentence that differs: delta += phi(gold) - phi(best), the
+ * second term only when the status is LT_SENT_OK; phi = counts of trigram scorer func's features.
+ *   delta     out, n_delta = lt_tables_desc.n_feat counts in desc order (exact integers)
+ *   differs   out, one flag per sentence;  n_differ  out, sentences that differ
+ * The count buffer belongs to the tables: no other lt_perceptron_delta on the same tables may run meanwhile. */
+int  lt_perceptron_delta(lt_batch* batch, const lt_pathset* gold, int32_t func, int64_t* delta, int64_t n_delta,
+                         uint8_t* differs, int64_t* n_differ);
 
 #ifdef __cplusplus
 }

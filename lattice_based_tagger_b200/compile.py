@@ -212,6 +212,7 @@ class CompiledTables:
             raise UnsupportedScoreFunction('at most %d score functions are supported' % _native.LT_MAX_FUNCS)
         prog = (_native.lt_func * max(1, len(funcs)))()
         self._weight_source = []
+        self._desc_sources = None
         self._funcs = funcs
         strings = _StringTable()
         feat_func, feat_tmpl, feat_s, feat_a, feat_w = [], [], [], [], []
@@ -292,6 +293,7 @@ class CompiledTables:
         desc.fstr_chars = _native.ptr(units)
         desc.fstr_off = _native.ptr(offsets)
         desc.n_feat = n_feat
+        self.n_desc = n_feat
         desc.feat_func = _native.ptr(a_func)
         desc.feat_template = _native.ptr(a_tmpl)
         desc.feat_s = _native.ptr(a_s)
@@ -375,6 +377,17 @@ class CompiledTables:
             feat_s.append(np.stack([cols['s0'][keep], cols['s1'][keep], cols['s2'][keep]], axis=1).astype(np.int32))
             feat_a.append(np.stack([np.where(ok, cols['a0'], 0)[keep], np.where(ok, cols['a1'], 0)[keep]], axis=1).astype(np.int32))
             feat_w.append(weights)
+
+    def desc_sources(self):
+        """Per feature of `lt_tables_desc` (the order of device feature indices and of a perceptron delta):
+        (index of its scorer in the score program, its `feature_dic` index)."""
+        if self._desc_sources is None:
+            funcs = [np.full(len(source), f, dtype=np.int64) for f, source in self._weight_source]
+            if funcs:
+                self._desc_sources = (np.concatenate(funcs), np.concatenate([source for _, source in self._weight_source]))
+            else:
+                self._desc_sources = (np.zeros(0, dtype=np.int64), np.zeros(0, dtype=np.int64))
+        return self._desc_sources
 
     def update_weights(self):
         """Write the scorers' CURRENT `coefficients` into the device tables in place (same features, new

@@ -17,6 +17,7 @@
 #include "beam.cuh"
 #include "hash.cuh"
 #include "lattice.cuh"
+#include "paths.cuh"
 #include "scan.cuh"
 #include "tables.cuh"
 
@@ -82,6 +83,10 @@ struct lt_tables {
     std::vector<unsigned char> dense_host;
     uint32_t* d_feat_dst = nullptr;
     double* d_weights = nullptr;
+    // path sets (paths.cuh): a feature hit is a slot of the hashed table or feat_slots + a dense offset; per hit the
+    // desc index of its feature, and the perceptron's count per hit — both made on first use
+    int32_t* d_hit_feat = nullptr;
+    unsigned long long* d_counts = nullptr;
     // feature table extent and the device's L2 persistence limits (LT_L2_PERSIST, see launch_beam)
     size_t feat_bytes = 0;
     int l2_bytes = 0, l2_persist_max = 0, l2_window_max = 0;
@@ -171,6 +176,8 @@ extern "C" void lt_tables_destroy(lt_tables* t) {
     for (void* p : t->allocations) cudaFree(p);
     if (t->d_feat_dst) cudaFree(t->d_feat_dst);
     if (t->d_weights) cudaFree(t->d_weights);
+    if (t->d_hit_feat) cudaFree(t->d_hit_feat);
+    if (t->d_counts) cudaFree(t->d_counts);
     delete t;
 }
 
@@ -461,6 +468,9 @@ struct lt_batch {
     DevBuf edges, trail, path_tmp, path_out, counters, ctl, order, retry;
     DevBuf kb_tmp, kb_out, kb_len, kb_off, kb_scores, kb_count;      // all survivors (lt_beam_kbest)
     DevBuf imp;                    // string hashes of an imported lattice (lt_lattice_import)
+    DevBuf pth_ch, pth_ha, pth_hb;               // lt_perceptron_delta: syllables and prefix hashes of the batch's sentences
+    DevBuf pth_scores, pth_feat, pth_nfeat;      // lt_pathset_eval results
+    DevBuf pc_delta, pc_differs, pc_count;       // lt_perceptron_delta results
     bool imported = false;
     const uint16_t* d_text = nullptr;
     const int32_t* d_sent_off = nullptr;
@@ -538,6 +548,14 @@ static int32_t unit_limit(const lt_tables* t) {
 
 extern "C" int32_t lt_tables_max_sentence_units(const lt_tables* t) { return t ? unit_limit(t) : 0; }
 
+// where each input feature's weight lives (feat_dst) on the device, uploaded on first use
+static int upload_feat_dst(lt_tables* t) {
+    if (t->d_feat_dst || t->feat_dst.empty()) return LT_OK;
+    CU(cudaMalloc(reinterpret_cast<void**>(&t->d_feat_dst), t->feat_dst.size() * 4));
+    CU(cudaMemcpy(t->d_feat_dst, t->feat_dst.data(), t->feat_dst.size() * 4, cudaMemcpyHostToDevice));
+    return LT_OK;
+}
+
 // New weights for the features the tables were built with (the trainer's epoch: same features, new
 // coefficients) — written in place: a scatter into the hashed table's weight fields and a rewrite of the small
 // dense blocks.  No table is rebuilt.  The caller must not have a batch in flight on these tables.
@@ -547,11 +565,8 @@ extern "C" int lt_tables_update_weights(lt_tables* t, const double* weights, int
         return fail(LT_ERR_INVALID, "the tables were built with %zu features, %lld weights given", t->feat_dst.size(), (long long)n_weights);
     ON_DEVICE(t->device);
     if (n_weights == 0) return LT_OK;
-    if (!t->d_feat_dst) {
-        CU(cudaMalloc(reinterpret_cast<void**>(&t->d_feat_dst), (size_t)n_weights * 4));
-        CU(cudaMalloc(reinterpret_cast<void**>(&t->d_weights), (size_t)n_weights * 8));
-        CU(cudaMemcpy(t->d_feat_dst, t->feat_dst.data(), (size_t)n_weights * 4, cudaMemcpyHostToDevice));
-    }
+    if (int rc = upload_feat_dst(t)) return rc;
+    if (!t->d_weights) CU(cudaMalloc(reinterpret_cast<void**>(&t->d_weights), (size_t)n_weights * 8));
     CU(cudaMemcpy(t->d_weights, weights, (size_t)n_weights * 8, cudaMemcpyHostToDevice));
     const unsigned grid = (unsigned)std::min<int64_t>((n_weights + 255) / 256, (int64_t)t->sm_count * 16);
     LT_LAUNCH(scatter_weights, grid, 256, 0, (cudaStream_t) nullptr, const_cast<FeatSlot*>(t->dev.feat), t->d_feat_dst, t->d_weights, n_weights);
@@ -598,7 +613,8 @@ extern "C" void lt_batch_destroy(lt_batch* b) {
     DevBuf* bufs[] = {&b->text, &b->sent_off, &b->pos, &b->scan_tmp, &b->sent_len, &b->sent_edges, &b->status,
                       &b->path_len, &b->path_off, &b->scores, &b->edges, &b->trail, &b->path_tmp, &b->path_out,
                       &b->counters, &b->ctl, &b->order, &b->retry, &b->kb_tmp, &b->kb_out, &b->kb_len, &b->kb_off,
-                      &b->kb_scores, &b->kb_count, &b->imp};
+                      &b->kb_scores, &b->kb_count, &b->imp, &b->pth_ch, &b->pth_ha, &b->pth_hb, &b->pth_scores,
+                      &b->pth_feat, &b->pth_nfeat, &b->pc_delta, &b->pc_differs, &b->pc_count};
     for (DevBuf* x : bufs)
         if (x->p) cudaFree(x->p);
     for (auto& e : b->ev)
@@ -1506,5 +1522,219 @@ extern "C" int lt_batch_timings(lt_batch* b, lt_timings* out) {
     ms(8, 0, &out->ms_h2d);
     ms(7, 9, &out->ms_d2h);
     ms(8, 9, &out->ms_total);
+    return LT_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// path sets: scoring / featurizing given paths, the perceptron step (paths.cuh)
+// ------------------------------------------------------------------------------------------------
+struct lt_pathset {
+    lt_tables* tables = nullptr;
+    int device = 0;
+    int32_t n_paths = 0;
+    int64_t n_words = 0;
+    int64_t* d_off = nullptr;
+    lt_edge* d_edges = nullptr;
+    H2* d_hashes = nullptr;
+};
+
+extern "C" void lt_pathset_destroy(lt_pathset* p) {
+    if (!p) return;
+    DeviceGuard guard(p->device);      // (the tables may be gone already)
+    if (p->d_off) cudaFree(p->d_off);
+    if (p->d_edges) cudaFree(p->d_edges);
+    if (p->d_hashes) cudaFree(p->d_hashes);
+    delete p;
+}
+
+extern "C" int lt_pathset_create(lt_tables* t, int32_t n_paths, const lt_edge* edges, const int64_t* path_off,
+                                 const uint16_t* str_chars, const int64_t* str_off, int64_t n_strings, lt_pathset** out) {
+    if (!t || !out || !path_off || n_paths < 0 || n_strings < 0) return fail(LT_ERR_INVALID, "bad argument");
+    *out = nullptr;
+    if (path_off[0] != 0) return fail(LT_ERR_INVALID, "path_off[0] must be 0");
+    for (int32_t p = 0; p < n_paths; ++p)
+        if (path_off[p + 1] < path_off[p]) return fail(LT_ERR_INVALID, "path_off is not monotone at %d", p);
+    const int64_t n_words = path_off[n_paths];
+    if (n_words > 0 && !edges) return fail(LT_ERR_INVALID, "null edge pointer");
+    if (n_strings % 3 != 0 || (n_strings > 0 && (!str_chars || !str_off))) return fail(LT_ERR_INVALID, "strings come in (word, morph0, morph1) triples");
+    if (n_strings > 0 && str_off[0] < 0) return fail(LT_ERR_INVALID, "str_off[0] is negative");
+    const int n_tags = t->dev.n_tags;
+    for (int64_t w = 0; w < n_words; ++w) {
+        const lt_edge& ed = edges[w];
+        if (!(ed.flags & LT_EDGE_EXPLICIT)) return fail(LT_ERR_INVALID, "word %lld is not LT_EDGE_EXPLICIT", (long long)w);
+        if ((int64_t)ed.rule * 3 + 2 >= n_strings) return fail(LT_ERR_INVALID, "word %lld: string index out of range", (long long)w);
+        if (ed.tag0 >= n_tags || (ed.tag1 != LT_NO_TAG && ed.tag1 >= n_tags)) return fail(LT_ERR_INVALID, "word %lld: tag id out of range", (long long)w);
+    }
+    std::vector<H2> hashes((size_t)n_strings);
+    for (int64_t i = 0; i < n_strings; ++i) {
+        if (str_off[i + 1] < str_off[i]) return fail(LT_ERR_INVALID, "str_off is not monotone at %lld", (long long)i);
+        hashes[i] = hash_units(str_chars + str_off[i], str_off[i + 1] - str_off[i]);
+    }
+    ON_DEVICE(t->device);
+    lt_pathset* p = new lt_pathset();
+    p->tables = t;
+    p->device = t->device;
+    p->n_paths = n_paths;
+    p->n_words = n_words;
+    auto put = [&](void** dst, const void* src, size_t bytes) -> cudaError_t {
+        cudaError_t e = cudaMalloc(dst, std::max<size_t>(bytes, 16));
+        if (e == cudaSuccess && bytes) e = cudaMemcpy(*dst, src, bytes, cudaMemcpyHostToDevice);
+        return e;
+    };
+    cudaError_t e = put(reinterpret_cast<void**>(&p->d_off), path_off, (size_t)(n_paths + 1) * 8);
+    if (e == cudaSuccess) e = put(reinterpret_cast<void**>(&p->d_edges), edges, (size_t)n_words * sizeof(lt_edge));
+    if (e == cudaSuccess) e = put(reinterpret_cast<void**>(&p->d_hashes), hashes.data(), hashes.size() * sizeof(H2));
+    if (e != cudaSuccess) {
+        lt_pathset_destroy(p);
+        return fail(LT_ERR_CUDA, "path set upload failed: %s", cudaGetErrorString(e));
+    }
+    *out = p;
+    return LT_OK;
+}
+
+static int check_trigram_func(const lt_tables* t, int32_t func) {
+    if (func < 0 || func >= t->dev.n_funcs || t->dev.funcs[func].kind != LT_FUNC_TRIGRAM)
+        return fail(LT_ERR_INVALID, "func %d is not an LT_FUNC_TRIGRAM scorer", func);
+    return LT_OK;
+}
+
+// hits: slots of the hashed table, then the dense blocks' doubles
+static uint32_t feat_slots(const lt_tables* t) { return (uint32_t)(t->dev.feat_mask + 1); }
+static size_t n_hits(const lt_tables* t) {
+    return (size_t)feat_slots(t) + (size_t)t->dev.n_tri * (size_t)dense_block_bytes(t->dev.n_tags) / 8;
+}
+
+static unsigned warp_grid(const lt_tables* t, int64_t n_warps) {
+    return (unsigned)std::max<int64_t>(1, std::min<int64_t>((n_warps + 7) / 8, (int64_t)t->sm_count * 8));
+}
+
+extern "C" int lt_pathset_eval(lt_batch* b, const lt_pathset* paths, int32_t func, double* scores, int64_t* feat_off,
+                               int32_t* feat_idx, int64_t feat_cap) {
+    if (!b || !paths) return fail(LT_ERR_INVALID, "null argument");
+    if (paths->tables != b->tables) return fail(LT_ERR_INVALID, "the path set belongs to other tables");
+    if (paths->n_paths > 0 && !scores) return fail(LT_ERR_INVALID, "null output pointer");
+    lt_tables* t = b->tables;
+    const bool want_feat = feat_off != nullptr;
+    if (want_feat) {
+        if (int rc = check_trigram_func(t, func)) return rc;
+        if (feat_cap < 0 || (feat_cap > 0 && !feat_idx)) return fail(LT_ERR_INVALID, "bad feature buffer");
+    }
+    ON_DEVICE(t->device);
+    cudaStream_t st = b->own_stream;
+    const int64_t nw = paths->n_words;
+    if (int rc = ensure(b->pth_scores, (size_t)std::max(1, paths->n_paths) * 8)) return rc;
+    if (want_feat) {
+        if (!t->d_hit_feat) {
+            std::vector<int32_t> inv(n_hits(t), -1);
+            for (size_t i = 0; i < t->feat_dst.size(); ++i) {
+                const uint32_t d = t->feat_dst[i];
+                if (d != kDstNone) inv[(d & kDstDense) ? feat_slots(t) + (d & ~kDstDense) : d] = (int32_t)i;
+            }
+            CU(cudaMalloc(reinterpret_cast<void**>(&t->d_hit_feat), inv.size() * 4));
+            CU(cudaMemcpy(t->d_hit_feat, inv.data(), inv.size() * 4, cudaMemcpyHostToDevice));
+        }
+        if (int rc = ensure(b->pth_feat, (size_t)std::max<int64_t>(1, nw) * 9 * 4)) return rc;
+        if (int rc = ensure(b->pth_nfeat, (size_t)std::max<int64_t>(1, nw))) return rc;
+    }
+    PathEvalArgs A{};
+    A.edges = paths->d_edges;
+    A.off = paths->d_off;
+    A.hashes = paths->d_hashes;
+    A.n_paths = paths->n_paths;
+    A.func = want_feat ? func : -1;
+    A.scores = static_cast<double*>(b->pth_scores.p);
+    A.feat = want_feat ? static_cast<int32_t*>(b->pth_feat.p) : nullptr;
+    A.nfeat = static_cast<uint8_t*>(b->pth_nfeat.p);
+    A.hit_feat = t->d_hit_feat;
+    if (paths->n_paths > 0) {
+        LT_LAUNCH(path_eval_kernel, warp_grid(t, paths->n_paths), 256, 0, st, t->dev, A);
+        CU(cudaGetLastError());
+        b->launches += 1;
+        CU(cudaMemcpyAsync(scores, A.scores, (size_t)paths->n_paths * 8, cudaMemcpyDeviceToHost, st));
+    }
+    std::vector<int32_t> feat;
+    std::vector<uint8_t> nfeat;
+    if (want_feat && nw > 0) {
+        feat.resize((size_t)nw * 9);
+        nfeat.resize((size_t)nw);
+        CU(cudaMemcpyAsync(feat.data(), A.feat, feat.size() * 4, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(nfeat.data(), A.nfeat, nfeat.size(), cudaMemcpyDeviceToHost, st));
+    }
+    CU(cudaStreamSynchronize(st));
+    if (want_feat) {
+        int64_t total = 0;
+        for (int64_t w = 0; w < nw; ++w) total += nfeat[(size_t)w];
+        if (total > feat_cap) return fail(LT_ERR_CAPACITY, "feature buffer holds %lld, need %lld", (long long)feat_cap, (long long)total);
+        int64_t o = 0;
+        for (int64_t w = 0; w < nw; ++w) {
+            feat_off[w] = o;
+            for (int i = 0; i < nfeat[(size_t)w]; ++i) feat_idx[o++] = feat[(size_t)w * 9 + i];
+        }
+        feat_off[nw] = o;
+    }
+    return LT_OK;
+}
+
+extern "C" int lt_perceptron_delta(lt_batch* b, const lt_pathset* gold, int32_t func, int64_t* delta, int64_t n_delta,
+                                   uint8_t* differs, int64_t* n_differ) {
+    if (!b || !gold || !n_differ) return fail(LT_ERR_INVALID, "null argument");
+    if (!b->have_paths) return fail(LT_ERR_INVALID, "no paths: run lt_tag_batch_host or lt_beam first");
+    if (gold->tables != b->tables) return fail(LT_ERR_INVALID, "the gold path set belongs to other tables");
+    lt_tables* t = b->tables;
+    if (int rc = check_trigram_func(t, func)) return rc;
+    if (gold->n_paths != b->n_sent) return fail(LT_ERR_INVALID, "%d gold paths for %d sentences", gold->n_paths, b->n_sent);
+    if ((size_t)n_delta != t->feat_dst.size())
+        return fail(LT_ERR_INVALID, "the tables were built with %zu features, delta has %lld", t->feat_dst.size(), (long long)n_delta);
+    if ((n_delta > 0 && !delta) || (b->n_sent > 0 && !differs)) return fail(LT_ERR_INVALID, "null output pointer");
+    ON_DEVICE(t->device);
+    if (int rc = resolve(b)) return rc;
+    cudaStream_t st = b->last_stream;
+    const int n_sent = b->n_sent;
+    const size_t nu = (size_t)b->n_units;
+    if (!t->d_counts) CU(cudaMalloc(reinterpret_cast<void**>(&t->d_counts), n_hits(t) * 8));
+    if (int rc = upload_feat_dst(t)) return rc;
+    if (int rc = ensure(b->pth_ch, std::max<size_t>(1, nu) * 2)) return rc;
+    if (int rc = ensure(b->pth_ha, (nu + n_sent + 1) * 8)) return rc;
+    if (int rc = ensure(b->pth_hb, (nu + n_sent + 1) * 8)) return rc;
+    if (int rc = ensure(b->pc_delta, (size_t)std::max<int64_t>(1, n_delta) * 8)) return rc;
+    if (int rc = ensure(b->pc_differs, (size_t)std::max(1, n_sent))) return rc;
+    if (int rc = ensure(b->pc_count, 8)) return rc;
+    CU(cudaMemsetAsync(t->d_counts, 0, n_hits(t) * 8, st));
+    CU(cudaMemsetAsync(b->pc_count.p, 0, 8, st));
+    PerceptronArgs A{};
+    A.text = b->d_text;
+    A.sent_off = b->d_sent_off;
+    A.n_sent = n_sent;
+    A.func = func;
+    A.status = static_cast<const int32_t*>(b->status.p);
+    A.path_off = static_cast<const uint32_t*>(b->path_off.p);
+    A.path_edges = static_cast<const lt_edge*>(b->path_out.p);
+    A.imp = b->imported ? static_cast<const H2*>(b->imp.p) : nullptr;
+    A.gold_edges = gold->d_edges;
+    A.gold_off = gold->d_off;
+    A.gold_hashes = gold->d_hashes;
+    A.ch = static_cast<uint16_t*>(b->pth_ch.p);
+    A.ha = static_cast<uint64_t*>(b->pth_ha.p);
+    A.hb = static_cast<uint64_t*>(b->pth_hb.p);
+    A.counts = t->d_counts;
+    A.differs = static_cast<uint8_t*>(b->pc_differs.p);
+    A.n_differ = static_cast<unsigned long long*>(b->pc_count.p);
+    if (n_sent > 0) {
+        LT_LAUNCH(perceptron_kernel, warp_grid(t, n_sent), 256, 0, st, t->dev, A);
+        CU(cudaGetLastError());
+        b->launches += 1;
+    }
+    if (n_delta > 0) {
+        const unsigned grid = (unsigned)std::min<int64_t>((n_delta + 255) / 256, (int64_t)t->sm_count * 16);
+        LT_LAUNCH(gather_counts, grid, 256, 0, st, t->d_counts, t->d_feat_dst, n_delta, feat_slots(t), static_cast<long long*>(b->pc_delta.p));
+        CU(cudaGetLastError());
+        b->launches += 1;
+        CU(cudaMemcpyAsync(delta, b->pc_delta.p, (size_t)n_delta * 8, cudaMemcpyDeviceToHost, st));
+    }
+    unsigned long long nd = 0;
+    if (n_sent > 0) CU(cudaMemcpyAsync(differs, b->pc_differs.p, (size_t)n_sent, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&nd, b->pc_count.p, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    *n_differ = (int64_t)nd;
     return LT_OK;
 }

@@ -173,6 +173,12 @@ __device__ __forceinline__ bool feat_resolve(const DevTables& T, FKey k, FeatPro
     if (in_s || in_t) w = __hiloint2double((int)(in_s ? p.s.w : p.t.w), (int)(in_s ? p.s.z : p.t.z));   // a miss leaves w alone
     return in_s || in_t;
 }
+// the slot that holds key k, for a probe feat_resolve found (the slot whose weight it took)
+__device__ __forceinline__ uint32_t feat_hit_slot(const DevTables& T, FKey k, const FeatProbe& p) {
+    const uint64_t x = feature_slot_hash(k.k1);
+    const bool in_s = (p.s.x == (uint32_t)k.k2) && (p.s.y == (uint32_t)(k.k2 >> 32));
+    return (uint32_t)(in_s ? cuckoo_slot1(x, T.feat_bits) : cuckoo_slot2(x, T.feat_bits));
+}
 
 __device__ __forceinline__ H2 pow_at(const DevTables& T, uint32_t n) {
     const uint64_t* p = reinterpret_cast<const uint64_t*>(T.pows + n);

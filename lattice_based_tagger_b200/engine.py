@@ -13,7 +13,7 @@ from collections.abc import Sequence as _SequenceABC
 import numpy as np
 
 from . import _native
-from .compile import CompiledTables
+from .compile import CompiledTables, _encode_units
 from .tagset import BOS, EOS
 
 _STATUS_MESSAGES = {
@@ -225,15 +225,37 @@ class Engine:
             out.append(self.records_to_words(chars, records[ends[offs[i]]:ends[offs[i + 1]]]))
         return out
 
+    def pack_words(self, words):
+        """`Word`s -> LT_EDGE_EXPLICIT records (record i names strings 3i, 3i+1, 3i+2: word, morph0,
+        morph1) and those strings as UTF-16: (edges, units, str_off, n_strings).  A tag the tables do not
+        know, a string outside the BMP or a field outside the record's range raises `ValueError`."""
+        tag_ids = self.tables.tag_ids
+        other = self.tables.other_tag_id
+        rec, strings = [], []
+        for idx, w in enumerate(words):
+            if not 0 <= w.len < 65536:
+                raise ValueError('Word.len %r is outside 0..65535' % (w.len,))
+            if not (0 <= w.b < 65536 and 0 <= w.e < 65536):
+                raise ValueError('Word span [%r, %r) is outside 0..65535' % (w.b, w.e))
+            tag0 = tag_ids.get(w.tag0, other)
+            tag1 = 0xFF if w.tag1 is None else tag_ids.get(w.tag1, other)
+            if tag0 is None or tag1 is None:
+                raise ValueError('tag %r / %r is unknown to the compiled tables' % (w.tag0, w.tag1))
+            flags = (_native.LT_EDGE_EXPLICIT | (_native.LT_EDGE_IS_L if w.is_l else 0) |
+                     (_native.LT_EDGE_LEMMA if w.tag1 is not None else 0))
+            rec.append((w.b, w.e, int(w.len), tag0, tag1, idx, 0, flags, 0))
+            strings += [w.word, w.morph0, w.morph1 or '']
+        edges = np.array(rec, dtype=_native.EDGE_DTYPE) if rec else np.zeros(1, dtype=_native.EDGE_DTYPE)
+        units, str_off = _encode_units(strings)
+        return edges, units, str_off, len(strings)
+
     def import_lattice(self, sents, lattices):
         """Upload caller-built lattices (`lattices[i]` = iterable of `Word`s of sentence i, any order)
         for `lt_beam*`; returns the flat list of the imported `Word`s (index = record.rule)."""
         text, offsets = pack_sentences(sents)
         n = len(sents)
         n_units = int(offsets[-1])
-        tag_ids = self.tables.tag_ids
-        other = self.tables.other_tag_id
-        flat, rec, strings = [], [], []
+        flat = []
         end_off = np.zeros(n_units + 1, dtype=np.int64)
         for i, words in enumerate(lattices):
             m = len(sents[i].replace(' ', ''))
@@ -247,29 +269,45 @@ class Engine:
             usable.sort(key=lambda t: t[:3])
             counts = np.zeros(top - base, dtype=np.int64)
             start = len(flat)
-            for e, b, _, w in usable:
-                idx = len(flat)
+            for e, _, _, w in usable:
                 flat.append(w)
-                if not 0 <= w.len < 65536:
-                    raise ValueError('Word.len %r is outside 0..65535' % (w.len,))
-                tag0 = tag_ids.get(w.tag0, other)
-                tag1 = 0xFF if w.tag1 is None else tag_ids.get(w.tag1, other)
-                if tag0 is None or tag1 is None:
-                    raise ValueError('tag %r / %r is unknown to the compiled tables' % (w.tag0, w.tag1))
-                flags = (_native.LT_EDGE_EXPLICIT | (_native.LT_EDGE_IS_L if w.is_l else 0) |
-                         (_native.LT_EDGE_LEMMA if w.tag1 is not None else 0))
-                rec.append((b, e, int(w.len), tag0, tag1, idx, 0, flags, 0))
-                strings += [w.word, w.morph0, w.morph1 or '']
                 counts[e - 1] += 1
             if top > base:
                 end_off[base + 1:top + 1] = start + np.cumsum(counts)
-        edges = np.array(rec, dtype=_native.EDGE_DTYPE) if rec else np.zeros(1, dtype=_native.EDGE_DTYPE)
-        from .compile import _encode_units
-        units, str_off = _encode_units(strings)
+        edges, units, str_off, n_strings = self.pack_words(flat)
         _native.check(self._lib.lt_lattice_import(self.batch, _native.ptr(text), _native.ptr(offsets), n, _native.ptr(edges),
-                                                  _native.ptr(end_off), _native.ptr(units), _native.ptr(str_off), len(strings)))
+                                                  _native.ptr(end_off), _native.ptr(units), _native.ptr(str_off), n_strings))
         self._imported_words = flat
         return flat
+
+    # -- given paths -----------------------------------------------------------------------------------
+    def upload_paths(self, paths):
+        """`paths[p]` = the `Word`s of path p without BOS / EOS -> a `PathSet` on these tables."""
+        return PathSet(self, paths)
+
+    def eval_paths(self, pathset, func=None):
+        """lt_pathset_eval: (scores, feat_off, feat_idx); the features (of scorer index `func`, desc order)
+        only with `func`, else (scores, None, None)."""
+        n = pathset.n_paths
+        scores = np.zeros(max(1, n), dtype=np.float64)
+        if func is None:
+            _native.check(self._lib.lt_pathset_eval(self.batch, pathset.handle, -1, _native.ptr(scores), None, None, 0))
+            return scores[:n], None, None
+        feat_off = np.zeros(pathset.n_words + 1, dtype=np.int64)
+        feat_idx = np.zeros(max(1, 9 * pathset.n_words), dtype=np.int32)
+        _native.check(self._lib.lt_pathset_eval(self.batch, pathset.handle, int(func), _native.ptr(scores),
+                                                _native.ptr(feat_off), _native.ptr(feat_idx), feat_idx.size))
+        return scores[:n], feat_off, feat_idx[:int(feat_off[-1])]
+
+    def perceptron_delta(self, gold, func):
+        """lt_perceptron_delta against the last search: (delta in desc order, differs, n_differ)."""
+        n_feat = self.tables.n_desc
+        delta = np.zeros(max(1, n_feat), dtype=np.int64)
+        differs = np.zeros(max(1, gold.n_paths), dtype=np.uint8)
+        n_differ = ctypes.c_int64()
+        _native.check(self._lib.lt_perceptron_delta(self.batch, gold.handle, int(func), _native.ptr(delta), n_feat,
+                                                    _native.ptr(differs), ctypes.byref(n_differ)))
+        return delta[:n_feat], differs[:gold.n_paths].astype(bool), int(n_differ.value)
 
     # -- unpacking -----------------------------------------------------------------------------------
     def _status_message(self, st, index):
@@ -382,3 +420,35 @@ class Engine:
         i = _native.lt_info()
         _native.check(self._lib.lt_batch_info(self.batch, ctypes.byref(i)))
         return i.as_dict()
+
+
+class PathSet:
+    """Word paths on the device (`lt_pathset`), tied to one `Engine`'s tables: packed once, then scored,
+    featurized or compared with the engine's search results as often as needed."""
+
+    def __init__(self, engine, paths):
+        self._lib = engine._lib
+        self.tables = engine.tables
+        self.handle = None
+        lengths = [len(p) for p in paths]
+        off = np.zeros(len(paths) + 1, dtype=np.int64)
+        np.cumsum(lengths, out=off[1:])
+        edges, units, str_off, n_strings = engine.pack_words([w for p in paths for w in p])
+        handle = ctypes.c_void_p()
+        _native.check(self._lib.lt_pathset_create(self.tables.handle, len(paths), _native.ptr(edges), _native.ptr(off),
+                                                  _native.ptr(units), _native.ptr(str_off), n_strings, ctypes.byref(handle)))
+        self.handle = handle
+        self.n_paths = len(paths)
+        self.n_words = int(off[-1])
+        self.path_off = off
+
+    def close(self):
+        if self.handle is not None:
+            self._lib.lt_pathset_destroy(self.handle)
+            self.handle = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass

@@ -20,6 +20,36 @@ from ..engine import Engine, PackedSequences, pack_sentences  # noqa: F401  (pac
 from ..tagset import BOS, EOS
 
 
+def _inner_words(paths):
+    """`Sequence`s or [BOS, ..., EOS] word lists -> the words between BOS and EOS of each."""
+    from ..beam.beam import Sequence
+    out = []
+    for path in paths:
+        words = path.sequences if isinstance(path, Sequence) else path
+        if not isinstance(words, (list, tuple)) or len(words) < 2:
+            raise ValueError('a path is a Sequence or a [BOS, ..., EOS] word list, got %r' % (path,))
+        words = [w if isinstance(w, Word) else Word._make(w) if isinstance(w, tuple) and len(w) == len(Word._fields) else None
+                 for w in words]
+        if any(w is None for w in words) or words[0].tag0 != BOS or words[-1].tag0 != EOS:
+            raise ValueError('a path is a Sequence or a [BOS, ..., EOS] word list, got %r' % (path,))
+        out.append(words[1:-1])
+    return out
+
+
+def _trigram_func(score_funcs, scorer=None):
+    """(index in the score program, scorer) of `scorer`, by default the first SimpleTrigramFeatureScore."""
+    from ..beam import SimpleTrigramFeatureScore
+    funcs = list(getattr(score_funcs, 'funcs', None) or [])
+    for f, func in enumerate(funcs):
+        if (func is scorer) if scorer is not None else isinstance(func, SimpleTrigramFeatureScore):
+            if not isinstance(func, SimpleTrigramFeatureScore):
+                raise ValueError('%r is not a SimpleTrigramFeatureScore' % (func,))
+            return f, func
+    if scorer is None:
+        raise ValueError('the tagger has no SimpleTrigramFeatureScore')
+    raise ValueError('the scorer is not one of the tagger\'s score functions')
+
+
 class Tagger:
     """
     >>> funcs = BeamScoreFunctions(RegularizationScore(unknown_penalty=-.1, known_preference=0.5))
@@ -34,7 +64,7 @@ class Tagger:
     """
 
     def __init__(self, dictionary='base', lookup='subword_lookup', encoder=None, score_funcs=None,
-                 device=0, k3_first=None):
+                 device=0, k3_first=None, extra_tags=()):
         if isinstance(dictionary, str):
             dictionary = BaseMorphemeDictionary()
         self.dictionary = dictionary
@@ -42,6 +72,8 @@ class Tagger:
         self.device = device
         self._k3_first = k3_first
         self._lookup_arg = lookup
+        # tags no dictionary word carries that given paths may name (`score_paths`, the trainer's gold paths)
+        self._extra_tags = tuple(extra_tags)
         self._engine = None
         self.eojeol_lookup = None
         self.refresh()
@@ -50,7 +82,7 @@ class Tagger:
     def refresh(self):
         """(Re)compile the device tables — call after mutating the dictionary or the weights."""
         self.close()
-        self._engine = Engine(self.dictionary, self.score_funcs, self.device, self._k3_first)
+        self._engine = Engine(self.dictionary, self.score_funcs, self.device, self._k3_first, extra_tags=self._extra_tags)
         if isinstance(self._lookup_arg, EojeolLookup):
             self.eojeol_lookup = self._lookup_arg
         else:
@@ -174,6 +206,39 @@ class Tagger:
                         break
                     seq.num_unk += 1
                 print(seq, end='\n\n')
+
+    # -- given paths ---------------------------------------------------------------------------------
+    def score_paths(self, paths):
+        """The score the model gives each path (float64 array): what the score classes' `evaluate(seq)`
+        computes in the reference, on the device, bit for bit the arithmetic of the search.  A path is a
+        `Sequence` or a [BOS, ..., EOS] word list; it need not be one the search could find."""
+        if self.score_funcs is None:
+            raise TypeError("'NoneType' object is not callable")
+        pathset = self._engine.upload_paths(_inner_words(paths))
+        try:
+            return self._engine.eval_paths(pathset)[0]
+        finally:
+            pathset.close()
+
+    def encode_paths(self, paths, scorer=None):
+        """Per path the list `scorer.encoder.encode_sequence(words)` returns (feature-dictionary indices of
+        the trigram features that fire, word by word, template order), computed on the device.  `scorer`:
+        one of the tagger's `SimpleTrigramFeatureScore`s, by default the first."""
+        func, scorer = _trigram_func(self.score_funcs, scorer)
+        words = _inner_words(paths)
+        pathset = self._engine.upload_paths(words)
+        try:
+            _, feat_off, feat_idx = self._engine.eval_paths(pathset, func)
+        finally:
+            pathset.close()
+        desc_func, desc_fdic = self._engine.tables.desc_sources()
+        fdic = desc_fdic[feat_idx].tolist()
+        offs = feat_off.tolist()
+        out, w = [], 0
+        for path in words:
+            out.append([fdic[offs[i]:offs[i + 1]] for i in range(w, w + len(path))])
+            w += len(path)
+        return out
 
     def unpack(self, sents, packed, errors='raise'):
         return self._engine.unpack(sents, packed, errors)

@@ -12,7 +12,9 @@ decoding step is `Tagger.tag_batch` — the whole corpus in one device pass per 
 
 with phi = counts of the trigram features of a path (`SimpleTrigramEncoder.encode_sequence`,
 `features/feature.py:62-68`).  All sentences of an epoch are decoded with the same weights (the
-updates of one epoch are summed), so an epoch is one `tag_batch` call plus host-side counting.
+updates of one epoch are summed).  The gold paths go to the device once per `fit_parameter` call; an
+epoch is then a weight update, one decode of the corpus and one `lt_perceptron_delta` call, which
+compares every prediction with its gold path and counts the features of both on the device.
 There is no CPU decoder: without the CUDA library `Tagger` raises.
 """
 
@@ -21,7 +23,9 @@ import numpy as np
 from ..beam import BeamScoreFunctions
 from ..dictionary.text import text_to_words
 from ..features.utils import scan_features
+from ..compile import _is_bmp
 from ..tagger import Tagger
+from ..tagset import BUILTIN_TAGS, MAX_TAGS
 
 
 def _surface(word_text):
@@ -57,7 +61,8 @@ def train(word_morph_pairs, dictionary, encoder, score_func, regularity_func,
 
     encoder.feature_dic = feature_to_idx
     funcs = BeamScoreFunctions(regularity_func, score_func.set_encoder(encoder))
-    tagger = Tagger(dictionary, encoder=encoder, score_funcs=funcs, device=device)
+    tagger = Tagger(dictionary, encoder=encoder, score_funcs=funcs, device=device,
+                    extra_tags=_gold_tags(word_morph_pairs, dictionary))
 
     if verbose:
         print('Estimating parameter ...')
@@ -72,6 +77,61 @@ def train(word_morph_pairs, dictionary, encoder, score_func, regularity_func,
     return params
 
 
+def _gold_tags(word_morph_pairs, dictionary):
+    """Tags of the annotation that the dictionary lacks, as long as the device tables can hold them all: gold
+    paths that name them are then evaluated on the device, and the features that name them are kept in the
+    tables (no dictionary word carries such a tag, so decoding is unchanged)."""
+    known = set(BUILTIN_TAGS) | set(dictionary.tag_to_morphs)
+    extra = {}
+    for word_text, morph_text in word_morph_pairs:
+        try:
+            words = text_to_words(word_text, morph_text)
+        except Exception:
+            continue
+        for w in words:
+            for tag in (w.tag0, w.tag1):
+                if tag is not None and tag not in known:
+                    extra[tag] = None
+    return list(extra) if len(known) + len(extra) <= MAX_TAGS else []
+
+
+class _GoldCorpus:
+    """The annotation of a corpus, parsed and packed once: the surfaces the tagger receives, the gold
+    paths of the sentences the device can compare (uploaded as a path set on the tagger's tables), and
+    the rest — text outside the BMP, a tag the tables do not know — for the host loop."""
+
+    def __init__(self, word_morph_pairs, tagger):
+        self.golds, self.sents = [], []
+        for word_text, morph_text in word_morph_pairs:
+            try:
+                gold = text_to_words(word_text, morph_text)
+            except Exception:                          # malformed pairs are skipped, as scan_features does
+                continue
+            self.golds.append(gold)
+            self.sents.append(_surface(word_text))
+        self.pathset = self.tables = None
+        self.device_idx, self.host_idx = list(range(len(self.golds))), []
+        engine = tagger._engine
+        if tagger.eojeol_lookup.flatten:                # no lt_tag_batch_host paths: everything on the host
+            self.device_idx, self.host_idx = [], self.device_idx
+            return
+        tag_ids = engine.tables.tag_ids
+        usable, rest = [], []
+        for i, (gold, sent) in enumerate(zip(self.golds, self.sents)):
+            ok = _is_bmp(sent) and all(_is_bmp(w.word) and _is_bmp(w.morph0) and (w.morph1 is None or _is_bmp(w.morph1)) and
+                                       w.tag0 in tag_ids and (w.tag1 is None or w.tag1 in tag_ids) for w in gold[1:-1])
+            (usable if ok else rest).append(i)
+        self.device_idx, self.host_idx = usable, rest
+        self.device_sents = [self.sents[i] for i in usable]
+        self.pathset = engine.upload_paths([self.golds[i][1:-1] for i in usable])
+        self.tables = engine.tables
+
+    def close(self):
+        if self.pathset is not None:
+            self.pathset.close()
+            self.pathset = None
+
+
 def fit_parameter(word_morph_pairs, encoder, tagger, max_epochs=100, verbose=False, beam_size=5, patience=5,
                   averaged=False):
     """Reference `fit_parameter()` (`train.py:44-59`).  Stops once an epoch makes no mistake, or when the
@@ -82,17 +142,22 @@ def fit_parameter(word_morph_pairs, encoder, tagger, max_epochs=100, verbose=Fal
     best_loss, best_coef, stale = None, coef, 0
     total = np.zeros_like(coef)
     epochs = 0
-    for epoch in range(1, max_epochs + 1):
-        decoded_with = coef
-        coef, loss = train_epoch(word_morph_pairs, encoder, tagger, coef, epoch, verbose, beam_size=beam_size)
-        total += coef
-        epochs += 1
-        if best_loss is None or loss < best_loss:
-            best_loss, best_coef, stale = loss, decoded_with, 0       # `loss` was measured with the weights the epoch started from
-        else:
-            stale += 1
-        if loss == 0 or stale >= patience:
-            break
+    _load_weights(tagger, encoder, coef)               # the tables the gold paths are uploaded to
+    gold = _GoldCorpus(word_morph_pairs, tagger)
+    try:
+        for epoch in range(1, max_epochs + 1):
+            decoded_with = coef
+            coef, loss = train_epoch(word_morph_pairs, encoder, tagger, coef, epoch, verbose, beam_size=beam_size, gold=gold)
+            total += coef
+            epochs += 1
+            if best_loss is None or loss < best_loss:
+                best_loss, best_coef, stale = loss, decoded_with, 0       # `loss` was measured with the weights the epoch started from
+            else:
+                stale += 1
+            if loss == 0 or stale >= patience:
+                break
+    finally:
+        gold.close()
     if averaged:
         return total / max(1, epochs)
     return best_coef
@@ -106,12 +171,8 @@ def _trigram_scorer(tagger):
     raise ValueError('the tagger has no SimpleTrigramFeatureScore to train')
 
 
-def train_epoch(word_morph_pairs, encoder, tagger, coef, epoch, verbose, beam_size=5):
-    """One perceptron pass (the reference's TODO, `train.py:61-65`): -> (coef, loss).
-
-    loss = number of sentences whose best path under `coef` differs from the annotation.
-    """
-    coef = np.asarray(coef, dtype=np.float64).copy()
+def _load_weights(tagger, encoder, coef):
+    """Put `coef` into the tagger's trigram scorer and the device tables; -> the scorer."""
     scorer = _trigram_scorer(tagger)
     if scorer.encoder is encoder and scorer.coefficients is not None and len(scorer.coefficients) == len(coef) \
             and getattr(tagger, '_trained_features', None) is encoder.feature_dic:
@@ -121,18 +182,50 @@ def train_epoch(word_morph_pairs, encoder, tagger, coef, epoch, verbose, beam_si
         scorer.set_encoder(encoder, coef)
         tagger.refresh()                               # first epoch: feature table compiled once
         tagger._trained_features = encoder.feature_dic
+    return scorer
 
-    golds, sents = [], []
-    for word_text, morph_text in word_morph_pairs:
-        try:
-            gold = text_to_words(word_text, morph_text)
-        except Exception:                              # malformed pairs are skipped, as scan_features does
-            continue
-        golds.append(gold)
-        sents.append(_surface(word_text))
 
+def train_epoch(word_morph_pairs, encoder, tagger, coef, epoch, verbose, beam_size=5, gold=None):
+    """One perceptron pass (the reference's TODO, `train.py:61-65`): -> (coef, loss).
+
+    loss = number of sentences whose best path under `coef` differs from the annotation.  `gold`: the
+    corpus as `fit_parameter` prepared it (parsed and uploaded once for all epochs).  The sentences on the
+    device are decoded, compared and counted there (`lt_perceptron_delta`); the update of an epoch is a sum
+    of +-1 counts, so it is exact in any order.
+    """
+    coef = np.asarray(coef, dtype=np.float64).copy()
+    scorer = _load_weights(tagger, encoder, coef)
+    own = gold is None or gold.pathset is not None and gold.tables is not tagger._engine.tables
+    if own:
+        gold = _GoldCorpus(word_morph_pairs, tagger)
+    try:
+        update = np.zeros_like(coef)
+        loss = 0
+        if gold.device_idx:
+            engine = tagger._engine
+            func = tagger.score_funcs.funcs.index(scorer)
+            engine.tag_packed(gold.device_sents, beam_size)
+            delta, _, n_differ = engine.perceptron_delta(gold.pathset, func)
+            desc_func, desc_fdic = engine.tables.desc_sources()
+            hit = np.flatnonzero((desc_func == func) & (delta != 0))
+            np.add.at(update, desc_fdic[hit], delta[hit].astype(np.float64))     # a feature_dic need not be one-to-one
+            loss += n_differ
+        if gold.host_idx:
+            loss += _host_update(encoder, tagger, [gold.golds[i] for i in gold.host_idx],
+                                 [gold.sents[i] for i in gold.host_idx], beam_size, update)
+    finally:
+        if own:
+            gold.close()
+    coef += update
+    if verbose:
+        print('epoch %d: %d of %d sentences differ from the annotation' % (epoch, loss, len(gold.golds)))
+    return coef, loss
+
+
+def _host_update(encoder, tagger, golds, sents, beam_size, update):
+    """The epoch's counting on the host for sentences the device cannot compare: update += phi(gold) -
+    phi(predicted) per mistaken sentence; -> the number of mistakes."""
     predicted = tagger.tag_batch(sents, beam_size=beam_size, errors='none')
-    update = np.zeros_like(coef)
     loss = 0
     for gold, seq in zip(golds, predicted):
         if seq is not None and _same_path(seq.sequences, gold):
@@ -145,7 +238,4 @@ def train_epoch(word_morph_pairs, encoder, tagger, coef, epoch, verbose, beam_si
             for idxs in encoder.encode_sequence(seq.sequences):
                 for idx in idxs:
                     update[idx] -= 1.0
-    coef += update
-    if verbose:
-        print('epoch %d: %d of %d sentences differ from the annotation' % (epoch, loss, len(golds)))
-    return coef, loss
+    return loss
