@@ -1,7 +1,10 @@
 """Differential fuzzing of the kernel SOURCES against the oracle on the CPU (test infrastructure; not
 collected by pytest): random dictionaries / rules / features / sentences per seed, every sentence's
 lattice, best path, fp64 score and work counters compared bit for bit through the SIMT emulator, with
-the beam sizes, sentence lengths, k-best survivors and lookup modes rotating over the seeds.
+the beam sizes, sentence lengths, k-best survivors and lookup modes rotating over the seeds.  Every seed
+also scores and featurizes random tilings of its sentences and runs the perceptron step against gold
+paths that include near misses (tests/test_gpu_path_edges.py, `check_path_stage`); the 110- and
+200-syllable sentences give paths of more than one 32-word chunk.
 
     python tests/fuzz_emulated.py FIRST_SEED LAST_SEED        # prints `ok SEED` / `FAIL SEED` + traceback
     python tests/fuzz_emulated.py FIRST_SEED LAST_SEED knobs  # + the library's debugging knobs rotating over the seeds
@@ -20,6 +23,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import lattice_based_tagger_b200 as pkg                      # noqa: E402
 from oracle import lattice_oracle as lo                      # noqa: E402
 from tests import _cases, _checks, _emu                      # noqa: E402
+from tests import test_gpu_path_edges as path_edges          # noqa: E402
 
 BEAMS = [(1, 5), (2, 10), (3, 33), (7, 64), (16, 40)]
 LENGTHS = (8, 25, 60, 110, 200)
@@ -48,6 +52,7 @@ def run_seed(seed, knobs=False):
     _checks.check_against_oracle(tagger, oracle, case['sentences'], beams, counters=True)
     if seed % 3 == 0:
         _checks.check_kbest(tagger, oracle, case['sentences'], (beams[0], 5))
+    path_edges.check_path_stage(case, funcs, tagger, seed, beams[0])
     if seed % 7 == 0:
         _checks.check_lookup_modes(case)
 

@@ -157,6 +157,25 @@ def test_update_weights_and_trainer():
     _checks.check_against_oracle(tagger, lo.OracleTagger(dictionary, funcs), case['sentences'], (1, 5))
 
 
+@pytest.mark.parametrize('block_order', ['forward', 'reverse'])
+def test_path_kernels(monkeypatch, block_order):
+    """The given-path kernels (tests/test_gpu_path_edges.py) on an emulated device of 2 SMs, whose launches are
+    small enough that the path and perceptron grids take their stride: paths across chunk boundaries, the
+    perceptron on long sentences, after each kind of search and through a sequence of batches."""
+    import tests.test_gpu_path_edges as path_edges
+    monkeypatch.setenv('LT_SIMT_BLOCK_ORDER', block_order)
+    monkeypatch.setenv('LT_SIMT_SMS', '2')
+    path_edges.check_chunk_boundaries(21, 'all', per_length=3)
+    path_edges.check_path_grid_stride(23, per_length=2)
+    path_edges.check_long_sentences(31, n_long=2)
+    for search in ('tag', 'kbest', 'imported'):
+        path_edges.check_after_search(search)
+    path_edges.check_batch_sequence(n_big=60)
+    monkeypatch.setenv('LT_HIT_CAP', '8')
+    monkeypatch.setenv('LT_EDGE_CAP', '16')
+    path_edges.check_after_search('rerun')
+
+
 def test_memcheck_self_test(tmp_path):
     """LT_SIMT_MEMCHECK=1 places device buffers and a launch's dynamic shared memory against guard pages: the
     emulator's own check that an access one element past either is caught (and that a clean kernel is not)."""
