@@ -16,6 +16,8 @@
  *   lt_pathset_eval    <- the score classes' `evaluate(seq)` hooks (beam/score_funcs.py) and
  *                         SimpleTrigramEncoder.encode_sequence (features/feature.py:62-68) on given paths.
  *   lt_perceptron_delta <- the trainer's epoch (trainer/train.py:61-65): phi(gold) - phi(predicted).
+ *   lt_evaluate        <- comparing the tagger's output with an annotated corpus (the trainer's loss,
+ *                         word-level matches, and why a wrong sentence is wrong).
  *
  * Plain pointers and sizes only.  No function throws; each returns LT_OK or an LT_ERR_* code and
  * lt_last_error() returns the message of the calling thread's last failure.
@@ -30,7 +32,7 @@
 extern "C" {
 #endif
 
-#define LT_ABI_VERSION 4
+#define LT_ABI_VERSION 5
 
 /* return codes */
 #define LT_OK            0
@@ -333,6 +335,54 @@ int  lt_pathset_eval(lt_batch* batch, const lt_pathset* paths, int32_t func, dou
  * The count buffer belongs to the tables: no other lt_perceptron_delta on the same tables may run meanwhile. */
 int  lt_perceptron_delta(lt_batch* batch, const lt_pathset* gold, int32_t func, int64_t* delta, int64_t n_delta,
                          uint8_t* differs, int64_t* n_differ);
+
+/* lt_evaluate: the class of a sentence */
+#define LT_EVAL_CORRECT      0  /* status LT_SENT_OK and the best path is the gold path (the negation of
+                                   lt_perceptron_delta's `differs`)                                  */
+#define LT_EVAL_FAILED       1  /* status is not LT_SENT_OK                                          */
+#define LT_EVAL_UNREACHABLE  2  /* the gold path is not in the search space of beam_search          */
+#define LT_EVAL_SEARCH_ERROR 3  /* reachable, and its image scores higher than the path found        */
+#define LT_EVAL_MODEL_ERROR  4  /* reachable, and its image scores at most the found path's score    */
+
+/* lt_evaluate: why a gold word is outside the search space (the first check it fails, in this order) */
+#define LT_GOLD_OK             0
+#define LT_GOLD_BREAKS_TILING  1  /* does not begin where the previous word ends (0 for the first word),
+                                     ends beyond the sentence, or is the last word and does not end at
+                                     its last syllable                                                   */
+#define LT_GOLD_BEYOND_WINDOW  2  /* e - b > LT_WINDOW                                                   */
+#define LT_GOLD_NOT_IN_LATTICE 3  /* no lattice edge of its (b, e) equals it on b, e, tag0, tag1, morph0,
+                                     morph1; where the lattice has no edge of that span at all, it is not
+                                     the beam's unknown word (tag0 Unk, no tag1, morph0 = the span's
+                                     syllables, no morph1)                                               */
+#define LT_GOLD_UNK_AFTER_UNK  4  /* tag0 Unk right after a tag0-Unk word, and b != max(0, e - LT_WINDOW)
+                                     (beam/beam.py:44-45)                                               */
+#define LT_GOLD_UNCHECKED   0xFF  /* the sentence's status is not LT_SENT_OK                              */
+
+/* lt_evaluate: counts[LT_EVAL_N_COUNTS * s + i] */
+#define LT_EVAL_GOLD_WORDS 0
+#define LT_EVAL_PRED_WORDS 1      /* 0 unless the status is LT_SENT_OK                                  */
+#define LT_EVAL_SEG        2      /* predicted words equal to a gold word on b, e                        */
+#define LT_EVAL_TAG        3      /* ... on b, e, tag0, tag1                                             */
+#define LT_EVAL_FULL       4      /* ... on b, e, tag0, tag1, morph0, morph1                              */
+#define LT_EVAL_GOLD_UNITS 5      /* (morph0, tag0) per word, plus (morph1, tag1) when tag1 is set        */
+#define LT_EVAL_PRED_UNITS 6
+#define LT_EVAL_UNIT_MATCH 7      /* units of words equal on b, e whose morpheme and tag are equal        */
+#define LT_EVAL_N_COUNTS   8
+
+/* The best paths of the batch's last search (lt_tag_batch_host, lt_tag_batch_device, lt_beam, lt_beam_kbest,
+ * also over an imported lattice) against gold path s for sentence s (gold->n_paths = the batch's sentences;
+ * every gold path has b < e and strictly increasing b).  Per sentence:
+ *   sent_class   LT_EVAL_* (required)
+ *   counts       LT_EVAL_N_COUNTS int32 (LT_EVAL_GOLD_WORDS ...), or NULL
+ *   gold_scores  the score of the gold path's image, NaN unless the gold path is reachable, or NULL
+ *   word_reason  per gold word (gold->n_words) LT_GOLD_*, or NULL
+ * A gold path is reachable when the status is LT_SENT_OK, every word passes the LT_GOLD_* checks, and the path
+ * is not empty unless the sentence is.  Its image takes for each word the first equal lattice edge of its end
+ * position's bucket (or the beam's unknown-word record), and its score is bit for bit lt_pathset_eval of the
+ * image, the search's own score when the image is the path the search found.  Runs on the batch's stream;
+ * synchronous. */
+int  lt_evaluate(lt_batch* batch, const lt_pathset* gold, uint8_t* sent_class, int32_t* counts,
+                 double* gold_scores, uint8_t* word_reason);
 
 #ifdef __cplusplus
 }

@@ -13,7 +13,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, 'liblt_b200.so')
 
-LT_ABI_VERSION = 4
+LT_ABI_VERSION = 5
 LT_OK = 0
 LT_SENT_OK, LT_SENT_NO_EDGES, LT_SENT_BAD_SPACE, LT_SENT_TOO_LONG, LT_SENT_UNSUPPORTED_CHAR = 0, 1, 2, 3, 4
 LT_NO_TAG = 0xFF
@@ -23,6 +23,13 @@ LT_EDGE_IS_L, LT_EDGE_UNK, LT_EDGE_LEMMA, LT_EDGE_SKIP2, LT_EDGE_EXPLICIT = 1, 2
  LT_LOOKUP_EXACT) = range(6)
 LT_FUNC_REG, LT_FUNC_MPREF, LT_FUNC_WPREF, LT_FUNC_TRIGRAM = 1, 2, 3, 4
 LT_MAX_BEAM = 64
+LT_WINDOW = 8
+LT_EVAL_CORRECT, LT_EVAL_FAILED, LT_EVAL_UNREACHABLE, LT_EVAL_SEARCH_ERROR, LT_EVAL_MODEL_ERROR = range(5)
+LT_GOLD_OK, LT_GOLD_BREAKS_TILING, LT_GOLD_BEYOND_WINDOW, LT_GOLD_NOT_IN_LATTICE, LT_GOLD_UNK_AFTER_UNK = range(5)
+LT_GOLD_UNCHECKED = 0xFF
+(LT_EVAL_GOLD_WORDS, LT_EVAL_PRED_WORDS, LT_EVAL_SEG, LT_EVAL_TAG, LT_EVAL_FULL, LT_EVAL_GOLD_UNITS, LT_EVAL_PRED_UNITS,
+ LT_EVAL_UNIT_MATCH) = range(8)
+LT_EVAL_N_COUNTS = 8
 LT_MAX_FUNCS = 8
 
 #: numpy view of `lt_edge` (16 bytes)
@@ -116,6 +123,7 @@ SYMBOLS = {
     'lt_pathset_destroy': (None, [_p]),
     'lt_pathset_eval': (ctypes.c_int, [_p, _p, ctypes.c_int32, _p, _p, _p, ctypes.c_int64]),
     'lt_perceptron_delta': (ctypes.c_int, [_p, _p, ctypes.c_int32, _p, ctypes.c_int64, _p, ctypes.POINTER(ctypes.c_int64)]),
+    'lt_evaluate': (ctypes.c_int, [_p, _p, _p, _p, _p, _p]),
 }
 
 _lib = None

@@ -15,6 +15,7 @@
 
 #include "../../include/lt_b200.h"
 #include "beam.cuh"
+#include "evaluate.cuh"
 #include "hash.cuh"
 #include "lattice.cuh"
 #include "paths.cuh"
@@ -471,6 +472,7 @@ struct lt_batch {
     DevBuf pth_ch, pth_ha, pth_hb;               // lt_perceptron_delta: syllables and prefix hashes of the batch's sentences
     DevBuf pth_scores, pth_feat, pth_nfeat;      // lt_pathset_eval results
     DevBuf pc_delta, pc_differs, pc_count;       // lt_perceptron_delta results
+    DevBuf ev_image, ev_class, ev_counts, ev_scores, ev_reason;   // lt_evaluate: gold images (scratch), results
     bool imported = false;
     const uint16_t* d_text = nullptr;
     const int32_t* d_sent_off = nullptr;
@@ -614,7 +616,8 @@ extern "C" void lt_batch_destroy(lt_batch* b) {
                       &b->path_len, &b->path_off, &b->scores, &b->edges, &b->trail, &b->path_tmp, &b->path_out,
                       &b->counters, &b->ctl, &b->order, &b->retry, &b->kb_tmp, &b->kb_out, &b->kb_len, &b->kb_off,
                       &b->kb_scores, &b->kb_count, &b->imp, &b->pth_ch, &b->pth_ha, &b->pth_hb, &b->pth_scores,
-                      &b->pth_feat, &b->pth_nfeat, &b->pc_delta, &b->pc_differs, &b->pc_count};
+                      &b->pth_feat, &b->pth_nfeat, &b->pc_delta, &b->pc_differs, &b->pc_count,
+                      &b->ev_image, &b->ev_class, &b->ev_counts, &b->ev_scores, &b->ev_reason};
     for (DevBuf* x : bufs)
         if (x->p) cudaFree(x->p);
     for (auto& e : b->ev)
@@ -1533,6 +1536,7 @@ struct lt_pathset {
     int device = 0;
     int32_t n_paths = 0;
     int64_t n_words = 0;
+    bool ordered = true;            // every path: b < e, b strictly increasing (lt_evaluate needs it)
     int64_t* d_off = nullptr;
     lt_edge* d_edges = nullptr;
     H2* d_hashes = nullptr;
@@ -1565,6 +1569,10 @@ extern "C" int lt_pathset_create(lt_tables* t, int32_t n_paths, const lt_edge* e
         if ((int64_t)ed.rule * 3 + 2 >= n_strings) return fail(LT_ERR_INVALID, "word %lld: string index out of range", (long long)w);
         if (ed.tag0 >= n_tags || (ed.tag1 != LT_NO_TAG && ed.tag1 >= n_tags)) return fail(LT_ERR_INVALID, "word %lld: tag id out of range", (long long)w);
     }
+    bool ordered = true;
+    for (int32_t q = 0; q < n_paths && ordered; ++q)
+        for (int64_t w = path_off[q]; w < path_off[q + 1] && ordered; ++w)
+            ordered = edges[w].b < edges[w].e && (w == path_off[q] || edges[w - 1].b < edges[w].b);
     std::vector<H2> hashes((size_t)n_strings);
     for (int64_t i = 0; i < n_strings; ++i) {
         if (str_off[i + 1] < str_off[i]) return fail(LT_ERR_INVALID, "str_off is not monotone at %lld", (long long)i);
@@ -1576,6 +1584,7 @@ extern "C" int lt_pathset_create(lt_tables* t, int32_t n_paths, const lt_edge* e
     p->device = t->device;
     p->n_paths = n_paths;
     p->n_words = n_words;
+    p->ordered = ordered;
     auto put = [&](void** dst, const void* src, size_t bytes) -> cudaError_t {
         cudaError_t e = cudaMalloc(dst, std::max<size_t>(bytes, 16));
         if (e == cudaSuccess && bytes) e = cudaMemcpy(*dst, src, bytes, cudaMemcpyHostToDevice);
@@ -1736,5 +1745,68 @@ extern "C" int lt_perceptron_delta(lt_batch* b, const lt_pathset* gold, int32_t 
     CU(cudaMemcpyAsync(&nd, b->pc_count.p, 8, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     *n_differ = (int64_t)nd;
+    return LT_OK;
+}
+
+// The best paths of the last search against gold paths (evaluate.cuh): class, counts, image scores and reason
+// codes per sentence / gold word.
+extern "C" int lt_evaluate(lt_batch* b, const lt_pathset* gold, uint8_t* sent_class, int32_t* counts, double* gold_scores,
+                           uint8_t* word_reason) {
+    if (!b || !gold) return fail(LT_ERR_INVALID, "null argument");
+    if (!b->have_paths) return fail(LT_ERR_INVALID, "no paths: run a search (lt_tag_batch_host, lt_beam, ...) first");
+    if (gold->tables != b->tables) return fail(LT_ERR_INVALID, "the gold path set belongs to other tables");
+    if (gold->n_paths != b->n_sent) return fail(LT_ERR_INVALID, "%d gold paths for %d sentences", gold->n_paths, b->n_sent);
+    if (!gold->ordered) return fail(LT_ERR_INVALID, "a gold path has a word with b >= e or a b that does not increase");
+    if (b->n_sent > 0 && !sent_class) return fail(LT_ERR_INVALID, "null output pointer");
+    lt_tables* t = b->tables;
+    ON_DEVICE(t->device);
+    if (int rc = resolve(b)) return rc;
+    cudaStream_t st = b->last_stream;
+    const int n_sent = b->n_sent;
+    const size_t nu = (size_t)b->n_units;
+    const size_t nw = (size_t)gold->n_words;
+    if (int rc = ensure(b->pth_ch, std::max<size_t>(1, nu) * 2)) return rc;
+    if (int rc = ensure(b->pth_ha, (nu + n_sent + 1) * 8)) return rc;
+    if (int rc = ensure(b->pth_hb, (nu + n_sent + 1) * 8)) return rc;
+    if (int rc = ensure(b->ev_image, std::max<size_t>(1, nw) * sizeof(lt_edge))) return rc;
+    if (int rc = ensure(b->ev_class, (size_t)std::max(1, n_sent))) return rc;
+    if (counts)
+        if (int rc = ensure(b->ev_counts, (size_t)std::max(1, n_sent) * LT_EVAL_N_COUNTS * 4)) return rc;
+    if (gold_scores)
+        if (int rc = ensure(b->ev_scores, (size_t)std::max(1, n_sent) * 8)) return rc;
+    if (word_reason)
+        if (int rc = ensure(b->ev_reason, std::max<size_t>(1, nw))) return rc;
+    EvaluateArgs A{};
+    A.text = b->d_text;
+    A.sent_off = b->d_sent_off;
+    A.n_sent = n_sent;
+    A.status = static_cast<const int32_t*>(b->status.p);
+    A.path_off = static_cast<const uint32_t*>(b->path_off.p);
+    A.path_edges = static_cast<const lt_edge*>(b->path_out.p);
+    A.scores = static_cast<const double*>(b->scores.p);
+    A.pos = static_cast<const uint2*>(b->pos.p);
+    A.edges = static_cast<const lt_edge*>(b->edges.p);
+    A.imp = b->imported ? static_cast<const H2*>(b->imp.p) : nullptr;
+    A.gold_edges = gold->d_edges;
+    A.gold_off = gold->d_off;
+    A.gold_hashes = gold->d_hashes;
+    A.ch = static_cast<uint16_t*>(b->pth_ch.p);
+    A.ha = static_cast<uint64_t*>(b->pth_ha.p);
+    A.hb = static_cast<uint64_t*>(b->pth_hb.p);
+    A.image = static_cast<lt_edge*>(b->ev_image.p);
+    A.sent_class = static_cast<uint8_t*>(b->ev_class.p);
+    A.counts = counts ? static_cast<int32_t*>(b->ev_counts.p) : nullptr;
+    A.gold_scores = gold_scores ? static_cast<double*>(b->ev_scores.p) : nullptr;
+    A.word_reason = word_reason ? static_cast<uint8_t*>(b->ev_reason.p) : nullptr;
+    if (n_sent > 0) {
+        LT_LAUNCH(evaluate_kernel, warp_grid(t, n_sent), 256, 0, st, t->dev, A);
+        CU(cudaGetLastError());
+        b->launches += 1;
+        CU(cudaMemcpyAsync(sent_class, A.sent_class, (size_t)n_sent, cudaMemcpyDeviceToHost, st));
+        if (counts) CU(cudaMemcpyAsync(counts, A.counts, (size_t)n_sent * LT_EVAL_N_COUNTS * 4, cudaMemcpyDeviceToHost, st));
+        if (gold_scores) CU(cudaMemcpyAsync(gold_scores, A.gold_scores, (size_t)n_sent * 8, cudaMemcpyDeviceToHost, st));
+        if (word_reason && nw > 0) CU(cudaMemcpyAsync(word_reason, A.word_reason, nw, cudaMemcpyDeviceToHost, st));
+    }
+    CU(cudaStreamSynchronize(st));
     return LT_OK;
 }

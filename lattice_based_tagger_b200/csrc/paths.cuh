@@ -119,11 +119,10 @@ __device__ __forceinline__ H2 shfl_h2(H2 x, int src) {
     return H2{__shfl_sync(kFull, x.a, src), __shfl_sync(kFull, x.b, src)};
 }
 
-// One path of n words edges[0 .. n) with one warp: word w (lane w % 32 of chunk w / 32) is loaded with its
-// hashes (edge_hashes_inline: strings of LT_EDGE_EXPLICIT words from v.imp, the others from the sentence's
-// prefix hashes in v) and handed to visit(w, valid, word, context).  Every lane calls visit once per chunk.
-template <class Visit>
-__device__ __forceinline__ void walk_path(const DevTables& T, const lt_edge* edges, int n, const SentView& v, int lane, Visit visit) {
+// One path of n words with one warp: word w (lane w % 32 of chunk w / 32) is loaded with its hashes by
+// load(w, word) and handed to visit(w, valid, word, context).  Every lane calls visit once per chunk.
+template <class Load, class Visit>
+__device__ __forceinline__ void walk_words(const DevTables& T, int n, int lane, Load load, Visit visit) {
     // words base-1 (j of lane 0) and base-2 (i of lane 0, j... of lane 1): BOS, then nothing, before the path
     H2 w1 = T.bos, mo1 = T.bos, w2{0, 0}, mo2{0, 0};
     uint32_t t1 = LT_TAG_BOS, len1 = 0, t2 = LT_TAG_BOS;
@@ -133,10 +132,7 @@ __device__ __forceinline__ void walk_path(const DevTables& T, const lt_edge* edg
         EdgeView k{};
         k.tag0 = LT_TAG_BOS;
         k.tag1 = LT_NO_TAG;
-        if (valid) {
-            unpack_edge(ldg16(edges + w), k);
-            edge_hashes_inline<1>(T, v, k, true);
-        }
+        if (valid) load(w, k);
         H2 wj = shfl_up_h2(k.wk, 1), mj = shfl_up_h2(k.mk, 1);
         uint32_t tj = __shfl_up_sync(kFull, k.tag0, 1), lenj = __shfl_up_sync(kFull, k.len, 1);
         H2 wi = shfl_up_h2(k.wk, 2), mi = shfl_up_h2(k.mk, 2);
@@ -160,6 +156,37 @@ __device__ __forceinline__ void walk_path(const DevTables& T, const lt_edge* edg
         w2 = shfl_h2(k.wk, 30); mo2 = shfl_h2(k.mk, 30);
         t2 = __shfl_sync(kFull, k.tag0, 30);
     }
+}
+
+// walk_words over the records edges[0 .. n) (read-only for the kernel's lifetime), hashed by
+// edge_hashes_inline: strings of LT_EDGE_EXPLICIT words from v.imp, the others from the sentence's prefix
+// hashes in v.
+template <class Visit>
+__device__ __forceinline__ void walk_path(const DevTables& T, const lt_edge* edges, int n, const SentView& v, int lane, Visit visit) {
+    walk_words(T, n, lane, [&](int w, EdgeView& k) {
+        unpack_edge(ldg16(edges + w), k);
+        edge_hashes_inline<1>(T, v, k, true);
+    }, visit);
+}
+
+// A sentence's syllables (spaces dropped) into ch[0 .. L) and their prefix hashes into ha / hb[0 .. L], as the
+// beam kernel stages them, in global scratch; -> L.
+__device__ __forceinline__ int stage_sentence_hashes(const uint16_t* text, int s0, int s1, int lane, uint16_t* ch,
+                                                     uint64_t* ha, uint64_t* hb) {
+    const unsigned lt_mask = (1u << lane) - 1u;
+    int L = 0;
+    for (int base = 0; base < s1 - s0; base += 32) {
+        const bool in = base + lane < s1 - s0;
+        const uint32_t cu = in ? (uint32_t)text[s0 + base + lane] : 0x20u;
+        const bool keep = in && cu != 0x20u;
+        const unsigned km = __ballot_sync(kFull, keep);
+        if (keep) ch[L + __popc(km & lt_mask)] = (uint16_t)cu;
+        L += __popc(km);
+    }
+    __syncwarp();
+    prefix_hashes_inline(ch, L, lane, ha, hb);
+    __syncwarp();
+    return L;
 }
 
 struct PathEvalArgs {
@@ -227,7 +254,6 @@ struct PerceptronArgs {
 // b, e, morph0, morph1, tag0, tag1), and if so count +1 per gold hit and -1 per predicted hit.
 __global__ void __launch_bounds__(256) perceptron_kernel(const __grid_constant__ DevTables T, const __grid_constant__ PerceptronArgs A) {
     const int lane = threadIdx.x & 31;
-    const unsigned lt_mask = (1u << lane) - 1u;
     const int warps = (int)(gridDim.x * blockDim.x) >> 5;
     for (int s = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5); s < A.n_sent; s += warps) {
         const int st = A.status[s];
@@ -239,21 +265,7 @@ __global__ void __launch_bounds__(256) perceptron_kernel(const __grid_constant__
         uint16_t* ch = A.ch + s0;
         uint64_t* ha = A.ha + s0 + s;
         uint64_t* hb = A.hb + s0 + s;
-        if (st == LT_SENT_OK) {
-            // syllables and prefix hashes of the sentence, as the beam kernel stages them
-            int L = 0;
-            for (int base = 0; base < s1 - s0; base += 32) {
-                const bool in = base + lane < s1 - s0;
-                const uint32_t cu = in ? (uint32_t)A.text[s0 + base + lane] : 0x20u;
-                const bool keep = in && cu != 0x20u;
-                const unsigned km = __ballot_sync(kFull, keep);
-                if (keep) ch[L + __popc(km & lt_mask)] = (uint16_t)cu;
-                L += __popc(km);
-            }
-            __syncwarp();
-            prefix_hashes_inline(ch, L, lane, ha, hb);
-            __syncwarp();
-        }
+        if (st == LT_SENT_OK) stage_sentence_hashes(A.text, s0, s1, lane, ch, ha, hb);
         const SentView pv{ch, ha, hb, nullptr, A.imp};
         const SentView gv{nullptr, nullptr, nullptr, nullptr, A.gold_hashes};
         bool differ = st != LT_SENT_OK || P != G;

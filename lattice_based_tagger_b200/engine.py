@@ -309,6 +309,18 @@ class Engine:
                                                     _native.ptr(differs), ctypes.byref(n_differ)))
         return delta[:n_feat], differs[:gold.n_paths].astype(bool), int(n_differ.value)
 
+    def evaluate(self, gold):
+        """lt_evaluate against the last search: (sent_class uint8 [n], counts int32 [n, LT_EVAL_N_COUNTS],
+        gold_scores float64 [n] (NaN unless reachable), word_reason uint8 [gold.n_words])."""
+        n = gold.n_paths
+        sent_class = np.zeros(max(1, n), dtype=np.uint8)
+        counts = np.zeros((max(1, n), _native.LT_EVAL_N_COUNTS), dtype=np.int32)
+        gold_scores = np.zeros(max(1, n), dtype=np.float64)
+        word_reason = np.zeros(max(1, gold.n_words), dtype=np.uint8)
+        _native.check(self._lib.lt_evaluate(self.batch, gold.handle, _native.ptr(sent_class), _native.ptr(counts),
+                                            _native.ptr(gold_scores), _native.ptr(word_reason)))
+        return sent_class[:n], counts[:n], gold_scores[:n], word_reason[:gold.n_words]
+
     # -- unpacking -----------------------------------------------------------------------------------
     def _status_message(self, st, index):
         msg = _STATUS_MESSAGES.get(st, 'sentence %d could not be tagged')

@@ -4,8 +4,9 @@ Same constructor and `tag()` signature as the reference (`tagger/tagger.py:47-48
 returns a `Sequence` whose `.sequences` is the word list BOS .. EOS, `.score` the path score and
 `.num_unk` the trailing-unknown count.  Added for the GPU: `tag_batch()` (many sentences per
 call — the unit the kernels are built for), `tag_batch_kbest()` (every beam survivor, the
-return value of the reference's `beam_search`) and `lattice_batch()` (the lattice alone, i.e.
-`sentence_lookup_as_begin_index`, `dictionary/lookup.py:344-369`).
+return value of the reference's `beam_search`), `lattice_batch()` (the lattice alone, i.e.
+`sentence_lookup_as_begin_index`, `dictionary/lookup.py:344-369`), `score_paths()` / `encode_paths()`
+(given paths) and `evaluate()` (the output against gold analyses).
 
 All work happens in `liblt_b200.so`: the sentences go to the device as raw UTF-16 text, the
 lattice and beam kernels run there, and packed 16-byte word records come back.  Nothing is
@@ -239,6 +240,36 @@ class Tagger:
             out.append([fdic[offs[i]:offs[i + 1]] for i in range(w, w + len(path))])
             w += len(path)
         return out
+
+    def evaluate(self, sents, golds, beam_size=5):
+        """Tag `sents` and compare each best path with its gold path (`golds[i]`: a `Sequence` or a [BOS, ...,
+        EOS] word list, as for `score_paths`), all on the device: one decode, one upload of the gold paths, one
+        `lt_evaluate`.  Returns an `Evaluation`: per-sentence classes (correct, failed, unreachable, search
+        error, model error), word-level precision / recall / F1, the model's score of each reachable gold path,
+        and per gold word why it is outside the search space (`missing_words()` lists the dictionary's gaps).
+
+        Gold words must have b < e with b increasing along the path.  A `flatten=True` lookup is not supported:
+        its lattices hold single-morpheme words only, while gold words may have two."""
+        from ..compile import _is_bmp
+        from .evaluation import evaluate_pathset, ordered
+        if self.score_funcs is None:
+            raise TypeError("'NoneType' object is not callable")
+        if self.eojeol_lookup.flatten:
+            raise ValueError('evaluate() does not support a flatten=True lookup: its lattices hold single-morpheme words')
+        sents = list(sents)
+        golds = _inner_words(golds)
+        if len(sents) != len(golds):
+            raise ValueError('%d sentences but %d gold paths' % (len(sents), len(golds)))
+        bad = [i for i, s in enumerate(sents) if not _is_bmp(s)]
+        if bad:
+            raise ValueError(self._engine._status_message(_native.LT_SENT_UNSUPPORTED_CHAR, bad[0]))
+        if not ordered(golds):
+            raise ValueError('every gold word needs b < e, and b must increase along its path')
+        pathset = self._engine.upload_paths(golds)
+        try:
+            return evaluate_pathset(self._engine, sents, golds, pathset, beam_size)
+        finally:
+            pathset.close()
 
     def unpack(self, sents, packed, errors='raise'):
         return self._engine.unpack(sents, packed, errors)

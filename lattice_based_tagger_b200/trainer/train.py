@@ -101,14 +101,15 @@ class _GoldCorpus:
     the rest — text outside the BMP, a tag the tables do not know — for the host loop."""
 
     def __init__(self, word_morph_pairs, tagger):
-        self.golds, self.sents = [], []
-        for word_text, morph_text in word_morph_pairs:
+        self.golds, self.sents, self.pair_idx = [], [], []
+        for p, (word_text, morph_text) in enumerate(word_morph_pairs):
             try:
                 gold = text_to_words(word_text, morph_text)
             except Exception:                          # malformed pairs are skipped, as scan_features does
                 continue
             self.golds.append(gold)
             self.sents.append(_surface(word_text))
+            self.pair_idx.append(p)
         self.pathset = self.tables = None
         self.device_idx, self.host_idx = list(range(len(self.golds))), []
         engine = tagger._engine
@@ -130,6 +131,30 @@ class _GoldCorpus:
         if self.pathset is not None:
             self.pathset.close()
             self.pathset = None
+
+
+def evaluate(word_morph_pairs, tagger, beam_size=5):
+    """The tagger's output on an annotated corpus (`word_morph_pairs` as for `train`) against the annotation,
+    on the device: one decode, one `lt_evaluate` -> `Evaluation` (classes, precision / recall / F1 per level,
+    gold-path scores, `missing_words()`).  Pairs the device cannot compare are listed by position in
+    `Evaluation.not_evaluated` and left out of every count: a malformed annotation, text outside the BMP, a
+    tag the tagger's tables do not know.  `Evaluation.indices` gives the position of each evaluated pair.
+    A `flatten=True` tagger raises `ValueError` (see `Tagger.evaluate`)."""
+    from ..tagger.evaluation import evaluate_pathset, ordered
+    if tagger.eojeol_lookup.flatten:
+        raise ValueError('evaluate() does not support a flatten=True lookup: its lattices hold single-morpheme words')
+    word_morph_pairs = list(word_morph_pairs)
+    gold = _GoldCorpus(word_morph_pairs, tagger)
+    try:
+        golds = [gold.golds[i][1:-1] for i in gold.device_idx]
+        if not ordered(golds):
+            raise ValueError('an annotation yields a word with b >= e or out of order')
+        indices = [gold.pair_idx[i] for i in gold.device_idx]
+        parsed = set(gold.pair_idx)
+        left_out = sorted([p for p in range(len(word_morph_pairs)) if p not in parsed] + [gold.pair_idx[i] for i in gold.host_idx])
+        return evaluate_pathset(tagger._engine, gold.device_sents, golds, gold.pathset, beam_size, indices, left_out)
+    finally:
+        gold.close()
 
 
 def fit_parameter(word_morph_pairs, encoder, tagger, max_epochs=100, verbose=False, beam_size=5, patience=5,
