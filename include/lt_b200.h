@@ -301,8 +301,7 @@ int  lt_batch_info(lt_batch* batch, lt_info* out);
 int  lt_batch_counters(lt_batch* batch, lt_counters* out);
 int  lt_batch_timings(lt_batch* batch, lt_timings* out);
 /* Per-stage CUDA events on / off for the batches to come (the first lt_batch_timings call switches them on).
- * While they are recorded BETWEEN the kernels of a batch, the kernels are launched one strictly after the other;
- * without them each kernel is a programmatic dependent launch whose prologue overlaps its predecessor's tail.   */
+ * They are recorded on the batch's stream between its kernels, which run one after the other either way.       */
 int  lt_batch_set_stage_timing(lt_batch* batch, int32_t on);
 
 /* Word paths given by the caller (a gold analysis, candidates from elsewhere), device-resident, tied to one

@@ -423,12 +423,9 @@ __global__ void __launch_bounds__(beam_max_threads(KT, UC, PROG, KB), beam_min_b
     // CTA-shared dense tables (tag x tag matrix, length vectors)
     const size_t dense_bytes = ((size_t)T.n_tri * dense_block_bytes(NT) + 15) & ~(size_t)15;
     unsigned char* dense_smem = smem_raw;
-    lt_pdl_trigger();
-    // (the score tables are constant: staging them does not wait for the lattice kernel)
     for (size_t i = threadIdx.x * 4; i < (size_t)T.n_tri * dense_block_bytes(NT); i += blockDim.x * 4)
         *reinterpret_cast<uint32_t*>(dense_smem + i) = *reinterpret_cast<const uint32_t*>(T.dense + i);
     __syncthreads();
-    lt_pdl_wait();          // the lattice of this batch is complete
     if (A.flags[kFlagEdgeOverflow] | A.flags[kFlagStageOverflow]) {
         // lattice incomplete: the host grows the buffer and reruns; the path lengths the scan / pack kernels
         // behind this launch read must still be defined

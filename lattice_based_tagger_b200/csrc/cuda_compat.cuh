@@ -11,34 +11,5 @@
 #define LT_LAUNCH(kernel, grid, block, smem, stream, ...) kernel<<<(grid), (block), (smem), (stream)>>>(__VA_ARGS__)
 #if defined(__CUDACC__)
 #define LT_DEVICE_CODE 1
-#include <utility>
-// Programmatic dependent launch: with `pdl` the kernel may be scheduled while its predecessor in the stream is
-// still draining (every kernel of this library calls lt_pdl_trigger() first thing); whatever it does before
-// lt_pdl_wait() — carving up shared memory, staging the constant score tables — overlaps the predecessor's tail,
-// and lt_pdl_wait() returns once the predecessor has completed and its writes are visible.
-template <typename... KArgs, typename... Args>
-static inline cudaError_t lt_launch_pdl(bool pdl, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
-                                        Args&&... args) {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
-}
-#define LT_LAUNCH_PDL(pdl, kernel, grid, block, smem, stream, ...) \
-    lt_launch_pdl((pdl), kernel, dim3((unsigned)(grid)), dim3((unsigned)(block)), (size_t)(smem), (stream), __VA_ARGS__)
-__device__ __forceinline__ void lt_pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void lt_pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 #endif
-#endif
-#if defined(LT_SIMT_EMU)
-#define LT_LAUNCH_PDL(pdl, kernel, grid, block, smem, stream, ...) (LT_LAUNCH(kernel, grid, block, smem, stream, __VA_ARGS__), cudaSuccess)
-static inline void lt_pdl_wait() {}
-static inline void lt_pdl_trigger() {}
 #endif

@@ -20,22 +20,10 @@
 namespace lt {
 
 struct EvaluateArgs {
-    const uint16_t* text;       // the batch's sentences (the last search)
-    const int32_t* sent_off;
-    int32_t n_sent;
-    const int32_t* status;
-    const uint32_t* path_off;   // best paths of the last search and their scores
-    const lt_edge* path_edges;
-    const double* scores;
+    SearchAndGold sg;
+    const double* scores;       // of the best paths
     const uint2* pos;           // lattice CSR: pos[sent_off[s] + e - 1] = (first edge, count) of the edges ending at e
     const lt_edge* edges;
-    const H2* imp;              // an imported lattice's string hashes, or nullptr
-    const lt_edge* gold_edges;  // gold path set, one path per sentence
-    const int64_t* gold_off;
-    const H2* gold_hashes;
-    uint16_t* ch;               // scratch: syllables [n_units], prefix hashes [n_units + n_sent]
-    uint64_t* ha;
-    uint64_t* hb;
     lt_edge* image;             // scratch: the image of gold word w [gold n_words]
     uint8_t* sent_class;        // [n_sent] LT_EVAL_*
     int32_t* counts;            // [LT_EVAL_N_COUNTS * n_sent]
@@ -62,20 +50,20 @@ __device__ __forceinline__ lt_edge unknown_record(int b, int e) {
 __global__ void __launch_bounds__(256) evaluate_kernel(const __grid_constant__ DevTables T, const __grid_constant__ EvaluateArgs A) {
     const int lane = threadIdx.x & 31;
     const int warps = (int)(gridDim.x * blockDim.x) >> 5;
-    for (int s = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5); s < A.n_sent; s += warps) {
-        const bool ok = A.status[s] == LT_SENT_OK;
-        const int64_t go = A.gold_off[s];
-        const int G = (int)(A.gold_off[s + 1] - go);
-        const lt_edge* gold = A.gold_edges + go;
-        const int s0 = A.sent_off[s], s1 = A.sent_off[s + 1];
-        const lt_edge* pred = A.path_edges + A.path_off[s];
-        const int P = ok ? (int)(A.path_off[s + 1] - A.path_off[s]) : 0;
-        uint16_t* ch = A.ch + s0;
-        uint64_t* ha = A.ha + s0 + s;
-        uint64_t* hb = A.hb + s0 + s;
-        const int L = ok ? stage_sentence_hashes(A.text, s0, s1, lane, ch, ha, hb) : 0;
-        const SentView pv{ch, ha, hb, nullptr, A.imp};
-        const SentView gv{nullptr, nullptr, nullptr, nullptr, A.gold_hashes};
+    for (int s = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5); s < A.sg.n_sent; s += warps) {
+        const bool ok = A.sg.status[s] == LT_SENT_OK;
+        const int64_t go = A.sg.gold_off[s];
+        const int G = (int)(A.sg.gold_off[s + 1] - go);
+        const lt_edge* gold = A.sg.gold_edges + go;
+        const int s0 = A.sg.sent_off[s], s1 = A.sg.sent_off[s + 1];
+        const lt_edge* pred = A.sg.path_edges + A.sg.path_off[s];
+        const int P = ok ? (int)(A.sg.path_off[s + 1] - A.sg.path_off[s]) : 0;
+        uint16_t* ch = A.sg.ch + s0;
+        uint64_t* ha = A.sg.ha + s0 + s;
+        uint64_t* hb = A.sg.hb + s0 + s;
+        const int L = ok ? stage_sentence_hashes(A.sg.text, s0, s1, lane, ch, ha, hb) : 0;
+        const SentView pv{ch, ha, hb, nullptr, A.sg.imp};
+        const SentView gv{nullptr, nullptr, nullptr, nullptr, A.sg.gold_hashes};
 
         // ---- 1. predicted words against the gold word with the same b ----
         int n_seg = 0, n_tag = 0, n_full = 0, n_pu = 0, n_um = 0;

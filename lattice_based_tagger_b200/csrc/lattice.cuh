@@ -624,8 +624,6 @@ __global__ void __launch_bounds__(lattice_max_threads(UC, HCT, LM), lattice_min_
     uint32_t* sub = const_cast<uint32_t*>(W.E.sub);
 
     unsigned long long acc_L = 0, acc_P = 0, acc_E = 0;
-    lt_pdl_trigger();
-    lt_pdl_wait();          // the batch prologue (queue cursor, work order) or the main pass (retry list) is complete
 
     while (true) {
         unsigned int s = 0;

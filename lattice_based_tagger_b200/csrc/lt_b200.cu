@@ -70,6 +70,43 @@ struct DeviceGuard {
     DeviceGuard _guard(device);                                                                   \
     if (_guard.err != cudaSuccess) return fail(LT_ERR_CUDA, "cudaSetDevice(%d) failed: %s", (int)(device), cudaGetErrorString(_guard.err))
 
+// A device buffer that frees itself; grown by ensure().
+struct DevBuf {
+    void* p = nullptr;
+    size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    ~DevBuf() {
+        if (p) cudaFree(p);
+    }
+};
+
+static int ensure(DevBuf& b, size_t bytes) {
+    if (bytes <= b.cap) return LT_OK;
+    if (b.p) cudaFree(b.p);
+    b.p = nullptr;
+    b.cap = 0;
+    size_t want = bytes + bytes / 4 + 256;
+    cudaError_t e = cudaMalloc(&b.p, want);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        e = cudaMalloc(&b.p, bytes);
+        want = bytes;
+    }
+    if (e != cudaSuccess) return fail(LT_ERR_CUDA, "cudaMalloc(%zu) failed: %s", bytes, cudaGetErrorString(e));
+    b.cap = want;
+    return LT_OK;
+}
+
+// Data uploaded once: a buffer of exactly `bytes` (at least 16, so that it is never null) and no slack behind it.
+static int upload_once(DevBuf& b, const void* src, size_t bytes) {
+    CU(cudaMalloc(&b.p, std::max<size_t>(bytes, 16)));
+    b.cap = std::max<size_t>(bytes, 16);
+    if (bytes) CU(cudaMemcpy(b.p, src, bytes, cudaMemcpyHostToDevice));
+    return LT_OK;
+}
+
 struct lt_tables {
     int device = 0;
     DevTables dev{};
@@ -82,15 +119,10 @@ struct lt_tables {
     // the dense blocks (kDstDense | byte offset / 8), or kDstNone for a feature no tuple can equal
     std::vector<uint32_t> feat_dst;
     std::vector<unsigned char> dense_host;
-    uint32_t* d_feat_dst = nullptr;
-    double* d_weights = nullptr;
+    DevBuf d_feat_dst, d_weights;
     // path sets (paths.cuh): a feature hit is a slot of the hashed table or feat_slots + a dense offset; per hit the
     // desc index of its feature, and the perceptron's count per hit — both made on first use
-    int32_t* d_hit_feat = nullptr;
-    unsigned long long* d_counts = nullptr;
-    // feature table extent and the device's L2 persistence limits (LT_L2_PERSIST, see launch_beam)
-    size_t feat_bytes = 0;
-    int l2_bytes = 0, l2_persist_max = 0, l2_window_max = 0;
+    DevBuf d_hit_feat, d_counts;
 };
 
 static H2 hash_units(const uint16_t* p, int64_t n) {
@@ -175,10 +207,6 @@ extern "C" void lt_tables_destroy(lt_tables* t) {
     if (!t) return;
     DeviceGuard guard(t->device);
     for (void* p : t->allocations) cudaFree(p);
-    if (t->d_feat_dst) cudaFree(t->d_feat_dst);
-    if (t->d_weights) cudaFree(t->d_weights);
-    if (t->d_hit_feat) cudaFree(t->d_hit_feat);
-    if (t->d_counts) cudaFree(t->d_counts);
     delete t;
 }
 
@@ -394,7 +422,6 @@ static int build_tables(const lt_tables_desc* d, lt_tables* t) {
         }
         D.feat_mask = table.size() - 1;
         if (int rc = upload(t, table, &D.feat)) return rc;
-        t->feat_bytes = table.size() * sizeof(FeatSlot);
     }
     if (int rc = upload(t, dense, &D.dense)) return rc;
     t->dense_host = dense;
@@ -414,11 +441,6 @@ extern "C" int lt_tables_create(const lt_tables_desc* desc, int device, lt_table
     cudaError_t e = cudaGetDeviceProperties(&prop, device);
     if (e != cudaSuccess) { delete t; return fail(LT_ERR_CUDA, "cudaGetDeviceProperties: %s", cudaGetErrorString(e)); }
     t->sm_count = prop.multiProcessorCount;
-#if !defined(LT_SIMT_EMU)
-    t->l2_bytes = prop.l2CacheSize;
-    t->l2_persist_max = prop.persistingL2CacheMaxSize;
-    t->l2_window_max = prop.accessPolicyMaxWindowSize;
-#endif
     int rc = build_tables(desc, t);
     if (rc != LT_OK) { lt_tables_destroy(t); return rc; }
     *out = t;
@@ -428,11 +450,6 @@ extern "C" int lt_tables_create(const lt_tables_desc* desc, int device, lt_table
 // ------------------------------------------------------------------------------------------------
 // batch workspace
 // ------------------------------------------------------------------------------------------------
-struct DevBuf {
-    void* p = nullptr;
-    size_t cap = 0;
-};
-
 // control words on the device: work-queue cursors, the 64-bit edge cursor, overflow flags, retry list length
 enum { kCtlLatticeQueue = 0, kCtlBeamQueue = 1, kCtlCursor = 2 /* 2 words */, kCtlFlags = 4 /* 2 words */, kCtlRetryQueue = 6,
        kCtlRetryCount = 7, kCtlWords = 8 };
@@ -457,6 +474,9 @@ struct BeamPlan {
     size_t smem = 0, warp_smem = 0;
     bool trail_smem = false;
 };
+
+// events of a timed batch (lt_batch_timings): host text in, lattice kernels, beam kernel, path packing, results out
+enum { kEvHostIn, kEvLatticeStart, kEvLatticeEnd, kEvBeamStart, kEvBeamEnd, kEvPackEnd, kEvHostOut, kStageEvents };
 
 struct lt_batch {
     lt_tables* tables = nullptr;
@@ -490,9 +510,6 @@ struct lt_batch {
     bool edge_cap_fixed = false;   // LT_EDGE_CAP given: start there instead of the size guess (tests)
     bool debug = false;            // LT_DEBUG: print launch shapes
     bool trail_smem_ok = true;     // LT_TRAIL_SMEM=0 keeps the back-pointers in HBM
-    int l2_persist_pct = 0;        // LT_L2_PERSIST=<percent of L2>: persisting access-policy window over the feature table
-    bool pdl = false;              // LT_PDL=1: programmatic dependent launch between the kernels of a batch (never while per-stage
-                                   // events are recorded between them).  Measured r2k: 5 us per C2 step SLOWER than plain launches
     int adapt_div = 32;            // LT_ADAPT_DIV: the main pass's staging area doubles when more than n_sent / this many eojeols
                                    // needed the retry pass (0 = never; measured on C3: the default is right)
     int sort_min = kSortMin;       // LT_SORT_MIN: staged hits per eojeol from which the lattice kernel ranks by sorting (tests: 1)
@@ -500,7 +517,7 @@ struct lt_batch {
     int64_t n_edges = 0;
     bool have_lattice = false, have_paths = false, have_kbest = false, resolved = false;
     bool beam_state_clean = false;   // beam queue cursor / counters still zero from the batch prologue
-    cudaEvent_t ev[10]{};
+    cudaEvent_t ev[kStageEvents]{};
     bool timed = false;
     int reruns = 0;                // grow-and-rerun rounds so far (cumulative)
     int64_t launches = 0;          // kernels launched so far (cumulative)
@@ -511,23 +528,6 @@ struct lt_batch {
     const LatticePlan* last_lattice_plan = nullptr;
     const BeamPlan* last_beam_plan = nullptr;
 };
-
-static int ensure(DevBuf& b, size_t bytes) {
-    if (bytes <= b.cap) return LT_OK;
-    if (b.p) cudaFree(b.p);
-    b.p = nullptr;
-    b.cap = 0;
-    size_t want = bytes + bytes / 4 + 256;
-    cudaError_t e = cudaMalloc(&b.p, want);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        e = cudaMalloc(&b.p, bytes);
-        want = bytes;
-    }
-    if (e != cudaSuccess) return fail(LT_ERR_CUDA, "cudaMalloc(%zu) failed: %s", bytes, cudaGetErrorString(e));
-    b.cap = want;
-    return LT_OK;
-}
 
 // Longest sentence (raw UTF-16 code units, spaces included) both kernels can hold in shared memory with
 // these tables: the lattice kernel's per-warp arrays grow with the longest dictionary string (substring
@@ -552,10 +552,8 @@ extern "C" int32_t lt_tables_max_sentence_units(const lt_tables* t) { return t ?
 
 // where each input feature's weight lives (feat_dst) on the device, uploaded on first use
 static int upload_feat_dst(lt_tables* t) {
-    if (t->d_feat_dst || t->feat_dst.empty()) return LT_OK;
-    CU(cudaMalloc(reinterpret_cast<void**>(&t->d_feat_dst), t->feat_dst.size() * 4));
-    CU(cudaMemcpy(t->d_feat_dst, t->feat_dst.data(), t->feat_dst.size() * 4, cudaMemcpyHostToDevice));
-    return LT_OK;
+    if (t->d_feat_dst.p || t->feat_dst.empty()) return LT_OK;
+    return upload_once(t->d_feat_dst, t->feat_dst.data(), t->feat_dst.size() * 4);
 }
 
 // New weights for the features the tables were built with (the trainer's epoch: same features, new
@@ -568,10 +566,11 @@ extern "C" int lt_tables_update_weights(lt_tables* t, const double* weights, int
     ON_DEVICE(t->device);
     if (n_weights == 0) return LT_OK;
     if (int rc = upload_feat_dst(t)) return rc;
-    if (!t->d_weights) CU(cudaMalloc(reinterpret_cast<void**>(&t->d_weights), (size_t)n_weights * 8));
-    CU(cudaMemcpy(t->d_weights, weights, (size_t)n_weights * 8, cudaMemcpyHostToDevice));
+    if (int rc = ensure(t->d_weights, (size_t)n_weights * 8)) return rc;
+    CU(cudaMemcpy(t->d_weights.p, weights, (size_t)n_weights * 8, cudaMemcpyHostToDevice));
     const unsigned grid = (unsigned)std::min<int64_t>((n_weights + 255) / 256, (int64_t)t->sm_count * 16);
-    LT_LAUNCH(scatter_weights, grid, 256, 0, (cudaStream_t) nullptr, const_cast<FeatSlot*>(t->dev.feat), t->d_feat_dst, t->d_weights, n_weights);
+    LT_LAUNCH(scatter_weights, grid, 256, 0, (cudaStream_t) nullptr, const_cast<FeatSlot*>(t->dev.feat),
+              static_cast<const uint32_t*>(t->d_feat_dst.p), static_cast<const double*>(t->d_weights.p), n_weights);
     CU(cudaGetLastError());
     double* dense = reinterpret_cast<double*>(t->dense_host.data());
     bool any_dense = false;
@@ -599,8 +598,6 @@ extern "C" int lt_batch_create(lt_tables* tables, lt_batch** out) {
     if (const char* env = getenv("LT_SORT_BY_LENGTH")) b->sort_by_length = atoi(env) != 0;
     if (const char* env = getenv("LT_EDGE_CAP")) { b->edge_cap = (uint32_t)std::max(16, atoi(env)); b->edge_cap_fixed = true; }
     if (const char* env = getenv("LT_TRAIL_SMEM")) b->trail_smem_ok = atoi(env) != 0;
-    if (const char* env = getenv("LT_L2_PERSIST")) b->l2_persist_pct = std::min(100, std::max(0, atoi(env)));
-    if (const char* env = getenv("LT_PDL")) b->pdl = atoi(env) != 0;
     if (const char* env = getenv("LT_ADAPT_DIV")) b->adapt_div = std::max(0, atoi(env));
     if (const char* env = getenv("LT_SORT_MIN")) b->sort_min = std::max(1, atoi(env));
     if (const char* env = getenv("LT_PROLOGUE_CTAS")) b->prologue_ctas = std::min(32, std::max(1, atoi(env)));
@@ -612,14 +609,6 @@ extern "C" int lt_batch_create(lt_tables* tables, lt_batch** out) {
 extern "C" void lt_batch_destroy(lt_batch* b) {
     if (!b) return;
     DeviceGuard guard(b->tables->device);
-    DevBuf* bufs[] = {&b->text, &b->sent_off, &b->pos, &b->scan_tmp, &b->sent_len, &b->sent_edges, &b->status,
-                      &b->path_len, &b->path_off, &b->scores, &b->edges, &b->trail, &b->path_tmp, &b->path_out,
-                      &b->counters, &b->ctl, &b->order, &b->retry, &b->kb_tmp, &b->kb_out, &b->kb_len, &b->kb_off,
-                      &b->kb_scores, &b->kb_count, &b->imp, &b->pth_ch, &b->pth_ha, &b->pth_hb, &b->pth_scores,
-                      &b->pth_feat, &b->pth_nfeat, &b->pc_delta, &b->pc_differs, &b->pc_count,
-                      &b->ev_image, &b->ev_class, &b->ev_counts, &b->ev_scores, &b->ev_reason};
-    for (DevBuf* x : bufs)
-        if (x->p) cudaFree(x->p);
     for (auto& e : b->ev)
         if (e) cudaEventDestroy(e);
     if (b->h_ctl) cudaFreeHost(b->h_ctl);
@@ -792,6 +781,49 @@ static int beam_plan(lt_batch* b, int lcap, int beam_size, bool kbest, const Bea
 }
 
 // ---- launches ----------------------------------------------------------------------------------
+// The inputs of the next lattice: text and sentence offsets in device memory, read on stream st.  The per-warp
+// arrays are sized for the longest sentence the caller reports, capped at what fits shared memory; the kernels
+// skip any sentence beyond that size (LT_SENT_TOO_LONG) instead of trusting the number.
+static void bind_batch(lt_batch* b, const uint16_t* d_text, const int32_t* d_sent_off, int32_t n_sent, int64_t n_units,
+                       int32_t max_sent_units, cudaStream_t st) {
+    b->last_stream = st;
+    b->d_text = d_text;
+    b->d_sent_off = d_sent_off;
+    b->n_sent = n_sent;
+    b->n_units = n_units;
+    b->max_sent_units = max_sent_units;
+    b->beam = 0;
+    b->lcap = std::max(8, (std::min(max_sent_units, unit_limit(b->tables)) + 7) & ~7);
+    b->have_lattice = b->have_paths = b->have_kbest = false;
+    b->imported = b->resolved = false;
+}
+
+// the order in which persistent warps take sentences (longest first), or nullptr: in input order
+static uint32_t* work_order(const lt_batch* b) {
+    return (b->sort_by_length && b->n_sent > 1) ? static_cast<uint32_t*>(b->order.p) : nullptr;
+}
+
+// Per-sentence buffers and control words of the bound batch; the batch prologue zeroes the control words and
+// counters and computes the work order.
+static int start_batch(lt_batch* b, cudaStream_t st) {
+    const int n_sent = b->n_sent;
+    if (int rc = ensure(b->pos, ((size_t)b->n_units + 1) * sizeof(uint2))) return rc;
+    if (int rc = ensure(b->sent_len, (size_t)std::max(1, n_sent) * 4)) return rc;
+    if (int rc = ensure(b->sent_edges, (size_t)std::max(1, n_sent) * 4)) return rc;
+    if (int rc = ensure(b->status, (size_t)std::max(1, n_sent) * 4)) return rc;
+    if (int rc = ensure(b->counters, 8 * sizeof(unsigned long long))) return rc;
+    if (int rc = ensure(b->ctl, kCtlWords * sizeof(unsigned int))) return rc;
+    if (b->sort_by_length && n_sent > 1)
+        if (int rc = ensure(b->order, (size_t)n_sent * 4)) return rc;
+    uint32_t* order = work_order(b);
+    LT_LAUNCH(batch_prologue, (unsigned)(order ? std::min(b->prologue_ctas, prologue_ctas(n_sent)) : 1), 1024, 0, st, b->d_sent_off, n_sent,
+              order, static_cast<unsigned int*>(b->ctl.p), kCtlWords, static_cast<unsigned long long*>(b->counters.p), 8);
+    CU(cudaGetLastError());
+    b->launches += 1;
+    b->beam_state_clean = true;
+    return LT_OK;
+}
+
 static int launch_lattice(lt_batch* b, cudaStream_t st) {
     lt_tables* t = b->tables;
     const int n_sent = b->n_sent;
@@ -800,19 +832,12 @@ static int launch_lattice(lt_batch* b, cudaStream_t st) {
     const LatticePlan* P = nullptr;
     if (int rc = lattice_plan(b, lcap, b->hcap, false, &P)) return rc;
     b->last_lattice_plan = P;
-
-    const size_t nu = (size_t)n_units + 1;
-    if (int rc = ensure(b->pos, nu * sizeof(uint2))) return rc;
-    if (int rc = ensure(b->sent_len, (size_t)std::max(1, n_sent) * 4)) return rc;
-    if (int rc = ensure(b->sent_edges, (size_t)std::max(1, n_sent) * 4)) return rc;
-    if (int rc = ensure(b->status, (size_t)std::max(1, n_sent) * 4)) return rc;
-    if (int rc = ensure(b->counters, 8 * sizeof(unsigned long long))) return rc;
-    if (int rc = ensure(b->ctl, kCtlWords * sizeof(unsigned int))) return rc;
     if (!b->edge_cap_fixed) {
         const uint64_t guess = (uint64_t)n_units * 3 + 4096;
         if (b->edge_cap < guess) b->edge_cap = (uint32_t)std::min<uint64_t>(guess, 0xFFFFFFF0ull);
     }
     if (int rc = ensure(b->edges, (size_t)b->edge_cap * sizeof(lt_edge))) return rc;
+    if (int rc = start_batch(b, st)) return rc;
 
     LatticeArgs A{};
     A.text = b->d_text;
@@ -835,19 +860,7 @@ static int launch_lattice(lt_batch* b, cudaStream_t st) {
     A.status = static_cast<int32_t*>(b->status.p);
     A.counters = static_cast<unsigned long long*>(b->counters.p);
     A.queue = ctl + kCtlLatticeQueue;
-    A.order = nullptr;
-    // prologue: control words and counters zeroed, work order (longest sentences first)
-    uint32_t* order = nullptr;
-    if (b->sort_by_length && n_sent > 1) {
-        if (int rc = ensure(b->order, (size_t)n_sent * 4)) return rc;
-        order = static_cast<uint32_t*>(b->order.p);
-    }
-    LT_LAUNCH(batch_prologue, (unsigned)(order ? std::min(b->prologue_ctas, prologue_ctas(n_sent)) : 1), 1024, 0, st, b->d_sent_off, n_sent, order, ctl, kCtlWords,
-              static_cast<unsigned long long*>(b->counters.p), 8);
-    CU(cudaGetLastError());
-    b->launches += 1;
-    A.order = order;
-    b->beam_state_clean = true;
+    A.order = work_order(b);
 
     const int64_t want_blocks = ((int64_t)n_sent + P->warps - 1) / P->warps;
     const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(want_blocks, (int64_t)t->sm_count * P->per_sm));
@@ -857,9 +870,9 @@ static int launch_lattice(lt_batch* b, cudaStream_t st) {
         A.retry_list = static_cast<uint2*>(b->retry.p);
         A.retry_count = ctl + kCtlRetryCount;
     }
-    if (b->timed) CU(cudaEventRecord(b->ev[0], st));
+    if (b->timed) CU(cudaEventRecord(b->ev[kEvLatticeStart], st));
     if (n_sent > 0) {
-        CU(LT_LAUNCH_PDL(b->pdl && !b->timed, P->fn, grid, P->warps * 32, P->smem, st, t->dev, A));
+        LT_LAUNCH(P->fn, grid, P->warps * 32, P->smem, st, t->dev, A);
         b->launches += 1;
     }
     CU(cudaGetLastError());
@@ -872,11 +885,11 @@ static int launch_lattice(lt_batch* b, cudaStream_t st) {
         R.hcap = Rp->hcap;
         R.queue = ctl + kCtlRetryQueue;
         R.retry_pass = 1;
-        CU(LT_LAUNCH_PDL(b->pdl && !b->timed, Rp->fn, (unsigned)(t->sm_count * Rp->per_sm), Rp->warps * 32, Rp->smem, st, t->dev, R));
+        LT_LAUNCH(Rp->fn, (unsigned)(t->sm_count * Rp->per_sm), Rp->warps * 32, Rp->smem, st, t->dev, R);
         CU(cudaGetLastError());
         b->launches += 1;
     }
-    if (b->timed) CU(cudaEventRecord(b->ev[1], st));
+    if (b->timed) CU(cudaEventRecord(b->ev[kEvLatticeEnd], st));
     b->have_lattice = true;
     b->have_paths = false;
     b->have_kbest = false;
@@ -933,7 +946,7 @@ static int launch_beam(lt_batch* b, cudaStream_t st, bool kbest) {
     A.scores = static_cast<double*>(b->scores.p);
     A.counters = static_cast<unsigned long long*>(b->counters.p);
     A.queue = ctl + kCtlBeamQueue;
-    A.order = (b->sort_by_length && n_sent > 1) ? static_cast<const uint32_t*>(b->order.p) : nullptr;
+    A.order = work_order(b);
     A.trail_smem = P->trail_smem ? 1 : 0;
     A.imp = b->imported ? static_cast<const H2*>(b->imp.p) : nullptr;
     A.kbest = kbest ? 1 : 0;
@@ -953,48 +966,20 @@ static int launch_beam(lt_batch* b, cudaStream_t st, bool kbest) {
         b->launches += 1;
     }
     b->beam_state_clean = false;
-#if !defined(LT_SIMT_EMU)
-    // Experiment (LT_L2_PERSIST, off by default; profiles/README.md has the measurement): a persisting L2 access-policy
-    // window over the feature table while the beam kernel runs.  The table is a hash table — its hot slots are
-    // scattered — so the window covers as much of it as the device allows and asks for the fraction that fits
-    // the persisting carve-out to stay resident.
-    bool windowed = false;
-    if (b->l2_persist_pct > 0 && t->feat_bytes > 0 && t->l2_persist_max > 0) {
-        const size_t carve = std::min<size_t>((size_t)t->l2_persist_max, (size_t)t->l2_bytes * (size_t)b->l2_persist_pct / 100);
-        CU(cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, carve));
-        cudaStreamAttrValue attr{};
-        attr.accessPolicyWindow.base_ptr = const_cast<FeatSlot*>(t->dev.feat);
-        attr.accessPolicyWindow.num_bytes = std::min<size_t>(t->feat_bytes, (size_t)t->l2_window_max);
-        attr.accessPolicyWindow.hitRatio = (float)std::min(1.0, (double)carve / (double)attr.accessPolicyWindow.num_bytes);
-        attr.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-        attr.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-        CU(cudaStreamSetAttribute(st, cudaStreamAttributeAccessPolicyWindow, &attr));
-        windowed = true;
-        if (b->debug) fprintf(stderr, "[lt] L2 persisting window: %zu B of the %zu B feature table, carve-out %zu B, hit ratio %.3f\n",
-                              (size_t)attr.accessPolicyWindow.num_bytes, t->feat_bytes, carve, attr.accessPolicyWindow.hitRatio);
-    }
-#endif
-    if (b->timed) CU(cudaEventRecord(b->ev[5], st));
+    if (b->timed) CU(cudaEventRecord(b->ev[kEvBeamStart], st));
     if (n_sent > 0) {
-        CU(LT_LAUNCH_PDL(b->pdl && !b->timed && !windowed, P->fn, grid, P->warps * 32, P->smem, st, t->dev, A));
+        LT_LAUNCH(P->fn, grid, P->warps * 32, P->smem, st, t->dev, A);
         b->launches += 1;
     }
     CU(cudaGetLastError());
-    if (b->timed) CU(cudaEventRecord(b->ev[6], st));
-#if !defined(LT_SIMT_EMU)
-    if (windowed) {
-        cudaStreamAttrValue attr{};
-        attr.accessPolicyWindow.num_bytes = 0;
-        CU(cudaStreamSetAttribute(st, cudaStreamAttributeAccessPolicyWindow, &attr));
-    }
-#endif
+    if (b->timed) CU(cudaEventRecord(b->ev[kEvBeamEnd], st));
     if (n_sent > 0 && n_sent <= kPackScanMax) {
         // offsets and packing in one launch (scan.cuh: pack_paths_scan)
         const int ctas = (int)std::min<int64_t>(((int64_t)n_sent + 31) / 32, (int64_t)t->sm_count);
         const int per = (n_sent + ctas - 1) / ctas;
-        CU(LT_LAUNCH_PDL(b->pdl && !b->timed, pack_paths_scan, (unsigned)((n_sent + per - 1) / per), kPackScanThreads, 0, st,
-                         static_cast<const lt_edge*>(b->path_tmp.p), b->d_sent_off, static_cast<const int32_t*>(b->path_len.p),
-                         static_cast<uint32_t*>(b->path_off.p), n_sent, per, static_cast<lt_edge*>(b->path_out.p)));
+        LT_LAUNCH(pack_paths_scan, (unsigned)((n_sent + per - 1) / per), kPackScanThreads, 0, st, static_cast<const lt_edge*>(b->path_tmp.p),
+                  b->d_sent_off, static_cast<const int32_t*>(b->path_len.p), static_cast<uint32_t*>(b->path_off.p), n_sent, per,
+                  static_cast<lt_edge*>(b->path_out.p));
         CU(cudaGetLastError());
         b->launches += 1;
     } else {
@@ -1022,7 +1007,7 @@ static int launch_beam(lt_batch* b, cudaStream_t st, bool kbest) {
             b->launches += 1;
         }
     }
-    if (b->timed) CU(cudaEventRecord(b->ev[7], st));
+    if (b->timed) CU(cudaEventRecord(b->ev[kEvPackEnd], st));
     b->have_paths = true;
     b->have_kbest = kbest;
     b->resolved = false;
@@ -1097,19 +1082,7 @@ extern "C" int lt_lattice(lt_batch* b, const uint16_t* d_text, const int32_t* d_
     if (n_sent > 0 && (!d_text || !d_sent_off)) return fail(LT_ERR_INVALID, "null input pointer");
     ON_DEVICE(b->tables->device);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    b->last_stream = st;
-    b->d_text = d_text;
-    b->d_sent_off = d_sent_off;
-    b->n_sent = n_sent;
-    b->n_units = n_units;
-    b->max_sent_units = max_sent_units;
-    b->have_lattice = b->have_paths = b->have_kbest = false;
-    b->imported = false;
-    b->beam = 0;
-    // the per-warp arrays are sized for the longest sentence the caller reports, capped at what fits shared
-    // memory; the kernels skip any sentence beyond that size (LT_SENT_TOO_LONG) instead of trusting the number
-    const int32_t limit = unit_limit(b->tables);
-    b->lcap = std::max(8, (std::min(max_sent_units, limit) + 7) & ~7);
+    bind_batch(b, d_text, d_sent_off, n_sent, n_units, max_sent_units, st);
     return launch_lattice(b, st);
 }
 
@@ -1271,9 +1244,8 @@ extern "C" int lt_kbest_fetch(lt_batch* b, int32_t* n_best, int32_t* path_off, l
     return LT_OK;
 }
 
-// host text -> device buffers of the batch
-static int upload_text(lt_batch* b, const uint16_t* text, const int32_t* sent_off, int32_t n_sent, cudaStream_t st,
-                       int64_t* n_units_out, int32_t* max_units_out) {
+// host text -> the batch's own buffers, bound as the input of the next lattice on the batch's own stream
+static int bind_host_text(lt_batch* b, const uint16_t* text, const int32_t* sent_off, int32_t n_sent) {
     if (!sent_off || n_sent < 0) return fail(LT_ERR_INVALID, "bad argument");
     const int64_t n_units = sent_off[n_sent];
     if (n_units > 0 && !text) return fail(LT_ERR_INVALID, "null text pointer");
@@ -1284,13 +1256,19 @@ static int upload_text(lt_batch* b, const uint16_t* text, const int32_t* sent_of
         max_units = std::max(max_units, len);
     }
     if (sent_off[0] != 0) return fail(LT_ERR_INVALID, "sent_off[0] must be 0");
+    cudaStream_t st = b->own_stream;
     if (int rc = ensure(b->text, (size_t)std::max<int64_t>(1, n_units) * 2)) return rc;
     if (int rc = ensure(b->sent_off, (size_t)(n_sent + 1) * 4)) return rc;
     if (n_units) CU(cudaMemcpyAsync(b->text.p, text, (size_t)n_units * 2, cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(b->sent_off.p, sent_off, (size_t)(n_sent + 1) * 4, cudaMemcpyHostToDevice, st));
-    *n_units_out = n_units;
-    *max_units_out = max_units;
+    bind_batch(b, static_cast<const uint16_t*>(b->text.p), static_cast<const int32_t*>(b->sent_off.p), n_sent, n_units, max_units, st);
     return LT_OK;
+}
+
+// ... and its lattice
+static int host_lattice(lt_batch* b, const uint16_t* text, const int32_t* sent_off, int32_t n_sent) {
+    if (int rc = bind_host_text(b, text, sent_off, n_sent)) return rc;
+    return launch_lattice(b, b->own_stream);
 }
 
 extern "C" int lt_tag_batch_host(lt_batch* b, const uint16_t* text, const int32_t* sent_off, int32_t n_sent,
@@ -1300,18 +1278,13 @@ extern "C" int lt_tag_batch_host(lt_batch* b, const uint16_t* text, const int32_
     ON_DEVICE(b->tables->device);
     cudaStream_t st = b->own_stream;
     const bool timed = b->timed;
-    if (timed) CU(cudaEventRecord(b->ev[8], st));
-    int64_t n_units = 0;
-    int32_t max_units = 0;
-    if (int rc = upload_text(b, text, sent_off, n_sent, st, &n_units, &max_units)) return rc;
-    if (int rc = lt_lattice(b, static_cast<const uint16_t*>(b->text.p), static_cast<const int32_t*>(b->sent_off.p), n_sent,
-                            n_units, max_units, st))
-        return rc;
+    if (timed) CU(cudaEventRecord(b->ev[kEvHostIn], st));
+    if (int rc = host_lattice(b, text, sent_off, n_sent)) return rc;
     if (int rc = lt_beam(b, beam_size, st)) return rc;
     if (int rc = fetch_paths(b, path_off, path_edges, path_cap, scores, status, st)) return rc;
     if (timed) {
-        CU(cudaEventRecord(b->ev[9], st));
-        CU(cudaEventSynchronize(b->ev[9]));
+        CU(cudaEventRecord(b->ev[kEvHostOut], st));
+        CU(cudaEventSynchronize(b->ev[kEvHostOut]));
     }
     return LT_OK;
 }
@@ -1321,14 +1294,8 @@ extern "C" int lt_tag_batch_host_kbest(lt_batch* b, const uint16_t* text, const 
                                        int32_t beam_size) {
     if (!b) return fail(LT_ERR_INVALID, "bad argument");
     ON_DEVICE(b->tables->device);
-    cudaStream_t st = b->own_stream;
-    int64_t n_units = 0;
-    int32_t max_units = 0;
-    if (int rc = upload_text(b, text, sent_off, n_sent, st, &n_units, &max_units)) return rc;
-    if (int rc = lt_lattice(b, static_cast<const uint16_t*>(b->text.p), static_cast<const int32_t*>(b->sent_off.p), n_sent,
-                            n_units, max_units, st))
-        return rc;
-    return lt_beam_kbest(b, beam_size, st);
+    if (int rc = host_lattice(b, text, sent_off, n_sent)) return rc;
+    return lt_beam_kbest(b, beam_size, b->own_stream);
 }
 
 // sentence_lookup_as_begin_index for a batch in HOST memory: copies the text in and builds the lattices
@@ -1336,12 +1303,28 @@ extern "C" int lt_tag_batch_host_kbest(lt_batch* b, const uint16_t* text, const 
 extern "C" int lt_lattice_host(lt_batch* b, const uint16_t* text, const int32_t* sent_off, int32_t n_sent) {
     if (!b) return fail(LT_ERR_INVALID, "bad argument");
     ON_DEVICE(b->tables->device);
-    cudaStream_t st = b->own_stream;
-    int64_t n_units = 0;
-    int32_t max_units = 0;
-    if (int rc = upload_text(b, text, sent_off, n_sent, st, &n_units, &max_units)) return rc;
-    return lt_lattice(b, static_cast<const uint16_t*>(b->text.p), static_cast<const int32_t*>(b->sent_off.p), n_sent, n_units,
-                      max_units, st);
+    return host_lattice(b, text, sent_off, n_sent);
+}
+
+// The (word, morph0, morph1) strings that LT_EDGE_EXPLICIT records name (lt_lattice_import, lt_pathset_create),
+// validated, then hashed.
+static int hash_strings(const uint16_t* str_chars, const int64_t* str_off, int64_t n_strings, std::vector<H2>* out) {
+    if (n_strings % 3 != 0 || (n_strings > 0 && (!str_chars || !str_off))) return fail(LT_ERR_INVALID, "strings come in (word, morph0, morph1) triples");
+    if (n_strings > 0 && str_off[0] < 0) return fail(LT_ERR_INVALID, "str_off[0] is negative");
+    out->resize((size_t)n_strings);
+    for (int64_t i = 0; i < n_strings; ++i) {
+        if (str_off[i + 1] < str_off[i]) return fail(LT_ERR_INVALID, "str_off is not monotone at %lld", (long long)i);
+        (*out)[(size_t)i] = hash_units(str_chars + str_off[i], str_off[i + 1] - str_off[i]);
+    }
+    return LT_OK;
+}
+
+// What is wrong with a given word record (nullptr: nothing): its tags, and the strings 3 * rule .. 3 * rule + 2
+// of an LT_EDGE_EXPLICIT record.
+static const char* check_explicit(const lt_edge& ed, int64_t n_strings, int n_tags) {
+    if (ed.tag0 >= n_tags || (ed.tag1 != LT_NO_TAG && ed.tag1 >= n_tags)) return "tag id out of range";
+    if ((ed.flags & LT_EDGE_EXPLICIT) && (int64_t)ed.rule * 3 + 2 >= n_strings) return "string index out of range";
+    return nullptr;
 }
 
 // beam_search's `bindex` argument: a lattice built by the caller (see include/lt_b200.h)
@@ -1350,24 +1333,15 @@ extern "C" int lt_lattice_import(lt_batch* b, const uint16_t* text, const int32_
                                  const int64_t* str_off, int64_t n_strings) {
     if (!b || !end_off || n_strings < 0) return fail(LT_ERR_INVALID, "bad argument");
     ON_DEVICE(b->tables->device);
+    if (int rc = bind_host_text(b, text, sent_off, n_sent)) return rc;
     cudaStream_t st = b->own_stream;
-    int64_t n_units = 0;
-    int32_t max_units = 0;
-    if (int rc = upload_text(b, text, sent_off, n_sent, st, &n_units, &max_units)) return rc;
+    const int64_t n_units = b->n_units;
     const int64_t n_edges = end_off[n_units];
     if (n_edges < 0 || n_edges > 0xFFFFFFF0ll) return fail(LT_ERR_INVALID, "edge count out of range");
+    if (end_off[0] < 0) return fail(LT_ERR_INVALID, "end_off[0] is negative");
     if (n_edges > 0 && !edges) return fail(LT_ERR_INVALID, "null edge pointer");
-    if (n_strings % 3 != 0 || (n_strings > 0 && (!str_chars || !str_off))) return fail(LT_ERR_INVALID, "strings come in (word, morph0, morph1) triples");
-    const int32_t limit = unit_limit(b->tables);
-    b->last_stream = st;
-    b->d_text = static_cast<const uint16_t*>(b->text.p);
-    b->d_sent_off = static_cast<const int32_t*>(b->sent_off.p);
-    b->n_sent = n_sent;
-    b->n_units = n_units;
-    b->max_sent_units = max_units;
-    b->beam = 0;
-    b->lcap = std::max(8, (std::min(max_units, limit) + 7) & ~7);
-    b->have_lattice = b->have_paths = b->have_kbest = false;
+    std::vector<H2> hashes;
+    if (int rc = hash_strings(str_chars, str_off, n_strings, &hashes)) return rc;
 
     // CSR rows, per-sentence status and syllable counts, validated on the host
     std::vector<uint2> pos((size_t)n_units + 1, make_uint2(0u, 0u));
@@ -1397,12 +1371,9 @@ extern "C" int lt_lattice_import(lt_batch* b, const uint16_t* text, const int32_
                 if (ed.e != p + 1 || ed.b >= ed.e) return fail(LT_ERR_INVALID, "edge %lld: span [%d, %d) does not end at syllable %d", (long long)k, ed.b, ed.e, p + 1);
                 if (k > lo && ed.b < prev_b) return fail(LT_ERR_INVALID, "edge %lld: edges of one end position must be sorted by begin", (long long)k);
                 prev_b = ed.b;
-                if (ed.tag0 >= n_tags || (ed.tag1 != LT_NO_TAG && ed.tag1 >= n_tags)) return fail(LT_ERR_INVALID, "edge %lld: tag id out of range", (long long)k);
-                if (ed.flags & LT_EDGE_EXPLICIT) {
-                    if ((int64_t)ed.rule * 3 + 2 >= n_strings) return fail(LT_ERR_INVALID, "edge %lld: string index out of range", (long long)k);
-                } else if ((ed.flags & LT_EDGE_LEMMA) && ed.rule != LT_NO_RULE) {
+                if (const char* why = check_explicit(ed, n_strings, n_tags)) return fail(LT_ERR_INVALID, "edge %lld: %s", (long long)k, why);
+                if (!(ed.flags & LT_EDGE_EXPLICIT) && (ed.flags & LT_EDGE_LEMMA) && ed.rule != LT_NO_RULE)
                     return fail(LT_ERR_INVALID, "edge %lld: imported lemma edges name their morphemes (LT_EDGE_EXPLICIT)", (long long)k);
-                }
             }
             total += hi - lo;
         }
@@ -1411,23 +1382,13 @@ extern "C" int lt_lattice_import(lt_batch* b, const uint16_t* text, const int32_
         else if (bad) status[s] = LT_SENT_BAD_SPACE;
         else if (L > 0 && total == 0) status[s] = LT_SENT_NO_EDGES;
     }
-    std::vector<H2> hashes((size_t)n_strings);
-    for (int64_t i = 0; i < n_strings; ++i) {
-        if (str_off[i + 1] < str_off[i]) return fail(LT_ERR_INVALID, "str_off is not monotone at %lld", (long long)i);
-        hashes[i] = hash_units(str_chars + str_off[i], str_off[i + 1] - str_off[i]);
-    }
 
-    const size_t nu = (size_t)n_units + 1;
-    if (int rc = ensure(b->pos, nu * sizeof(uint2))) return rc;
-    if (int rc = ensure(b->sent_len, (size_t)std::max(1, n_sent) * 4)) return rc;
-    if (int rc = ensure(b->sent_edges, (size_t)std::max(1, n_sent) * 4)) return rc;
-    if (int rc = ensure(b->status, (size_t)std::max(1, n_sent) * 4)) return rc;
-    if (int rc = ensure(b->counters, 8 * sizeof(unsigned long long))) return rc;
-    if (int rc = ensure(b->ctl, kCtlWords * sizeof(unsigned int))) return rc;
+    // control words / counters zeroed and the work order computed, exactly as before a device-built lattice
     if (b->edge_cap < (uint64_t)n_edges + 16) b->edge_cap = (uint32_t)(n_edges + 16);
     if (int rc = ensure(b->edges, (size_t)b->edge_cap * sizeof(lt_edge))) return rc;
     if (int rc = ensure(b->imp, std::max<size_t>(1, hashes.size()) * sizeof(H2))) return rc;
-    CU(cudaMemcpyAsync(b->pos.p, pos.data(), nu * sizeof(uint2), cudaMemcpyHostToDevice, st));
+    if (int rc = start_batch(b, st)) return rc;
+    CU(cudaMemcpyAsync(b->pos.p, pos.data(), pos.size() * sizeof(uint2), cudaMemcpyHostToDevice, st));
     if (n_edges) CU(cudaMemcpyAsync(b->edges.p, edges, (size_t)n_edges * sizeof(lt_edge), cudaMemcpyHostToDevice, st));
     if (n_sent) {
         CU(cudaMemcpyAsync(b->status.p, status.data(), (size_t)n_sent * 4, cudaMemcpyHostToDevice, st));
@@ -1435,18 +1396,7 @@ extern "C" int lt_lattice_import(lt_batch* b, const uint16_t* text, const int32_
         CU(cudaMemcpyAsync(b->sent_edges.p, sedges.data(), (size_t)n_sent * 4, cudaMemcpyHostToDevice, st));
     }
     if (!hashes.empty()) CU(cudaMemcpyAsync(b->imp.p, hashes.data(), hashes.size() * sizeof(H2), cudaMemcpyHostToDevice, st));
-    // control words / counters zeroed and the work order computed, exactly as before a device-built lattice
-    uint32_t* order = nullptr;
-    if (b->sort_by_length && n_sent > 1) {
-        if (int rc = ensure(b->order, (size_t)n_sent * 4)) return rc;
-        order = static_cast<uint32_t*>(b->order.p);
-    }
-    LT_LAUNCH(batch_prologue, (unsigned)(order ? std::min(b->prologue_ctas, prologue_ctas(n_sent)) : 1), 1024, 0, st, b->d_sent_off, n_sent, order, static_cast<unsigned int*>(b->ctl.p), kCtlWords,
-              static_cast<unsigned long long*>(b->counters.p), 8);
-    CU(cudaGetLastError());
-    b->launches += 1;
     CU(cudaStreamSynchronize(st));          // the staging vectors above go out of scope
-    b->beam_state_clean = true;
     b->have_lattice = true;
     b->imported = true;
     b->resolved = true;
@@ -1519,12 +1469,12 @@ extern "C" int lt_batch_timings(lt_batch* b, lt_timings* out) {
         if (cudaEventElapsedTime(&v, b->ev[a], b->ev[c]) == cudaSuccess) *dst = v;
         else cudaGetLastError();
     };
-    ms(0, 1, &out->ms_lattice);
-    ms(5, 6, &out->ms_beam);
-    ms(6, 7, &out->ms_pack);
-    ms(8, 0, &out->ms_h2d);
-    ms(7, 9, &out->ms_d2h);
-    ms(8, 9, &out->ms_total);
+    ms(kEvLatticeStart, kEvLatticeEnd, &out->ms_lattice);
+    ms(kEvBeamStart, kEvBeamEnd, &out->ms_beam);
+    ms(kEvBeamEnd, kEvPackEnd, &out->ms_pack);
+    ms(kEvHostIn, kEvLatticeStart, &out->ms_h2d);
+    ms(kEvPackEnd, kEvHostOut, &out->ms_d2h);
+    ms(kEvHostIn, kEvHostOut, &out->ms_total);
     return LT_OK;
 }
 
@@ -1537,17 +1487,12 @@ struct lt_pathset {
     int32_t n_paths = 0;
     int64_t n_words = 0;
     bool ordered = true;            // every path: b < e, b strictly increasing (lt_evaluate needs it)
-    int64_t* d_off = nullptr;
-    lt_edge* d_edges = nullptr;
-    H2* d_hashes = nullptr;
+    DevBuf off, edges, hashes;      // [n_paths + 1] offsets, [n_words] records, [n_strings] string hashes
 };
 
 extern "C" void lt_pathset_destroy(lt_pathset* p) {
     if (!p) return;
     DeviceGuard guard(p->device);      // (the tables may be gone already)
-    if (p->d_off) cudaFree(p->d_off);
-    if (p->d_edges) cudaFree(p->d_edges);
-    if (p->d_hashes) cudaFree(p->d_hashes);
     delete p;
 }
 
@@ -1560,24 +1505,17 @@ extern "C" int lt_pathset_create(lt_tables* t, int32_t n_paths, const lt_edge* e
         if (path_off[p + 1] < path_off[p]) return fail(LT_ERR_INVALID, "path_off is not monotone at %d", p);
     const int64_t n_words = path_off[n_paths];
     if (n_words > 0 && !edges) return fail(LT_ERR_INVALID, "null edge pointer");
-    if (n_strings % 3 != 0 || (n_strings > 0 && (!str_chars || !str_off))) return fail(LT_ERR_INVALID, "strings come in (word, morph0, morph1) triples");
-    if (n_strings > 0 && str_off[0] < 0) return fail(LT_ERR_INVALID, "str_off[0] is negative");
-    const int n_tags = t->dev.n_tags;
+    std::vector<H2> hashes;
+    if (int rc = hash_strings(str_chars, str_off, n_strings, &hashes)) return rc;
     for (int64_t w = 0; w < n_words; ++w) {
         const lt_edge& ed = edges[w];
         if (!(ed.flags & LT_EDGE_EXPLICIT)) return fail(LT_ERR_INVALID, "word %lld is not LT_EDGE_EXPLICIT", (long long)w);
-        if ((int64_t)ed.rule * 3 + 2 >= n_strings) return fail(LT_ERR_INVALID, "word %lld: string index out of range", (long long)w);
-        if (ed.tag0 >= n_tags || (ed.tag1 != LT_NO_TAG && ed.tag1 >= n_tags)) return fail(LT_ERR_INVALID, "word %lld: tag id out of range", (long long)w);
+        if (const char* why = check_explicit(ed, n_strings, t->dev.n_tags)) return fail(LT_ERR_INVALID, "word %lld: %s", (long long)w, why);
     }
     bool ordered = true;
     for (int32_t q = 0; q < n_paths && ordered; ++q)
         for (int64_t w = path_off[q]; w < path_off[q + 1] && ordered; ++w)
             ordered = edges[w].b < edges[w].e && (w == path_off[q] || edges[w - 1].b < edges[w].b);
-    std::vector<H2> hashes((size_t)n_strings);
-    for (int64_t i = 0; i < n_strings; ++i) {
-        if (str_off[i + 1] < str_off[i]) return fail(LT_ERR_INVALID, "str_off is not monotone at %lld", (long long)i);
-        hashes[i] = hash_units(str_chars + str_off[i], str_off[i + 1] - str_off[i]);
-    }
     ON_DEVICE(t->device);
     lt_pathset* p = new lt_pathset();
     p->tables = t;
@@ -1585,17 +1523,12 @@ extern "C" int lt_pathset_create(lt_tables* t, int32_t n_paths, const lt_edge* e
     p->n_paths = n_paths;
     p->n_words = n_words;
     p->ordered = ordered;
-    auto put = [&](void** dst, const void* src, size_t bytes) -> cudaError_t {
-        cudaError_t e = cudaMalloc(dst, std::max<size_t>(bytes, 16));
-        if (e == cudaSuccess && bytes) e = cudaMemcpy(*dst, src, bytes, cudaMemcpyHostToDevice);
-        return e;
-    };
-    cudaError_t e = put(reinterpret_cast<void**>(&p->d_off), path_off, (size_t)(n_paths + 1) * 8);
-    if (e == cudaSuccess) e = put(reinterpret_cast<void**>(&p->d_edges), edges, (size_t)n_words * sizeof(lt_edge));
-    if (e == cudaSuccess) e = put(reinterpret_cast<void**>(&p->d_hashes), hashes.data(), hashes.size() * sizeof(H2));
-    if (e != cudaSuccess) {
-        lt_pathset_destroy(p);
-        return fail(LT_ERR_CUDA, "path set upload failed: %s", cudaGetErrorString(e));
+    int rc = upload_once(p->off, path_off, (size_t)(n_paths + 1) * 8);
+    if (rc == LT_OK) rc = upload_once(p->edges, edges, (size_t)n_words * sizeof(lt_edge));
+    if (rc == LT_OK) rc = upload_once(p->hashes, hashes.data(), hashes.size() * sizeof(H2));
+    if (rc != LT_OK) {
+        delete p;
+        return rc;
     }
     *out = p;
     return LT_OK;
@@ -1633,28 +1566,27 @@ extern "C" int lt_pathset_eval(lt_batch* b, const lt_pathset* paths, int32_t fun
     const int64_t nw = paths->n_words;
     if (int rc = ensure(b->pth_scores, (size_t)std::max(1, paths->n_paths) * 8)) return rc;
     if (want_feat) {
-        if (!t->d_hit_feat) {
+        if (!t->d_hit_feat.p) {
             std::vector<int32_t> inv(n_hits(t), -1);
             for (size_t i = 0; i < t->feat_dst.size(); ++i) {
                 const uint32_t d = t->feat_dst[i];
                 if (d != kDstNone) inv[(d & kDstDense) ? feat_slots(t) + (d & ~kDstDense) : d] = (int32_t)i;
             }
-            CU(cudaMalloc(reinterpret_cast<void**>(&t->d_hit_feat), inv.size() * 4));
-            CU(cudaMemcpy(t->d_hit_feat, inv.data(), inv.size() * 4, cudaMemcpyHostToDevice));
+            if (int rc = upload_once(t->d_hit_feat, inv.data(), inv.size() * 4)) return rc;
         }
         if (int rc = ensure(b->pth_feat, (size_t)std::max<int64_t>(1, nw) * 9 * 4)) return rc;
         if (int rc = ensure(b->pth_nfeat, (size_t)std::max<int64_t>(1, nw))) return rc;
     }
     PathEvalArgs A{};
-    A.edges = paths->d_edges;
-    A.off = paths->d_off;
-    A.hashes = paths->d_hashes;
+    A.edges = static_cast<const lt_edge*>(paths->edges.p);
+    A.off = static_cast<const int64_t*>(paths->off.p);
+    A.hashes = static_cast<const H2*>(paths->hashes.p);
     A.n_paths = paths->n_paths;
     A.func = want_feat ? func : -1;
     A.scores = static_cast<double*>(b->pth_scores.p);
     A.feat = want_feat ? static_cast<int32_t*>(b->pth_feat.p) : nullptr;
     A.nfeat = static_cast<uint8_t*>(b->pth_nfeat.p);
-    A.hit_feat = t->d_hit_feat;
+    A.hit_feat = static_cast<const int32_t*>(t->d_hit_feat.p);
     if (paths->n_paths > 0) {
         LT_LAUNCH(path_eval_kernel, warp_grid(t, paths->n_paths), 256, 0, st, t->dev, A);
         CU(cudaGetLastError());
@@ -1684,14 +1616,42 @@ extern "C" int lt_pathset_eval(lt_batch* b, const lt_pathset* paths, int32_t fun
     return LT_OK;
 }
 
+// lt_perceptron_delta / lt_evaluate: the best paths of the last search next to one gold path per sentence
+static int check_gold(const lt_batch* b, const lt_pathset* gold) {
+    if (!b->have_paths) return fail(LT_ERR_INVALID, "no paths: run a search (lt_tag_batch_host, lt_beam, ...) first");
+    if (gold->tables != b->tables) return fail(LT_ERR_INVALID, "the gold path set belongs to other tables");
+    if (gold->n_paths != b->n_sent) return fail(LT_ERR_INVALID, "%d gold paths for %d sentences", gold->n_paths, b->n_sent);
+    return LT_OK;
+}
+
+// ... and what their kernels read of both, with the sentence scratch sized for the batch
+static int search_and_gold(lt_batch* b, const lt_pathset* gold, SearchAndGold* g) {
+    const size_t nu = (size_t)b->n_units, n_sent = (size_t)b->n_sent;
+    if (int rc = ensure(b->pth_ch, std::max<size_t>(1, nu) * 2)) return rc;
+    if (int rc = ensure(b->pth_ha, (nu + n_sent + 1) * 8)) return rc;
+    if (int rc = ensure(b->pth_hb, (nu + n_sent + 1) * 8)) return rc;
+    g->text = b->d_text;
+    g->sent_off = b->d_sent_off;
+    g->n_sent = b->n_sent;
+    g->status = static_cast<const int32_t*>(b->status.p);
+    g->path_off = static_cast<const uint32_t*>(b->path_off.p);
+    g->path_edges = static_cast<const lt_edge*>(b->path_out.p);
+    g->imp = b->imported ? static_cast<const H2*>(b->imp.p) : nullptr;
+    g->gold_edges = static_cast<const lt_edge*>(gold->edges.p);
+    g->gold_off = static_cast<const int64_t*>(gold->off.p);
+    g->gold_hashes = static_cast<const H2*>(gold->hashes.p);
+    g->ch = static_cast<uint16_t*>(b->pth_ch.p);
+    g->ha = static_cast<uint64_t*>(b->pth_ha.p);
+    g->hb = static_cast<uint64_t*>(b->pth_hb.p);
+    return LT_OK;
+}
+
 extern "C" int lt_perceptron_delta(lt_batch* b, const lt_pathset* gold, int32_t func, int64_t* delta, int64_t n_delta,
                                    uint8_t* differs, int64_t* n_differ) {
     if (!b || !gold || !n_differ) return fail(LT_ERR_INVALID, "null argument");
-    if (!b->have_paths) return fail(LT_ERR_INVALID, "no paths: run lt_tag_batch_host or lt_beam first");
-    if (gold->tables != b->tables) return fail(LT_ERR_INVALID, "the gold path set belongs to other tables");
+    if (int rc = check_gold(b, gold)) return rc;
     lt_tables* t = b->tables;
     if (int rc = check_trigram_func(t, func)) return rc;
-    if (gold->n_paths != b->n_sent) return fail(LT_ERR_INVALID, "%d gold paths for %d sentences", gold->n_paths, b->n_sent);
     if ((size_t)n_delta != t->feat_dst.size())
         return fail(LT_ERR_INVALID, "the tables were built with %zu features, delta has %lld", t->feat_dst.size(), (long long)n_delta);
     if ((n_delta > 0 && !delta) || (b->n_sent > 0 && !differs)) return fail(LT_ERR_INVALID, "null output pointer");
@@ -1699,33 +1659,17 @@ extern "C" int lt_perceptron_delta(lt_batch* b, const lt_pathset* gold, int32_t 
     if (int rc = resolve(b)) return rc;
     cudaStream_t st = b->last_stream;
     const int n_sent = b->n_sent;
-    const size_t nu = (size_t)b->n_units;
-    if (!t->d_counts) CU(cudaMalloc(reinterpret_cast<void**>(&t->d_counts), n_hits(t) * 8));
+    PerceptronArgs A{};
+    if (int rc = search_and_gold(b, gold, &A.sg)) return rc;
+    if (int rc = ensure(t->d_counts, n_hits(t) * 8)) return rc;
     if (int rc = upload_feat_dst(t)) return rc;
-    if (int rc = ensure(b->pth_ch, std::max<size_t>(1, nu) * 2)) return rc;
-    if (int rc = ensure(b->pth_ha, (nu + n_sent + 1) * 8)) return rc;
-    if (int rc = ensure(b->pth_hb, (nu + n_sent + 1) * 8)) return rc;
     if (int rc = ensure(b->pc_delta, (size_t)std::max<int64_t>(1, n_delta) * 8)) return rc;
     if (int rc = ensure(b->pc_differs, (size_t)std::max(1, n_sent))) return rc;
     if (int rc = ensure(b->pc_count, 8)) return rc;
-    CU(cudaMemsetAsync(t->d_counts, 0, n_hits(t) * 8, st));
+    CU(cudaMemsetAsync(t->d_counts.p, 0, n_hits(t) * 8, st));
     CU(cudaMemsetAsync(b->pc_count.p, 0, 8, st));
-    PerceptronArgs A{};
-    A.text = b->d_text;
-    A.sent_off = b->d_sent_off;
-    A.n_sent = n_sent;
     A.func = func;
-    A.status = static_cast<const int32_t*>(b->status.p);
-    A.path_off = static_cast<const uint32_t*>(b->path_off.p);
-    A.path_edges = static_cast<const lt_edge*>(b->path_out.p);
-    A.imp = b->imported ? static_cast<const H2*>(b->imp.p) : nullptr;
-    A.gold_edges = gold->d_edges;
-    A.gold_off = gold->d_off;
-    A.gold_hashes = gold->d_hashes;
-    A.ch = static_cast<uint16_t*>(b->pth_ch.p);
-    A.ha = static_cast<uint64_t*>(b->pth_ha.p);
-    A.hb = static_cast<uint64_t*>(b->pth_hb.p);
-    A.counts = t->d_counts;
+    A.counts = static_cast<unsigned long long*>(t->d_counts.p);
     A.differs = static_cast<uint8_t*>(b->pc_differs.p);
     A.n_differ = static_cast<unsigned long long*>(b->pc_count.p);
     if (n_sent > 0) {
@@ -1735,7 +1679,8 @@ extern "C" int lt_perceptron_delta(lt_batch* b, const lt_pathset* gold, int32_t 
     }
     if (n_delta > 0) {
         const unsigned grid = (unsigned)std::min<int64_t>((n_delta + 255) / 256, (int64_t)t->sm_count * 16);
-        LT_LAUNCH(gather_counts, grid, 256, 0, st, t->d_counts, t->d_feat_dst, n_delta, feat_slots(t), static_cast<long long*>(b->pc_delta.p));
+        LT_LAUNCH(gather_counts, grid, 256, 0, st, A.counts, static_cast<const uint32_t*>(t->d_feat_dst.p), n_delta, feat_slots(t),
+                  static_cast<long long*>(b->pc_delta.p));
         CU(cudaGetLastError());
         b->launches += 1;
         CU(cudaMemcpyAsync(delta, b->pc_delta.p, (size_t)n_delta * 8, cudaMemcpyDeviceToHost, st));
@@ -1753,9 +1698,7 @@ extern "C" int lt_perceptron_delta(lt_batch* b, const lt_pathset* gold, int32_t 
 extern "C" int lt_evaluate(lt_batch* b, const lt_pathset* gold, uint8_t* sent_class, int32_t* counts, double* gold_scores,
                            uint8_t* word_reason) {
     if (!b || !gold) return fail(LT_ERR_INVALID, "null argument");
-    if (!b->have_paths) return fail(LT_ERR_INVALID, "no paths: run a search (lt_tag_batch_host, lt_beam, ...) first");
-    if (gold->tables != b->tables) return fail(LT_ERR_INVALID, "the gold path set belongs to other tables");
-    if (gold->n_paths != b->n_sent) return fail(LT_ERR_INVALID, "%d gold paths for %d sentences", gold->n_paths, b->n_sent);
+    if (int rc = check_gold(b, gold)) return rc;
     if (!gold->ordered) return fail(LT_ERR_INVALID, "a gold path has a word with b >= e or a b that does not increase");
     if (b->n_sent > 0 && !sent_class) return fail(LT_ERR_INVALID, "null output pointer");
     lt_tables* t = b->tables;
@@ -1763,11 +1706,9 @@ extern "C" int lt_evaluate(lt_batch* b, const lt_pathset* gold, uint8_t* sent_cl
     if (int rc = resolve(b)) return rc;
     cudaStream_t st = b->last_stream;
     const int n_sent = b->n_sent;
-    const size_t nu = (size_t)b->n_units;
     const size_t nw = (size_t)gold->n_words;
-    if (int rc = ensure(b->pth_ch, std::max<size_t>(1, nu) * 2)) return rc;
-    if (int rc = ensure(b->pth_ha, (nu + n_sent + 1) * 8)) return rc;
-    if (int rc = ensure(b->pth_hb, (nu + n_sent + 1) * 8)) return rc;
+    EvaluateArgs A{};
+    if (int rc = search_and_gold(b, gold, &A.sg)) return rc;
     if (int rc = ensure(b->ev_image, std::max<size_t>(1, nw) * sizeof(lt_edge))) return rc;
     if (int rc = ensure(b->ev_class, (size_t)std::max(1, n_sent))) return rc;
     if (counts)
@@ -1776,23 +1717,9 @@ extern "C" int lt_evaluate(lt_batch* b, const lt_pathset* gold, uint8_t* sent_cl
         if (int rc = ensure(b->ev_scores, (size_t)std::max(1, n_sent) * 8)) return rc;
     if (word_reason)
         if (int rc = ensure(b->ev_reason, std::max<size_t>(1, nw))) return rc;
-    EvaluateArgs A{};
-    A.text = b->d_text;
-    A.sent_off = b->d_sent_off;
-    A.n_sent = n_sent;
-    A.status = static_cast<const int32_t*>(b->status.p);
-    A.path_off = static_cast<const uint32_t*>(b->path_off.p);
-    A.path_edges = static_cast<const lt_edge*>(b->path_out.p);
     A.scores = static_cast<const double*>(b->scores.p);
     A.pos = static_cast<const uint2*>(b->pos.p);
     A.edges = static_cast<const lt_edge*>(b->edges.p);
-    A.imp = b->imported ? static_cast<const H2*>(b->imp.p) : nullptr;
-    A.gold_edges = gold->d_edges;
-    A.gold_off = gold->d_off;
-    A.gold_hashes = gold->d_hashes;
-    A.ch = static_cast<uint16_t*>(b->pth_ch.p);
-    A.ha = static_cast<uint64_t*>(b->pth_ha.p);
-    A.hb = static_cast<uint64_t*>(b->pth_hb.p);
     A.image = static_cast<lt_edge*>(b->ev_image.p);
     A.sent_class = static_cast<uint8_t*>(b->ev_class.p);
     A.counts = counts ? static_cast<int32_t*>(b->ev_counts.p) : nullptr;

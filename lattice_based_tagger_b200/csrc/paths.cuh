@@ -230,11 +230,11 @@ __global__ void __launch_bounds__(256) path_eval_kernel(const __grid_constant__ 
     }
 }
 
-struct PerceptronArgs {
+// What the perceptron and evaluation kernels read of the batch's last search and of the gold path set.
+struct SearchAndGold {
     const uint16_t* text;       // the batch's sentences (the last search)
     const int32_t* sent_off;
     int32_t n_sent;
-    int32_t func;               // the trigram scorer whose features are counted
     const int32_t* status;
     const uint32_t* path_off;   // best paths of the last search
     const lt_edge* path_edges;
@@ -245,6 +245,11 @@ struct PerceptronArgs {
     uint16_t* ch;               // scratch: syllables [n_units], prefix hashes [n_units + n_sent]
     uint64_t* ha;
     uint64_t* hb;
+};
+
+struct PerceptronArgs {
+    SearchAndGold sg;
+    int32_t func;               // the trigram scorer whose features are counted
     unsigned long long* counts; // per hit, two's complement
     uint8_t* differs;           // [n_sent]
     unsigned long long* n_differ;
@@ -255,19 +260,19 @@ struct PerceptronArgs {
 __global__ void __launch_bounds__(256) perceptron_kernel(const __grid_constant__ DevTables T, const __grid_constant__ PerceptronArgs A) {
     const int lane = threadIdx.x & 31;
     const int warps = (int)(gridDim.x * blockDim.x) >> 5;
-    for (int s = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5); s < A.n_sent; s += warps) {
-        const int st = A.status[s];
-        const int64_t go = A.gold_off[s];
-        const int G = (int)(A.gold_off[s + 1] - go);
-        const int s0 = A.sent_off[s], s1 = A.sent_off[s + 1];
-        const lt_edge* pred = A.path_edges + A.path_off[s];
-        const int P = (st == LT_SENT_OK) ? (int)(A.path_off[s + 1] - A.path_off[s]) : 0;
-        uint16_t* ch = A.ch + s0;
-        uint64_t* ha = A.ha + s0 + s;
-        uint64_t* hb = A.hb + s0 + s;
-        if (st == LT_SENT_OK) stage_sentence_hashes(A.text, s0, s1, lane, ch, ha, hb);
-        const SentView pv{ch, ha, hb, nullptr, A.imp};
-        const SentView gv{nullptr, nullptr, nullptr, nullptr, A.gold_hashes};
+    for (int s = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5); s < A.sg.n_sent; s += warps) {
+        const int st = A.sg.status[s];
+        const int64_t go = A.sg.gold_off[s];
+        const int G = (int)(A.sg.gold_off[s + 1] - go);
+        const int s0 = A.sg.sent_off[s], s1 = A.sg.sent_off[s + 1];
+        const lt_edge* pred = A.sg.path_edges + A.sg.path_off[s];
+        const int P = (st == LT_SENT_OK) ? (int)(A.sg.path_off[s + 1] - A.sg.path_off[s]) : 0;
+        uint16_t* ch = A.sg.ch + s0;
+        uint64_t* ha = A.sg.ha + s0 + s;
+        uint64_t* hb = A.sg.hb + s0 + s;
+        if (st == LT_SENT_OK) stage_sentence_hashes(A.sg.text, s0, s1, lane, ch, ha, hb);
+        const SentView pv{ch, ha, hb, nullptr, A.sg.imp};
+        const SentView gv{nullptr, nullptr, nullptr, nullptr, A.sg.gold_hashes};
         bool differ = st != LT_SENT_OK || P != G;
         for (int base = 0; base < P && !differ; base += 32) {
             const int w = base + lane;
@@ -276,7 +281,7 @@ __global__ void __launch_bounds__(256) perceptron_kernel(const __grid_constant__
                 EdgeView k, g;
                 unpack_edge(ldg16(pred + w), k);
                 edge_hashes_inline<1>(T, pv, k, true);
-                unpack_edge(ldg16(A.gold_edges + go + w), g);
+                unpack_edge(ldg16(A.sg.gold_edges + go + w), g);
                 edge_hashes_inline<1>(T, gv, g, true);
                 mismatch = k.b != g.b || k.e != g.e || k.tag0 != g.tag0 || k.tag1 != g.tag1 || k.mk.a != g.mk.a || k.mk.b != g.mk.b ||
                            k.m1.a != g.m1.a || k.m1.b != g.m1.b;
@@ -294,7 +299,7 @@ __global__ void __launch_bounds__(256) perceptron_kernel(const __grid_constant__
                         if (hit[i] != kNoHit) atomicAdd(A.counts + hit[i], delta);
                 };
             };
-            walk_path(T, A.gold_edges + go, G, gv, lane, count(1ull));
+            walk_path(T, A.sg.gold_edges + go, G, gv, lane, count(1ull));
             if (st == LT_SENT_OK) walk_path(T, pred, P, pv, lane, count(~0ull));     // -1
         }
         if (lane == 0) {

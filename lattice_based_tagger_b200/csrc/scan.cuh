@@ -42,7 +42,6 @@ __device__ __forceinline__ uint32_t block_exclusive_scan(uint32_t v, uint32_t* w
 
 // pass 1: per-tile sums
 __global__ void __launch_bounds__(kScanThreads) scan_tile_sums(const uint32_t* __restrict__ in, int64_t n, uint32_t* __restrict__ sums) {
-    lt_pdl_wait();
     __shared__ uint32_t ws[kScanThreads / 32 + 1];
     const int64_t base = (int64_t)blockIdx.x * kScanTile + (int64_t)threadIdx.x * kScanItems;
     uint32_t local = 0;
@@ -93,7 +92,6 @@ __global__ void __launch_bounds__(kScanThreads) scan_apply(const uint32_t* __res
 constexpr int kScanSmallThreads = 1024;
 constexpr int64_t kScanSmallMax = 64 * 1024;
 __global__ void __launch_bounds__(kScanSmallThreads) scan_small(const uint32_t* __restrict__ in, uint32_t* __restrict__ out, int64_t n) {
-    lt_pdl_wait();
     __shared__ uint32_t warp_sums[33];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int64_t per = (n + kScanSmallThreads - 1) / kScanSmallThreads;
@@ -147,8 +145,6 @@ __global__ void __launch_bounds__(1024) batch_prologue(const int32_t* __restrict
                                                        uint32_t* __restrict__ order, unsigned int* __restrict__ ctl, int n_ctl,
                                                        unsigned long long* __restrict__ counters, int n_counters) {
     const int G = (int)gridDim.x, g = (int)blockIdx.x;
-    lt_pdl_trigger();
-    lt_pdl_wait();
     if (g == 0) {
         if ((int)threadIdx.x < n_ctl) ctl[threadIdx.x] = 0;
         if ((int)threadIdx.x < n_counters) counters[threadIdx.x] = 0;
@@ -217,7 +213,6 @@ __global__ void beam_reset(unsigned int* __restrict__ queue, unsigned long long*
 // best paths: reversed per-sentence scratch -> contiguous forward order
 __global__ void pack_paths(const lt_edge* __restrict__ tmp, const int32_t* __restrict__ sent_off,
                            const uint32_t* __restrict__ path_off, int32_t n_sent, lt_edge* __restrict__ out) {
-    lt_pdl_wait();
     const int warps_per_block = blockDim.x >> 5;
     const int lane = threadIdx.x & 31;
     for (int s = blockIdx.x * warps_per_block + (threadIdx.x >> 5); s < n_sent; s += gridDim.x * warps_per_block) {
@@ -242,8 +237,6 @@ __global__ void __launch_bounds__(kPackScanThreads) pack_paths_scan(const lt_edg
     __shared__ uint32_t warp_sums[kPackScanThreads / 32 + 1];
     __shared__ uint32_t s_off[kPackScanThreads + 1];
     const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
-    lt_pdl_trigger();
-    lt_pdl_wait();          // the beam kernel's paths are complete
     const int r0 = (int)blockIdx.x * per;
     const int r1 = min(n_sent, r0 + per);
     if (r0 >= n_sent) return;

@@ -425,7 +425,7 @@ class Engine:
         return t.as_dict()
 
     def set_stage_timing(self, on):
-        """Per-stage CUDA events between the kernels of a batch on / off (off: programmatic dependent launches)."""
+        """Per-stage CUDA events between the kernels of a batch on / off."""
         _native.check(self._lib.lt_batch_set_stage_timing(self.batch, 1 if on else 0))
 
     def info(self):

@@ -304,8 +304,7 @@ class Tagger:
         return self._engine.timings()
 
     def set_stage_timing(self, on):
-        """Per-stage events on / off for the batches to come; off lets the kernels of a batch overlap their
-        launch prologues with their predecessors' tails (programmatic dependent launch)."""
+        """Per-stage events between the kernels of a batch on / off for the batches to come."""
         self._engine.set_stage_timing(on)
 
     def info(self):

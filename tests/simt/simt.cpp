@@ -215,6 +215,8 @@ static void guarded_free(void* p) {
     munmap(it->second.base, it->second.len);
     g_guarded.erase(it);
 }
+// the device buffers live under LT_SIMT_MEMCHECK=1: a leak check compares the count before and after
+extern "C" size_t simt_live_buffers() { return g_guarded.size(); }
 
 void* dev_alloc(size_t n) {
     if (memcheck()) return guarded_alloc(n ? n : 1, fill_byte(0xCD));
