@@ -18,6 +18,8 @@
  *   lt_perceptron_delta <- the trainer's epoch (trainer/train.py:61-65): phi(gold) - phi(predicted).
  *   lt_evaluate        <- comparing the tagger's output with an annotated corpus (the trainer's loss,
  *                         word-level matches, and why a wrong sentence is wrong).
+ *   lt_trainer_*       <- an online, averaged perceptron in mini-batches: the weights and their running
+ *                         average stay on the device between steps.
  *
  * Plain pointers and sizes only.  No function throws; each returns LT_OK or an LT_ERR_* code and
  * lt_last_error() returns the message of the calling thread's last failure.
@@ -32,7 +34,7 @@
 extern "C" {
 #endif
 
-#define LT_ABI_VERSION 5
+#define LT_ABI_VERSION 6
 
 /* return codes */
 #define LT_OK            0
@@ -382,6 +384,42 @@ int  lt_perceptron_delta(lt_batch* batch, const lt_pathset* gold, int32_t func, 
  * synchronous. */
 int  lt_evaluate(lt_batch* batch, const lt_pathset* gold, uint8_t* sent_class, int32_t* counts,
                  double* gold_scores, uint8_t* word_reason);
+
+/* Mini-batch perceptron training on the device.  The trainer keeps the weights in coefficient space, w[n_coef]
+ * (indexed like the encoder's feature_dic, which need not be one-to-one), and u[n_coef] for the average.  Step
+ * t = 1, 2, ... decodes sentences [first, first + count) of the corpus with the current tables, takes delta as
+ * lt_perceptron_delta does (per sentence that differs: phi(gold) - phi(best), only phi(gold) when the status is
+ * not LT_SENT_OK; desc feature f of `func` adds to coefficient feat_coef[f]), then
+ *     w += delta,   u += (t - 1) * delta,
+ * and writes w[feat_coef[f]] into the tables for every feature f of `func` with feat_coef[f] >= 0 (hashed slots
+ * and dense blocks).  A step without a mistake still counts.  The averaged weights after T steps are
+ * w - u / T, the mean of the weights after steps 1 .. T.  Counts are exact integers, so w and u are the same
+ * whatever the order of the atomic adds.
+ *
+ * lt_trainer_create  corpus `text` / `sent_off` (n_sent + 1 offsets, sent_off[0] = 0, non-decreasing) in host
+ *                    memory, uploaded once; `gold` one path per corpus sentence (gold->n_paths == n_sent), on the
+ *                    same tables, and it must outlive the trainer; `func` a trigram scorer;
+ *                    feat_coef[desc->n_feat] the coefficient of each desc feature of `func` (-1: not trained, its
+ *                    weight stays), -1 for every feature of another scorer; coef[n_coef] = w_0, written into the
+ *                    tables here (synchronous, no batch may be in flight on the tables).
+ * lt_trainer_step    one step on `batch` (same tables): the slice is copied and searched on the batch's own stream
+ *                    (one host wait, for the lattice-overflow check), then compared and applied there without a
+ *                    copy to or from the host.  Afterwards the batch holds the slice as its last search:
+ *                    lt_paths_fetch, lt_evaluate etc. work on it, also after lt_trainer_destroy.  The step writes
+ *                    the tables and the tables' count buffer: no other search, lt_perceptron_delta or trainer step
+ *                    on the same tables may run meanwhile, and lt_tables_update_weights afterwards rewrites every
+ *                    weight, dense blocks included.
+ * lt_trainer_fetch   waits for the last step; any pointer may be NULL.  coef / averaged: n_coef doubles
+ *                    (averaged = w while no step has run); steps; mistakes: sentences that differed, summed over
+ *                    all steps; differs[n_sent]: per corpus sentence, from the last step that covered it (0 before). */
+typedef struct lt_trainer lt_trainer;
+int  lt_trainer_create(lt_tables* tables, int32_t func, const uint16_t* text, const int32_t* sent_off, int32_t n_sent,
+                       const lt_pathset* gold, int64_t n_coef, const int64_t* feat_coef, const double* coef,
+                       lt_trainer** out);
+int  lt_trainer_step(lt_trainer* trainer, lt_batch* batch, int32_t first, int32_t count, int32_t beam_size);
+int  lt_trainer_fetch(lt_trainer* trainer, double* coef, double* averaged, int64_t* steps, int64_t* mistakes,
+                      uint8_t* differs);
+void lt_trainer_destroy(lt_trainer* trainer);
 
 #ifdef __cplusplus
 }

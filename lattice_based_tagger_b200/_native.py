@@ -13,7 +13,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, 'liblt_b200.so')
 
-LT_ABI_VERSION = 5
+LT_ABI_VERSION = 6
 LT_OK = 0
 LT_SENT_OK, LT_SENT_NO_EDGES, LT_SENT_BAD_SPACE, LT_SENT_TOO_LONG, LT_SENT_UNSUPPORTED_CHAR = 0, 1, 2, 3, 4
 LT_NO_TAG = 0xFF
@@ -124,6 +124,10 @@ SYMBOLS = {
     'lt_pathset_eval': (ctypes.c_int, [_p, _p, ctypes.c_int32, _p, _p, _p, ctypes.c_int64]),
     'lt_perceptron_delta': (ctypes.c_int, [_p, _p, ctypes.c_int32, _p, ctypes.c_int64, _p, ctypes.POINTER(ctypes.c_int64)]),
     'lt_evaluate': (ctypes.c_int, [_p, _p, _p, _p, _p, _p]),
+    'lt_trainer_create': (ctypes.c_int, [_p, ctypes.c_int32, _p, _p, ctypes.c_int32, _p, ctypes.c_int64, _p, _p, ctypes.POINTER(_p)]),
+    'lt_trainer_step': (ctypes.c_int, [_p, _p, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32]),
+    'lt_trainer_fetch': (ctypes.c_int, [_p, _p, _p, ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int64), _p]),
+    'lt_trainer_destroy': (None, [_p]),
 }
 
 _lib = None

@@ -21,6 +21,7 @@
 #include "paths.cuh"
 #include "scan.cuh"
 #include "tables.cuh"
+#include "train.cuh"
 
 using namespace lt;
 
@@ -118,6 +119,7 @@ struct lt_tables {
     // where the weight of input feature i lives (lt_tables_update_weights): a slot of the hashed table, an offset into
     // the dense blocks (kDstDense | byte offset / 8), or kDstNone for a feature no tuple can equal
     std::vector<uint32_t> feat_dst;
+    std::vector<uint8_t> feat_func;                    // owning scorer of input feature i (lt_trainer_create's check)
     std::vector<unsigned char> dense_host;
     DevBuf d_feat_dst, d_weights;
     // path sets (paths.cuh): a feature hit is a slot of the hashed table or feat_slots + a dense offset; per hit the
@@ -337,6 +339,7 @@ static int build_tables(const lt_tables_desc* d, lt_tables* t) {
     std::vector<int64_t> pending_src;                    // input feature of a hashed entry (-1: a preference)
     pending.reserve((size_t)(d->n_feat + d->n_pref));
     t->feat_dst.assign((size_t)d->n_feat, kDstNone);
+    t->feat_func.assign(d->feat_func, d->feat_func + d->n_feat);
     for (int64_t i = 0; i < d->n_feat; ++i) {
         const int f = d->feat_func[i];
         if (f >= d->n_funcs || D.func_dense[f] < 0) return fail(LT_ERR_INVALID, "feature %lld belongs to scorer %d which is not a trigram scorer", (long long)i, f);
@@ -1735,5 +1738,188 @@ extern "C" int lt_evaluate(lt_batch* b, const lt_pathset* gold, uint8_t* sent_cl
         if (word_reason && nw > 0) CU(cudaMemcpyAsync(word_reason, A.word_reason, nw, cudaMemcpyDeviceToHost, st));
     }
     CU(cudaStreamSynchronize(st));
+    return LT_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// mini-batch perceptron (train.cuh): weights and their running average in device memory
+// ------------------------------------------------------------------------------------------------
+struct lt_trainer {
+    lt_tables* tables = nullptr;
+    int device = 0;
+    const lt_pathset* gold = nullptr;
+    int32_t func = 0;
+    int32_t n_sent = 0;
+    int64_t n_coef = 0;
+    int64_t steps = 0;
+    std::vector<int32_t> sent_off;          // host copy: the size and longest sentence of a step's slice
+    DevBuf text, off;                       // the corpus
+    DevBuf feat_coef, w, u, acc;            // [n_feat] coefficient of each desc feature; [n_coef] w, u, step counts
+    DevBuf differs, mistakes;               // [n_sent] flags of each sentence's last step; running count of mistakes
+    cudaEvent_t done = nullptr;             // recorded after the last kernel of every step
+};
+
+extern "C" void lt_trainer_destroy(lt_trainer* tr) {
+    if (!tr) return;
+    DeviceGuard guard(tr->device);      // (the tables may be gone already)
+    if (tr->done) cudaEventDestroy(tr->done);
+    delete tr;
+}
+
+static int zeroed(DevBuf& b, size_t bytes) {
+    if (int rc = ensure(b, std::max<size_t>(bytes, 16))) return rc;
+    CU(cudaMemsetAsync(b.p, 0, std::max<size_t>(bytes, 16), nullptr));
+    return LT_OK;
+}
+
+// the tables' weight of every trained feature := w[feat_coef[i]], on stream st
+static int scatter_trainer_weights(lt_trainer* tr, cudaStream_t st) {
+    lt_tables* t = tr->tables;
+    const int64_t n_feat = (int64_t)t->feat_dst.size();
+    if (n_feat == 0) return LT_OK;
+    const unsigned grid = (unsigned)std::min<int64_t>((n_feat + 255) / 256, (int64_t)t->sm_count * 16);
+    LT_LAUNCH(scatter_coef, grid, 256, 0, st, const_cast<FeatSlot*>(t->dev.feat),
+              reinterpret_cast<double*>(const_cast<unsigned char*>(t->dev.dense)), static_cast<const uint32_t*>(t->d_feat_dst.p),
+              static_cast<const int64_t*>(tr->feat_coef.p), n_feat, static_cast<const double*>(tr->w.p));
+    CU(cudaGetLastError());
+    return LT_OK;
+}
+
+extern "C" int lt_trainer_create(lt_tables* t, int32_t func, const uint16_t* text, const int32_t* sent_off, int32_t n_sent,
+                                 const lt_pathset* gold, int64_t n_coef, const int64_t* feat_coef, const double* coef,
+                                 lt_trainer** out) {
+    if (!t || !out || !gold || !sent_off || n_sent < 0 || n_coef < 0) return fail(LT_ERR_INVALID, "bad argument");
+    *out = nullptr;
+    if (int rc = check_trigram_func(t, func)) return rc;
+    if (gold->tables != t) return fail(LT_ERR_INVALID, "the gold path set belongs to other tables");
+    if (gold->n_paths != n_sent) return fail(LT_ERR_INVALID, "%d gold paths for %d sentences", gold->n_paths, n_sent);
+    if (sent_off[0] != 0) return fail(LT_ERR_INVALID, "sent_off[0] must be 0");
+    for (int32_t i = 0; i < n_sent; ++i)
+        if (sent_off[i + 1] < sent_off[i]) return fail(LT_ERR_INVALID, "sent_off is not monotone at %d", i);
+    const int64_t n_units = sent_off[n_sent];
+    const int64_t n_feat = (int64_t)t->feat_dst.size();
+    if ((n_units > 0 && !text) || (n_feat > 0 && !feat_coef) || (n_coef > 0 && !coef)) return fail(LT_ERR_INVALID, "null input pointer");
+    for (int64_t i = 0; i < n_feat; ++i) {
+        if (feat_coef[i] < -1 || feat_coef[i] >= n_coef)
+            return fail(LT_ERR_INVALID, "feat_coef[%lld] = %lld is outside [-1, %lld)", (long long)i, (long long)feat_coef[i], (long long)n_coef);
+        if (feat_coef[i] >= 0 && t->feat_func[(size_t)i] != func)
+            return fail(LT_ERR_INVALID, "feature %lld belongs to scorer %d, not to the trained scorer %d", (long long)i, t->feat_func[(size_t)i], func);
+    }
+    ON_DEVICE(t->device);
+    lt_trainer* tr = new lt_trainer();
+    tr->tables = t;
+    tr->device = t->device;
+    tr->gold = gold;
+    tr->func = func;
+    tr->n_sent = n_sent;
+    tr->n_coef = n_coef;
+    tr->sent_off.assign(sent_off, sent_off + n_sent + 1);
+    int rc = upload_once(tr->text, text, (size_t)n_units * 2);
+    if (rc == LT_OK) rc = upload_once(tr->off, sent_off, (size_t)(n_sent + 1) * 4);
+    if (rc == LT_OK) rc = upload_once(tr->feat_coef, feat_coef, (size_t)n_feat * 8);
+    if (rc == LT_OK) rc = upload_once(tr->w, coef, (size_t)n_coef * 8);
+    if (rc == LT_OK) rc = zeroed(tr->u, (size_t)n_coef * 8);
+    if (rc == LT_OK) rc = zeroed(tr->acc, (size_t)n_coef * 8);
+    if (rc == LT_OK) rc = zeroed(tr->differs, (size_t)n_sent);
+    if (rc == LT_OK) rc = zeroed(tr->mistakes, 8);
+    if (rc == LT_OK) rc = upload_feat_dst(t);
+    if (rc == LT_OK) rc = scatter_trainer_weights(tr, nullptr);
+    if (rc == LT_OK && cudaEventCreate(&tr->done) != cudaSuccess) rc = fail(LT_ERR_CUDA, "cudaEventCreate failed");
+    if (rc == LT_OK && cudaDeviceSynchronize() != cudaSuccess) rc = fail(LT_ERR_CUDA, "writing the initial weights failed");
+    if (rc != LT_OK) {
+        lt_trainer_destroy(tr);
+        return rc;
+    }
+    *out = tr;
+    return LT_OK;
+}
+
+// Decode the slice on the batch's stream (its text copied device to device into the batch's own buffers, so that
+// the batch does not point into the trainer), wait once for the lattice-overflow check, then compare with the gold
+// range and apply the update without leaving the device.
+extern "C" int lt_trainer_step(lt_trainer* tr, lt_batch* b, int32_t first, int32_t count, int32_t beam_size) {
+    if (!tr || !b) return fail(LT_ERR_INVALID, "null argument");
+    lt_tables* t = tr->tables;
+    if (b->tables != t) return fail(LT_ERR_INVALID, "the batch belongs to other tables");
+    if (count < 1 || first < 0 || (int64_t)first + count > tr->n_sent)
+        return fail(LT_ERR_INVALID, "sentences [%d, %lld) are not a non-empty range of the %d corpus sentences", first,
+                    (long long)first + count, tr->n_sent);
+    if (beam_size < 1 || beam_size > LT_MAX_BEAM) return fail(LT_ERR_INVALID, "beam_size must be in 1..%d", LT_MAX_BEAM);
+    ON_DEVICE(t->device);
+    cudaStream_t st = b->own_stream;
+    const int32_t* off = tr->sent_off.data() + first;
+    const int64_t n_units = (int64_t)off[count] - off[0];
+    int32_t max_units = 0;
+    for (int32_t i = 0; i < count; ++i) max_units = std::max(max_units, off[i + 1] - off[i]);
+    if (int rc = ensure(b->text, (size_t)std::max<int64_t>(1, n_units) * 2)) return rc;
+    if (int rc = ensure(b->sent_off, (size_t)(count + 1) * 4)) return rc;
+    if (n_units) CU(cudaMemcpyAsync(b->text.p, static_cast<const uint16_t*>(tr->text.p) + off[0], (size_t)n_units * 2, cudaMemcpyDeviceToDevice, st));
+    LT_LAUNCH(rebase_offsets, (unsigned)std::min<int64_t>(((int64_t)count + 256) / 256, (int64_t)t->sm_count), 256, 0, st,
+              static_cast<const int32_t*>(tr->off.p), first, count, static_cast<int32_t*>(b->sent_off.p));
+    CU(cudaGetLastError());
+    b->launches += 1;
+    bind_batch(b, static_cast<const uint16_t*>(b->text.p), static_cast<const int32_t*>(b->sent_off.p), count, n_units, max_units, st);
+    if (int rc = launch_lattice(b, st)) return rc;
+    b->beam = beam_size;
+    if (int rc = launch_beam(b, st, false)) return rc;
+    if (int rc = resolve(b)) return rc;
+
+    PerceptronArgs A{};
+    if (int rc = search_and_gold(b, tr->gold, &A.sg)) return rc;
+    A.sg.gold_off += first;                       // gold offsets are absolute word indices: the slice's paths start there
+    if (int rc = ensure(t->d_counts, n_hits(t) * 8)) return rc;
+    CU(cudaMemsetAsync(t->d_counts.p, 0, n_hits(t) * 8, st));
+    A.func = tr->func;
+    A.counts = static_cast<unsigned long long*>(t->d_counts.p);
+    A.differs = static_cast<uint8_t*>(tr->differs.p) + first;
+    A.n_differ = static_cast<unsigned long long*>(tr->mistakes.p);
+    LT_LAUNCH(perceptron_kernel, warp_grid(t, count), 256, 0, st, t->dev, A);
+    CU(cudaGetLastError());
+    b->launches += 1;
+
+    const int64_t step = ++tr->steps;
+    const int64_t n_feat = (int64_t)t->feat_dst.size();
+    const int64_t cap = (int64_t)t->sm_count * 16;
+    if (n_feat > 0) {
+        LT_LAUNCH(gather_coef_counts, (unsigned)std::min<int64_t>((n_feat + 255) / 256, cap), 256, 0, st, A.counts,
+                  static_cast<const uint32_t*>(t->d_feat_dst.p), static_cast<const int64_t*>(tr->feat_coef.p), n_feat, feat_slots(t),
+                  static_cast<unsigned long long*>(tr->acc.p));
+        CU(cudaGetLastError());
+        b->launches += 1;
+    }
+    if (tr->n_coef > 0) {
+        LT_LAUNCH(apply_coef_delta, (unsigned)std::min<int64_t>((tr->n_coef + 255) / 256, cap), 256, 0, st,
+                  static_cast<unsigned long long*>(tr->acc.p), tr->n_coef, (long long)(step - 1), static_cast<double*>(tr->w.p),
+                  static_cast<double*>(tr->u.p));
+        CU(cudaGetLastError());
+        b->launches += 1;
+    }
+    if (int rc = scatter_trainer_weights(tr, st)) return rc;
+    if (n_feat > 0) b->launches += 1;
+    CU(cudaEventRecord(tr->done, st));
+    return LT_OK;
+}
+
+extern "C" int lt_trainer_fetch(lt_trainer* tr, double* coef, double* averaged, int64_t* steps, int64_t* mistakes, uint8_t* differs) {
+    if (!tr) return fail(LT_ERR_INVALID, "null argument");
+    ON_DEVICE(tr->tables->device);
+    CU(cudaEventSynchronize(tr->done));
+    const size_t n = (size_t)tr->n_coef;
+    if (coef && n) CU(cudaMemcpy(coef, tr->w.p, n * 8, cudaMemcpyDeviceToHost));
+    if (averaged && n) {
+        // mean of the weights after steps 1 .. T: (T * w_T - sum_t (t - 1) * delta_t) / T
+        std::vector<double> u(n);
+        CU(cudaMemcpy(averaged, tr->w.p, n * 8, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(u.data(), tr->u.p, n * 8, cudaMemcpyDeviceToHost));
+        if (tr->steps > 0)
+            for (size_t c = 0; c < n; ++c) averaged[c] = averaged[c] - u[c] / (double)tr->steps;
+    }
+    if (steps) *steps = tr->steps;
+    if (mistakes) {
+        unsigned long long m = 0;
+        CU(cudaMemcpy(&m, tr->mistakes.p, 8, cudaMemcpyDeviceToHost));
+        *mistakes = (int64_t)m;
+    }
+    if (differs && tr->n_sent) CU(cudaMemcpy(differs, tr->differs.p, (size_t)tr->n_sent, cudaMemcpyDeviceToHost));
     return LT_OK;
 }

@@ -285,6 +285,10 @@ class Engine:
         """`paths[p]` = the `Word`s of path p without BOS / EOS -> a `PathSet` on these tables."""
         return PathSet(self, paths)
 
+    def trainer(self, sents, gold, func, n_coef, feat_coef, coef):
+        """A `DeviceTrainer` over `sents` (gold path i for sentence i) training scorer index `func`."""
+        return DeviceTrainer(self, sents, gold, func, n_coef, feat_coef, coef)
+
     def eval_paths(self, pathset, func=None):
         """lt_pathset_eval: (scores, feat_off, feat_idx); the features (of scorer index `func`, desc order)
         only with `func`, else (scores, None, None)."""
@@ -457,6 +461,58 @@ class PathSet:
     def close(self):
         if self.handle is not None:
             self._lib.lt_pathset_destroy(self.handle)
+            self.handle = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class DeviceTrainer:
+    """Mini-batch perceptron on the device (`lt_trainer`), tied to one `Engine`: the corpus `sents` and its gold
+    `PathSet` (which must stay open while the trainer lives) go up once; `step(first, count, beam_size)` decodes
+    sentences [first, first + count) on the engine's batch and updates the weights there; `fetch()` brings them
+    back.  `feat_coef[i]`: the coefficient of desc feature i (`CompiledTables.desc_sources` order) of scorer
+    `func`, -1 for the others; `coef`: the initial weights, written into the tables at once."""
+
+    def __init__(self, engine, sents, gold, func, n_coef, feat_coef, coef):
+        self._lib = engine._lib
+        self._engine = engine
+        self.handle = None
+        text, offsets = pack_sentences(sents)
+        feat_coef = np.ascontiguousarray(feat_coef, dtype=np.int64)
+        coef = np.ascontiguousarray(coef, dtype=np.float64)
+        if len(coef) != n_coef:
+            raise ValueError('%d initial weights for %d coefficients' % (len(coef), n_coef))
+        if len(feat_coef) != engine.tables.n_desc:
+            raise ValueError('feat_coef has %d entries, the tables %d features' % (len(feat_coef), engine.tables.n_desc))
+        handle = ctypes.c_void_p()
+        _native.check(self._lib.lt_trainer_create(
+            engine.tables.handle, int(func), _native.ptr(text), _native.ptr(offsets), len(sents), gold.handle, int(n_coef),
+            _native.ptr(feat_coef) if feat_coef.size else None, _native.ptr(coef) if coef.size else None, ctypes.byref(handle)))
+        self.handle = handle
+        self.n_sent = len(sents)
+        self.n_coef = int(n_coef)
+
+    def step(self, first, count, beam_size):
+        _native.check(self._lib.lt_trainer_step(self.handle, self._engine.batch, int(first), int(count), int(beam_size)))
+
+    def fetch(self):
+        """-> (coef, averaged, steps, mistakes, differs): the weights, their mean over the steps so far, the number
+        of steps, of mistaken sentences summed over them, and per sentence whether its last step got it wrong."""
+        coef = np.zeros(max(1, self.n_coef), dtype=np.float64)
+        averaged = np.zeros_like(coef)
+        differs = np.zeros(max(1, self.n_sent), dtype=np.uint8)
+        steps, mistakes = ctypes.c_int64(), ctypes.c_int64()
+        _native.check(self._lib.lt_trainer_fetch(self.handle, _native.ptr(coef), _native.ptr(averaged), ctypes.byref(steps),
+                                                 ctypes.byref(mistakes), _native.ptr(differs)))
+        return coef[:self.n_coef], averaged[:self.n_coef], int(steps.value), int(mistakes.value), differs[:self.n_sent].astype(bool)
+
+    def close(self):
+        if self.handle is not None:
+            self._lib.lt_trainer_destroy(self.handle)
             self.handle = None
 
     def __del__(self):

@@ -15,6 +15,10 @@ with phi = counts of the trigram features of a path (`SimpleTrigramEncoder.encod
 updates of one epoch are summed).  The gold paths go to the device once per `fit_parameter` call; an
 epoch is then a weight update, one decode of the corpus and one `lt_perceptron_delta` call, which
 compares every prediction with its gold path and counts the features of both on the device.
+
+With `batch_size` the perceptron is online instead: the corpus is cut into consecutive mini-batches, and
+each one is decoded with the weights the previous ones left (`lt_trainer_step`), optionally averaged over
+all steps.  The weights and their running average then stay on the device for the whole run.
 There is no CPU decoder: without the CUDA library `Tagger` raises.
 """
 
@@ -46,8 +50,9 @@ def _same_path(predicted, gold):
 
 def train(word_morph_pairs, dictionary, encoder, score_func, regularity_func,
           max_epochs=100, min_feature_count=1, predefined_features=None,
-          verbose=False, debug=False, beam_size=5, device=0):
-    """Reference `train()` (`trainer/train.py:1-42`): -> {'idx_to_feature': [...], 'coefficient': [...]}"""
+          verbose=False, debug=False, beam_size=5, device=0, batch_size=None, averaged=False):
+    """Reference `train()` (`trainer/train.py:1-42`): -> {'idx_to_feature': [...], 'coefficient': [...]}
+    `batch_size` and `averaged` are passed to `fit_parameter`."""
     word_morph_pairs = list(word_morph_pairs)
     if verbose:
         print('Scanning features ...')
@@ -67,7 +72,8 @@ def train(word_morph_pairs, dictionary, encoder, score_func, regularity_func,
     if verbose:
         print('Estimating parameter ...')
     try:
-        coef = fit_parameter(word_morph_pairs, encoder, tagger, max_epochs, verbose=verbose, beam_size=beam_size)
+        coef = fit_parameter(word_morph_pairs, encoder, tagger, max_epochs, verbose=verbose, beam_size=beam_size,
+                             averaged=averaged, batch_size=batch_size)
     finally:
         tagger.close()
 
@@ -158,11 +164,15 @@ def evaluate(word_morph_pairs, tagger, beam_size=5):
 
 
 def fit_parameter(word_morph_pairs, encoder, tagger, max_epochs=100, verbose=False, beam_size=5, patience=5,
-                  averaged=False):
+                  averaged=False, batch_size=None):
     """Reference `fit_parameter()` (`train.py:44-59`).  Stops once an epoch makes no mistake, or when the
     number of mistakes has not improved for `patience` epochs (a corpus with an unreachable gold path — a word the
     dictionary cannot produce — never reaches zero); returns the best weights seen (`averaged=True`: the mean of
-    the weights of all epochs, the averaged perceptron)."""
+    the weights of all epochs, the averaged perceptron).
+
+    With an integer `batch_size`: mini-batch perceptron steps on the device, see `_fit_minibatch`."""
+    if batch_size is not None:
+        return _fit_minibatch(word_morph_pairs, encoder, tagger, max_epochs, verbose, beam_size, patience, averaged, batch_size)
     coef = np.zeros(len(encoder.feature_dic), dtype=np.float64)
     best_loss, best_coef, stale = None, coef, 0
     total = np.zeros_like(coef)
@@ -186,6 +196,57 @@ def fit_parameter(word_morph_pairs, encoder, tagger, max_epochs=100, verbose=Fal
     if averaged:
         return total / max(1, epochs)
     return best_coef
+
+
+def _fit_minibatch(word_morph_pairs, encoder, tagger, max_epochs, verbose, beam_size, patience, averaged, batch_size):
+    """The online perceptron: the sentences the device can compare, in corpus order, cut into consecutive mini-batches
+    of `batch_size` (the last one may be shorter); every epoch walks them in that order, one `lt_trainer_step` each.
+    An epoch's loss is its number of mistakes; it stops on loss 0 or after `patience` epochs without a new minimum.
+    Returns the weights after the last step (`averaged=True`: their mean over all steps) — not the "best" ones, since an
+    online epoch's mistakes measure no single weight vector — and leaves them in the scorer and the tables.  Pairs the
+    device cannot compare are left out."""
+    if tagger.eojeol_lookup.flatten:
+        raise ValueError('mini-batch training does not support a flatten=True lookup: its lattices hold single-morpheme words')
+    if int(batch_size) != batch_size or batch_size < 1:
+        raise ValueError('batch_size must be a positive integer, got %r' % (batch_size,))
+    batch_size = int(batch_size)
+    coef = np.zeros(len(encoder.feature_dic), dtype=np.float64)
+    scorer = _load_weights(tagger, encoder, coef)
+    word_morph_pairs = list(word_morph_pairs)
+    gold = _GoldCorpus(word_morph_pairs, tagger)
+    try:
+        n = len(gold.device_idx)
+        if verbose:
+            print('mini-batch training on %d of %d pairs (%d left out: malformed, outside the BMP or an unknown tag)'
+                  % (n, len(word_morph_pairs), len(word_morph_pairs) - n))
+        if n:
+            engine = tagger._engine
+            func = tagger.score_funcs.funcs.index(scorer)
+            desc_func, desc_fdic = engine.tables.desc_sources()
+            feat_coef = np.where(desc_func == func, desc_fdic, -1)
+            trainer = engine.trainer(gold.device_sents, gold.pathset, func, len(coef), feat_coef, coef)
+            try:
+                best_loss, stale, seen = None, 0, 0
+                for epoch in range(1, max_epochs + 1):
+                    for first in range(0, n, batch_size):
+                        trainer.step(first, min(batch_size, n - first), beam_size)
+                    w, mean, steps, mistakes, _ = trainer.fetch()
+                    loss, seen = mistakes - seen, mistakes
+                    if verbose:
+                        print('epoch %d: %d of %d sentences differ from the annotation (%d steps)' % (epoch, loss, n, steps))
+                    if best_loss is None or loss < best_loss:
+                        best_loss, stale = loss, 0
+                    else:
+                        stale += 1
+                    if loss == 0 or stale >= patience:
+                        break
+                coef = mean if averaged else w
+            finally:
+                trainer.close()
+    finally:
+        gold.close()
+    _load_weights(tagger, encoder, coef)
+    return coef
 
 
 def _trigram_scorer(tagger):
