@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define LT_ABI_VERSION 6
+#define LT_ABI_VERSION 7
 
 /* return codes */
 #define LT_OK            0
@@ -420,6 +420,31 @@ int  lt_trainer_step(lt_trainer* trainer, lt_batch* batch, int32_t first, int32_
 int  lt_trainer_fetch(lt_trainer* trainer, double* coef, double* averaged, int64_t* steps, int64_t* mistakes,
                       uint8_t* differs);
 void lt_trainer_destroy(lt_trainer* trainer);
+
+/* The update a trainer step makes for a sentence that differs and has status LT_SENT_OK (every other sentence is
+ * updated as above in every mode; which sentences differ, the mistakes and the w / u bookkeeping do not change).
+ * Let gold words 1..W end at e_1 < ... < e_W = L (e_0 = 0), R_m the ranks the search kept at end position e_m whose
+ * hypothesis equals gold words 1..m on (b, e, tags, morphemes) (R_0 = {0}), B_m the score of rank 0 at e_m and G_m
+ * the score of gold words 1..m as lt_pathset_eval sums it.  The update is phi(gold words 1..m*) - phi(the rank-0
+ * hypothesis at e_{m*}) with
+ *   LT_UPDATE_FULL           m* = W: phi(gold) - phi(best path), the default
+ *   LT_UPDATE_EARLY          m* = the first m with R_m empty, else W (Collins and Roark 2004)
+ *   LT_UPDATE_MAX_VIOLATION  m* = the m with 0 not in R_m that maximises B_m - G_m, ties to the larger m
+ *                            (Huang, Fayong and Guo 2012)
+ * A gold path that does not tile [0, L) with non-empty words (lt_evaluate: LT_GOLD_BREAKS_TILING) gets m* = W.
+ * EARLY and MAX_VIOLATION steps keep the search's back-pointers in HBM and read them there.
+ *
+ * lt_trainer_set_update    the mode of the steps that follow; LT_ERR_INVALID for an unknown mode.
+ * lt_trainer_fetch_update  waits for the last step; per corpus sentence, from the last step that covered it (either
+ *                          pointer may be NULL): prefix_words[n_sent] = m* (0 when the sentence did not differ or was
+ *                          never covered, W for a full update, also when the status is not LT_SENT_OK);
+ *                          violation[n_sent] = B_{m*} - G_{m*}, NaN where there was no update, a FULL step, or the
+ *                          tiling fallback. */
+#define LT_UPDATE_FULL          0
+#define LT_UPDATE_EARLY         1
+#define LT_UPDATE_MAX_VIOLATION 2
+int  lt_trainer_set_update(lt_trainer* trainer, int32_t mode);
+int  lt_trainer_fetch_update(lt_trainer* trainer, int32_t* prefix_words, double* violation);
 
 #ifdef __cplusplus
 }

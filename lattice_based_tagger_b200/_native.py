@@ -13,7 +13,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, 'liblt_b200.so')
 
-LT_ABI_VERSION = 6
+LT_ABI_VERSION = 7
 LT_OK = 0
 LT_SENT_OK, LT_SENT_NO_EDGES, LT_SENT_BAD_SPACE, LT_SENT_TOO_LONG, LT_SENT_UNSUPPORTED_CHAR = 0, 1, 2, 3, 4
 LT_NO_TAG = 0xFF
@@ -30,6 +30,7 @@ LT_GOLD_UNCHECKED = 0xFF
 (LT_EVAL_GOLD_WORDS, LT_EVAL_PRED_WORDS, LT_EVAL_SEG, LT_EVAL_TAG, LT_EVAL_FULL, LT_EVAL_GOLD_UNITS, LT_EVAL_PRED_UNITS,
  LT_EVAL_UNIT_MATCH) = range(8)
 LT_EVAL_N_COUNTS = 8
+LT_UPDATE_FULL, LT_UPDATE_EARLY, LT_UPDATE_MAX_VIOLATION = range(3)
 LT_MAX_FUNCS = 8
 
 #: numpy view of `lt_edge` (16 bytes)
@@ -128,6 +129,8 @@ SYMBOLS = {
     'lt_trainer_step': (ctypes.c_int, [_p, _p, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32]),
     'lt_trainer_fetch': (ctypes.c_int, [_p, _p, _p, ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int64), _p]),
     'lt_trainer_destroy': (None, [_p]),
+    'lt_trainer_set_update': (ctypes.c_int, [_p, ctypes.c_int32]),
+    'lt_trainer_fetch_update': (ctypes.c_int, [_p, _p, _p]),
 }
 
 _lib = None

@@ -10,6 +10,8 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <limits>
+#include <mutex>
 #include <string>
 #include <vector>
 
@@ -22,6 +24,7 @@
 #include "scan.cuh"
 #include "tables.cuh"
 #include "train.cuh"
+#include "violation.cuh"
 
 using namespace lt;
 
@@ -114,8 +117,6 @@ struct lt_tables {
     std::vector<void*> allocations;
     int64_t bytes = 0;
     int sm_count = 0;
-    // kernels whose dynamic shared-memory limit was already raised on this device (function, bytes)
-    std::vector<std::pair<const void*, size_t>> smem_limits;
     // where the weight of input feature i lives (lt_tables_update_weights): a slot of the hashed table, an offset into
     // the dense blocks (kDstDense | byte offset / 8), or kDstNone for a feature no tuple can equal
     std::vector<uint32_t> feat_dst;
@@ -471,7 +472,7 @@ struct LatticePlan {
 };
 struct BeamPlan {
     int units = 0, beam = 0;                  // key
-    bool kbest = false;
+    bool kbest = false, hbm_trail = false;
     void (*fn)(const DevTables, const BeamArgs) = nullptr;
     int warps = 0, per_sm = 1;
     size_t smem = 0, warp_smem = 0;
@@ -513,6 +514,7 @@ struct lt_batch {
     bool edge_cap_fixed = false;   // LT_EDGE_CAP given: start there instead of the size guess (tests)
     bool debug = false;            // LT_DEBUG: print launch shapes
     bool trail_smem_ok = true;     // LT_TRAIL_SMEM=0 keeps the back-pointers in HBM
+    bool hbm_trail = false;        // a trainer step that reads the back-pointers: HBM, 0xFF before every search of the step
     int adapt_div = 32;            // LT_ADAPT_DIV: the main pass's staging area doubles when more than n_sent / this many eojeols
                                    // needed the retry pass (0 = never; measured on C3: the default is right)
     int sort_min = kSortMin;       // LT_SORT_MIN: staged hits per eojeol from which the lattice kernel ranks by sorting (tests: 1)
@@ -644,11 +646,17 @@ static int scan_u32(lt_batch* b, const uint32_t* in, uint32_t* out, int64_t n, c
     return LT_OK;
 }
 
-// raise a kernel's dynamic shared-memory limit once per device (and again only when more is needed)
+// raise a kernel's dynamic shared-memory limit once per device (and again only when more is needed).  The limit
+// belongs to the function on the device, not to the tables: the cache is keyed by (device, function) and shared by all
+// tables, or a second tables' smaller request would lower the limit below what the first one's plans were sized for.
+// (One cache per kernel signature Fn; the function pointer in the key tells the instantiations apart.)
 template <typename Fn>
 static int smem_limit(lt_tables* t, Fn fn, size_t bytes) {
-    const void* key = reinterpret_cast<const void*>(fn);
-    for (auto& kv : t->smem_limits)
+    static std::mutex mu;
+    static std::vector<std::pair<std::pair<int, const void*>, size_t>> limits;
+    std::lock_guard<std::mutex> lock(mu);
+    const std::pair<int, const void*> key(t->device, reinterpret_cast<const void*>(fn));
+    for (auto& kv : limits)
         if (kv.first == key) {
             if (kv.second >= bytes) return LT_OK;
             CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
@@ -656,7 +664,7 @@ static int smem_limit(lt_tables* t, Fn fn, size_t bytes) {
             return LT_OK;
         }
     CU(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    t->smem_limits.emplace_back(key, bytes);
+    limits.emplace_back(key, bytes);
     return LT_OK;
 }
 
@@ -722,7 +730,7 @@ static int beam_plan(lt_batch* b, int lcap, int beam_size, bool kbest, const Bea
     const int uclass = (!kbest && (beam_size == 5 || beam_size == 10)) ? beam_units_class(lcap) : 0;
     const int units = uclass ? uclass : lcap + 8;
     for (const BeamPlan& p : b->beam_plans)
-        if (p.units == units && p.beam == beam_size && p.kbest == kbest) { *out = &p; return LT_OK; }
+        if (p.units == units && p.beam == beam_size && p.kbest == kbest && p.hbm_trail == b->hbm_trail) { *out = &p; return LT_OK; }
     const size_t dense_bytes = ((size_t)t->dev.n_tri * dense_block_bytes(t->dev.n_tags) + 15) & ~(size_t)15;
     const bool reg_tri = t->dev.n_funcs == 2 && t->dev.funcs[0].kind == LT_FUNC_REG && t->dev.funcs[1].kind == LT_FUNC_TRIGRAM;
     const bool prog1 = reg_tri && !kbest;                      // the instantiation specialised for that score program
@@ -754,7 +762,8 @@ static int beam_plan(lt_batch* b, int lcap, int beam_size, bool kbest, const Bea
     P.units = units;
     P.beam = beam_size;
     P.kbest = kbest;
-    P.trail_smem = b->trail_smem_ok && w_own > 0 && resident_warps(smem_own_trail, w_own) >= resident_warps(smem_hbm_trail, w_hbm);
+    P.hbm_trail = b->hbm_trail;
+    P.trail_smem = !b->hbm_trail && b->trail_smem_ok && w_own > 0 && resident_warps(smem_own_trail, w_own) >= resident_warps(smem_hbm_trail, w_hbm);
     P.warp_smem = P.trail_smem ? smem_own_trail : smem_hbm_trail;
     P.warps = P.trail_smem ? w_own : w_hbm;
     P.smem = dense_bytes + P.warp_smem * P.warps;
@@ -930,6 +939,8 @@ static int launch_beam(lt_batch* b, cudaStream_t st, bool kbest) {
     b->last_beam_plan = P;
     if (!P->trail_smem)
         if (int rc = ensure(b->trail, nu * (size_t)beam_size * 8)) return rc;
+    // span byte 0xFF (> LT_WINDOW) marks the ranks this search leaves unfilled (violation.cuh)
+    if (b->hbm_trail) CU(cudaMemsetAsync(b->trail.p, 0xFF, nu * (size_t)beam_size * 8, st));
 
     unsigned int* ctl = static_cast<unsigned int*>(b->ctl.p);
     BeamArgs A{};
@@ -1756,6 +1767,11 @@ struct lt_trainer {
     DevBuf text, off;                       // the corpus
     DevBuf feat_coef, w, u, acc;            // [n_feat] coefficient of each desc feature; [n_coef] w, u, step counts
     DevBuf differs, mistakes;               // [n_sent] flags of each sentence's last step; running count of mistakes
+    int32_t mode = LT_UPDATE_FULL;          // lt_trainer_set_update
+    std::vector<int64_t> gold_off;          // host copy: W of each sentence
+    std::vector<uint8_t> full_last;         // [n_sent] the last step that covered the sentence was LT_UPDATE_FULL
+    DevBuf prefix_words, violation;         // [n_sent] of the last EARLY / MAX_VIOLATION step that covered the sentence
+    DevBuf gscore, chain;                   // violation_kernel scratch: [gold n_words] G_m, [step units] a rank-0 hypothesis
     cudaEvent_t done = nullptr;             // recorded after the last kernel of every step
 };
 
@@ -1822,6 +1838,18 @@ extern "C" int lt_trainer_create(lt_tables* t, int32_t func, const uint16_t* tex
     if (rc == LT_OK) rc = zeroed(tr->acc, (size_t)n_coef * 8);
     if (rc == LT_OK) rc = zeroed(tr->differs, (size_t)n_sent);
     if (rc == LT_OK) rc = zeroed(tr->mistakes, 8);
+    if (rc == LT_OK) rc = zeroed(tr->prefix_words, (size_t)n_sent * 4);
+    if (rc == LT_OK) {
+        const std::vector<double> nan((size_t)std::max(1, n_sent), std::numeric_limits<double>::quiet_NaN());
+        rc = upload_once(tr->violation, nan.data(), nan.size() * 8);
+    }
+    if (rc == LT_OK) rc = ensure(tr->gscore, (size_t)std::max<int64_t>(1, gold->n_words) * 8);
+    if (rc == LT_OK) {
+        tr->gold_off.resize((size_t)n_sent + 1);
+        tr->full_last.assign((size_t)n_sent, 1);
+        if (cudaMemcpy(tr->gold_off.data(), gold->off.p, tr->gold_off.size() * 8, cudaMemcpyDeviceToHost) != cudaSuccess)
+            rc = fail(LT_ERR_CUDA, "reading the gold offsets failed");
+    }
     if (rc == LT_OK) rc = upload_feat_dst(t);
     if (rc == LT_OK) rc = scatter_trainer_weights(tr, nullptr);
     if (rc == LT_OK && cudaEventCreate(&tr->done) != cudaSuccess) rc = fail(LT_ERR_CUDA, "cudaEventCreate failed");
@@ -1861,8 +1889,12 @@ extern "C" int lt_trainer_step(lt_trainer* tr, lt_batch* b, int32_t first, int32
     bind_batch(b, static_cast<const uint16_t*>(b->text.p), static_cast<const int32_t*>(b->sent_off.p), count, n_units, max_units, st);
     if (int rc = launch_lattice(b, st)) return rc;
     b->beam = beam_size;
-    if (int rc = launch_beam(b, st, false)) return rc;
-    if (int rc = resolve(b)) return rc;
+    // (the flag holds through the reruns resolve may launch; later searches of the batch keep the usual trail)
+    b->hbm_trail = tr->mode != LT_UPDATE_FULL;
+    int rc = launch_beam(b, st, false);
+    if (rc == LT_OK) rc = resolve(b);
+    b->hbm_trail = false;
+    if (rc) return rc;
 
     PerceptronArgs A{};
     if (int rc = search_and_gold(b, tr->gold, &A.sg)) return rc;
@@ -1873,9 +1905,25 @@ extern "C" int lt_trainer_step(lt_trainer* tr, lt_batch* b, int32_t first, int32
     A.counts = static_cast<unsigned long long*>(t->d_counts.p);
     A.differs = static_cast<uint8_t*>(tr->differs.p) + first;
     A.n_differ = static_cast<unsigned long long*>(tr->mistakes.p);
-    LT_LAUNCH(perceptron_kernel, warp_grid(t, count), 256, 0, st, t->dev, A);
+    if (tr->mode == LT_UPDATE_FULL) {
+        LT_LAUNCH(perceptron_kernel, warp_grid(t, count), 256, 0, st, t->dev, A);
+    } else {
+        if (int rc = ensure(tr->chain, (size_t)std::max<int64_t>(1, n_units) * sizeof(lt_edge))) return rc;
+        ViolationArgs V{};
+        V.pc = A;
+        V.mode = tr->mode;
+        V.beam = beam_size;
+        V.trail = static_cast<const uint64_t*>(b->trail.p);
+        V.edges = static_cast<const lt_edge*>(b->edges.p);
+        V.gscore = static_cast<double*>(tr->gscore.p);
+        V.chain = static_cast<lt_edge*>(tr->chain.p);
+        V.prefix_words = static_cast<int32_t*>(tr->prefix_words.p) + first;
+        V.violation = static_cast<double*>(tr->violation.p) + first;
+        LT_LAUNCH(violation_kernel, warp_grid(t, count), 256, 0, st, t->dev, V);
+    }
     CU(cudaGetLastError());
     b->launches += 1;
+    std::fill(tr->full_last.begin() + first, tr->full_last.begin() + first + count, tr->mode == LT_UPDATE_FULL ? 1 : 0);
 
     const int64_t step = ++tr->steps;
     const int64_t n_feat = (int64_t)t->feat_dst.size();
@@ -1921,5 +1969,32 @@ extern "C" int lt_trainer_fetch(lt_trainer* tr, double* coef, double* averaged, 
         *mistakes = (int64_t)m;
     }
     if (differs && tr->n_sent) CU(cudaMemcpy(differs, tr->differs.p, (size_t)tr->n_sent, cudaMemcpyDeviceToHost));
+    return LT_OK;
+}
+
+extern "C" int lt_trainer_set_update(lt_trainer* tr, int32_t mode) {
+    if (!tr) return fail(LT_ERR_INVALID, "null argument");
+    if (mode != LT_UPDATE_FULL && mode != LT_UPDATE_EARLY && mode != LT_UPDATE_MAX_VIOLATION)
+        return fail(LT_ERR_INVALID, "unknown update mode %d", mode);
+    tr->mode = mode;
+    return LT_OK;
+}
+
+extern "C" int lt_trainer_fetch_update(lt_trainer* tr, int32_t* prefix_words, double* violation) {
+    if (!tr) return fail(LT_ERR_INVALID, "null argument");
+    ON_DEVICE(tr->tables->device);
+    CU(cudaEventSynchronize(tr->done));
+    const size_t n = (size_t)tr->n_sent;
+    if (n == 0) return LT_OK;
+    std::vector<uint8_t> differs(n);
+    CU(cudaMemcpy(differs.data(), tr->differs.p, n, cudaMemcpyDeviceToHost));
+    if (prefix_words) CU(cudaMemcpy(prefix_words, tr->prefix_words.p, n * 4, cudaMemcpyDeviceToHost));
+    if (violation) CU(cudaMemcpy(violation, tr->violation.p, n * 8, cudaMemcpyDeviceToHost));
+    // a FULL step updates a differing sentence on its whole gold path
+    for (size_t i = 0; i < n; ++i) {
+        if (!tr->full_last[i]) continue;
+        if (prefix_words) prefix_words[i] = differs[i] ? (int32_t)(tr->gold_off[i + 1] - tr->gold_off[i]) : 0;
+        if (violation) violation[i] = std::numeric_limits<double>::quiet_NaN();
+    }
     return LT_OK;
 }

@@ -285,9 +285,10 @@ class Engine:
         """`paths[p]` = the `Word`s of path p without BOS / EOS -> a `PathSet` on these tables."""
         return PathSet(self, paths)
 
-    def trainer(self, sents, gold, func, n_coef, feat_coef, coef):
-        """A `DeviceTrainer` over `sents` (gold path i for sentence i) training scorer index `func`."""
-        return DeviceTrainer(self, sents, gold, func, n_coef, feat_coef, coef)
+    def trainer(self, sents, gold, func, n_coef, feat_coef, coef, update='full'):
+        """A `DeviceTrainer` over `sents` (gold path i for sentence i) training scorer index `func` with `update`
+        ('full', 'early' or 'max_violation')."""
+        return DeviceTrainer(self, sents, gold, func, n_coef, feat_coef, coef, update)
 
     def eval_paths(self, pathset, func=None):
         """lt_pathset_eval: (scores, feat_off, feat_idx); the features (of scorer index `func`, desc order)
@@ -475,9 +476,14 @@ class DeviceTrainer:
     `PathSet` (which must stay open while the trainer lives) go up once; `step(first, count, beam_size)` decodes
     sentences [first, first + count) on the engine's batch and updates the weights there; `fetch()` brings them
     back.  `feat_coef[i]`: the coefficient of desc feature i (`CompiledTables.desc_sources` order) of scorer
-    `func`, -1 for the others; `coef`: the initial weights, written into the tables at once."""
+    `func`, -1 for the others; `coef`: the initial weights, written into the tables at once.  `update` ('full',
+    'early' or 'max_violation', see `lt_trainer_set_update`) applies to the steps that follow and may be changed
+    between them with `set_update`."""
 
-    def __init__(self, engine, sents, gold, func, n_coef, feat_coef, coef):
+    UPDATE_MODES = {'full': _native.LT_UPDATE_FULL, 'early': _native.LT_UPDATE_EARLY,
+                    'max_violation': _native.LT_UPDATE_MAX_VIOLATION}
+
+    def __init__(self, engine, sents, gold, func, n_coef, feat_coef, coef, update='full'):
         self._lib = engine._lib
         self._engine = engine
         self.handle = None
@@ -488,6 +494,8 @@ class DeviceTrainer:
             raise ValueError('%d initial weights for %d coefficients' % (len(coef), n_coef))
         if len(feat_coef) != engine.tables.n_desc:
             raise ValueError('feat_coef has %d entries, the tables %d features' % (len(feat_coef), engine.tables.n_desc))
+        if update not in self.UPDATE_MODES:         # (before lt_trainer_create, which writes coef into the tables)
+            raise ValueError('update must be one of %s, got %r' % (', '.join(self.UPDATE_MODES), update))
         handle = ctypes.c_void_p()
         _native.check(self._lib.lt_trainer_create(
             engine.tables.handle, int(func), _native.ptr(text), _native.ptr(offsets), len(sents), gold.handle, int(n_coef),
@@ -495,6 +503,13 @@ class DeviceTrainer:
         self.handle = handle
         self.n_sent = len(sents)
         self.n_coef = int(n_coef)
+        self.set_update(update)
+
+    def set_update(self, update):
+        """The update of the following steps: 'full', 'early' or 'max_violation'."""
+        if update not in self.UPDATE_MODES:
+            raise ValueError('update must be one of %s, got %r' % (', '.join(self.UPDATE_MODES), update))
+        _native.check(self._lib.lt_trainer_set_update(self.handle, self.UPDATE_MODES[update]))
 
     def step(self, first, count, beam_size):
         _native.check(self._lib.lt_trainer_step(self.handle, self._engine.batch, int(first), int(count), int(beam_size)))
@@ -509,6 +524,16 @@ class DeviceTrainer:
         _native.check(self._lib.lt_trainer_fetch(self.handle, _native.ptr(coef), _native.ptr(averaged), ctypes.byref(steps),
                                                  ctypes.byref(mistakes), _native.ptr(differs)))
         return coef[:self.n_coef], averaged[:self.n_coef], int(steps.value), int(mistakes.value), differs[:self.n_sent].astype(bool)
+
+    def update_info(self):
+        """-> (prefix_words int32 [n_sent], violation float64 [n_sent]) per sentence, from the last step that covered
+        it: the gold words the update took (0: no update, W: the whole path) and B - G at that prefix, the score of
+        the best hypothesis minus the gold prefix's (NaN without an update, for a full step or a gold path that
+        does not tile the sentence)."""
+        prefix = np.zeros(max(1, self.n_sent), dtype=np.int32)
+        violation = np.zeros(max(1, self.n_sent), dtype=np.float64)
+        _native.check(self._lib.lt_trainer_fetch_update(self.handle, _native.ptr(prefix), _native.ptr(violation)))
+        return prefix[:self.n_sent], violation[:self.n_sent]
 
     def close(self):
         if self.handle is not None:

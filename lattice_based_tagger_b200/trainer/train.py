@@ -18,7 +18,10 @@ compares every prediction with its gold path and counts the features of both on 
 
 With `batch_size` the perceptron is online instead: the corpus is cut into consecutive mini-batches, and
 each one is decoded with the weights the previous ones left (`lt_trainer_step`), optionally averaged over
-all steps.  The weights and their running average then stay on the device for the whole run.
+all steps.  The weights and their running average then stay on the device for the whole run.  `update` picks
+the prefix a mini-batch step updates on: 'full' (the whole path), 'early' (up to the first gold word that fell out
+of the beam) or 'max_violation' (where the best hypothesis beats the gold prefix by the most); see
+`lt_trainer_set_update`.
 There is no CPU decoder: without the CUDA library `Tagger` raises.
 """
 
@@ -50,9 +53,10 @@ def _same_path(predicted, gold):
 
 def train(word_morph_pairs, dictionary, encoder, score_func, regularity_func,
           max_epochs=100, min_feature_count=1, predefined_features=None,
-          verbose=False, debug=False, beam_size=5, device=0, batch_size=None, averaged=False):
+          verbose=False, debug=False, beam_size=5, device=0, batch_size=None, averaged=False, update='full'):
     """Reference `train()` (`trainer/train.py:1-42`): -> {'idx_to_feature': [...], 'coefficient': [...]}
-    `batch_size` and `averaged` are passed to `fit_parameter`."""
+    `batch_size`, `averaged` and `update` are passed to `fit_parameter`."""
+    _check_update(update, batch_size)
     word_morph_pairs = list(word_morph_pairs)
     if verbose:
         print('Scanning features ...')
@@ -73,7 +77,7 @@ def train(word_morph_pairs, dictionary, encoder, score_func, regularity_func,
         print('Estimating parameter ...')
     try:
         coef = fit_parameter(word_morph_pairs, encoder, tagger, max_epochs, verbose=verbose, beam_size=beam_size,
-                             averaged=averaged, batch_size=batch_size)
+                             averaged=averaged, batch_size=batch_size, update=update)
     finally:
         tagger.close()
 
@@ -163,16 +167,30 @@ def evaluate(word_morph_pairs, tagger, beam_size=5):
         gold.close()
 
 
+UPDATE_MODES = ('full', 'early', 'max_violation')
+
+
+def _check_update(update, batch_size):
+    if update not in UPDATE_MODES:
+        raise ValueError('update must be one of %s, got %r' % (', '.join(UPDATE_MODES), update))
+    if update != 'full' and batch_size is None:
+        raise ValueError("update=%r needs batch_size: it reads the back-pointers of each mini-batch's search on the device "
+                         "(one decode of the whole corpus is batch_size=len(corpus))" % (update,))
+
+
 def fit_parameter(word_morph_pairs, encoder, tagger, max_epochs=100, verbose=False, beam_size=5, patience=5,
-                  averaged=False, batch_size=None):
+                  averaged=False, batch_size=None, update='full'):
     """Reference `fit_parameter()` (`train.py:44-59`).  Stops once an epoch makes no mistake, or when the
     number of mistakes has not improved for `patience` epochs (a corpus with an unreachable gold path — a word the
     dictionary cannot produce — never reaches zero); returns the best weights seen (`averaged=True`: the mean of
     the weights of all epochs, the averaged perceptron).
 
-    With an integer `batch_size`: mini-batch perceptron steps on the device, see `_fit_minibatch`."""
+    With an integer `batch_size`: mini-batch perceptron steps on the device, see `_fit_minibatch`; `update` ('full',
+    'early' or 'max_violation') is their update, and anything but 'full' needs `batch_size`."""
+    _check_update(update, batch_size)
     if batch_size is not None:
-        return _fit_minibatch(word_morph_pairs, encoder, tagger, max_epochs, verbose, beam_size, patience, averaged, batch_size)
+        return _fit_minibatch(word_morph_pairs, encoder, tagger, max_epochs, verbose, beam_size, patience, averaged, batch_size,
+                              update)
     coef = np.zeros(len(encoder.feature_dic), dtype=np.float64)
     best_loss, best_coef, stale = None, coef, 0
     total = np.zeros_like(coef)
@@ -198,7 +216,7 @@ def fit_parameter(word_morph_pairs, encoder, tagger, max_epochs=100, verbose=Fal
     return best_coef
 
 
-def _fit_minibatch(word_morph_pairs, encoder, tagger, max_epochs, verbose, beam_size, patience, averaged, batch_size):
+def _fit_minibatch(word_morph_pairs, encoder, tagger, max_epochs, verbose, beam_size, patience, averaged, batch_size, update):
     """The online perceptron: the sentences the device can compare, in corpus order, cut into consecutive mini-batches
     of `batch_size` (the last one may be shorter); every epoch walks them in that order, one `lt_trainer_step` each.
     An epoch's loss is its number of mistakes; it stops on loss 0 or after `patience` epochs without a new minimum.
@@ -224,7 +242,7 @@ def _fit_minibatch(word_morph_pairs, encoder, tagger, max_epochs, verbose, beam_
             func = tagger.score_funcs.funcs.index(scorer)
             desc_func, desc_fdic = engine.tables.desc_sources()
             feat_coef = np.where(desc_func == func, desc_fdic, -1)
-            trainer = engine.trainer(gold.device_sents, gold.pathset, func, len(coef), feat_coef, coef)
+            trainer = engine.trainer(gold.device_sents, gold.pathset, func, len(coef), feat_coef, coef, update=update)
             try:
                 best_loss, stale, seen = None, 0, 0
                 for epoch in range(1, max_epochs + 1):
