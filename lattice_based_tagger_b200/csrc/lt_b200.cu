@@ -716,8 +716,9 @@ static int lattice_plan(lt_batch* b, int lcap, int hcap, bool retry_pass, const 
     CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&P.per_sm, P.fn, P.warps * 32, P.smem));
     P.per_sm = std::max(1, P.per_sm);
     if (b->debug)
-        fprintf(stderr, "[lt] lattice kernel%s: units %d hcap %d max_str %d, %zu B/warp, %d warps/CTA, %zu B/CTA, %d CTAs/SM\n",
-                retry_pass ? " (retry pass)" : "", units, hcap, max_str, P.warp_smem, P.warps, P.smem, P.per_sm);
+        fprintf(stderr, "[lt] lattice kernel%s: units %d%s hcap %d%s max_str %d, %zu B/warp, %d warps/CTA, %zu B/CTA, %d CTAs/SM\n",
+                retry_pass ? " (retry pass)" : "", units, uclass ? " (sized instantiation)" : "", hcap, any_lookup ? " any lookup" : "",
+                max_str, P.warp_smem, P.warps, P.smem, P.per_sm);
     b->lattice_plans.push_back(P);
     *out = &b->lattice_plans.back();
     return LT_OK;
@@ -785,8 +786,9 @@ static int beam_plan(lt_batch* b, int lcap, int beam_size, bool kbest, const Bea
     CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&P.per_sm, P.fn, P.warps * 32, P.smem));
     P.per_sm = std::max(1, P.per_sm);
     if (b->debug)
-        fprintf(stderr, "[lt] beam kernel: beam %d units %d, %zu B/warp, %d warps/CTA, %zu B/CTA, %d CTAs/SM, trail in %s\n", beam_size,
-                units, P.warp_smem, P.warps, P.smem, P.per_sm, P.trail_smem ? "shared memory" : "HBM");
+        fprintf(stderr, "[lt] beam kernel: beam %d units %d%s, %zu B/warp, %d warps/CTA, %zu B/CTA, %d CTAs/SM, trail in %s%s%s\n", beam_size,
+                units, uclass ? " (sized instantiation)" : "", P.warp_smem, P.warps, P.smem, P.per_sm, P.trail_smem ? "shared memory" : "HBM",
+                prog1 ? ", reg+trigram program" : "", kbest ? ", k-best" : "");
     b->beam_plans.push_back(P);
     *out = &b->beam_plans.back();
     return LT_OK;

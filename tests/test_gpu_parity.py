@@ -242,7 +242,7 @@ def test_trail_in_hbm_and_generic_array_sizes(monkeypatch):
     tagger = pkg.Tagger(dictionary, score_funcs=funcs)
     _check_against_oracle(tagger, oracle, sents, (5, 10, 12))
     short = [s for s in sents if len(s) <= 40]
-    _check_against_oracle(tagger, oracle, short, (5, 10))              # 64-element arrays, trail in shared memory
+    _check_against_oracle(tagger, oracle, short, (5, 10))              # 64-element arrays (beam 10: trail never in shared memory)
     monkeypatch.setenv('LT_TRAIL_SMEM', '0')
     _check_against_oracle(tagger, oracle, short, (5, 10, 12))          # same kernels, trail in HBM
 
