@@ -20,6 +20,8 @@
  *                         word-level matches, and why a wrong sentence is wrong).
  *   lt_trainer_*       <- an online, averaged perceptron in mini-batches: the weights and their running
  *                         average stay on the device between steps.
+ *   lt_constraints_*   <- spans the caller already knows to be words (with or without their tag), kept by
+ *                         the beam search itself (lt_batch_set_constraints).
  *
  * Plain pointers and sizes only.  No function throws; each returns LT_OK or an LT_ERR_* code and
  * lt_last_error() returns the message of the calling thread's last failure.
@@ -34,7 +36,7 @@
 extern "C" {
 #endif
 
-#define LT_ABI_VERSION 7
+#define LT_ABI_VERSION 8
 
 /* return codes */
 #define LT_OK            0
@@ -54,6 +56,9 @@ extern "C" {
                                 rest of the batch is tagged                                     */
 #define LT_SENT_UNSUPPORTED_CHAR 4  /* set by host bindings for text that has no UTF-16 BMP form
                                 (the library itself never sees such a sentence)                 */
+#define LT_SENT_BAD_CONSTRAINT 5    /* a constrained search (lt_batch_set_constraints): a constraint of the
+                                sentence ends beyond its last syllable; no path, the rest of the
+                                batch is tagged                                                 */
 
 /* eojeol lookup that builds the lattice (dictionary/lookup.py), lt_batch_set_lookup():
  *   MORPHEME  MorphemeLookup  (lookup.py:99-132, :212-279) — what Tagger.tag always uses (tagger.py:60)
@@ -89,6 +94,9 @@ enum { LT_TAG_NOUN = 0, LT_TAG_PRONOUN, LT_TAG_NUMBER, LT_TAG_JOSA, LT_TAG_ADJEC
 
 #define LT_EDGE_EXPLICIT 0x10 /* imported lattice (lt_lattice_import): word / morph0 / morph1 are the
                                 strings 3*rule, 3*rule+1, 3*rule+2 given with the import           */
+#define LT_EDGE_FORCED 0x20  /* forced word of a tagged constraint whose span has no lattice edge of that
+                                tag: word = morph0 = chars[b:e], no morph1, tag0 = the constraint's
+                                tag, len = e - b (lt_batch_set_constraints)                       */
 
 /* One lattice edge = the reference's `Word` (dictionary/dictionary.py:169) in 16 bytes.
  * word  = chars[b:e]
@@ -445,6 +453,44 @@ void lt_trainer_destroy(lt_trainer* trainer);
 #define LT_UPDATE_MAX_VIOLATION 2
 int  lt_trainer_set_update(lt_trainer* trainer, int32_t mode);
 int  lt_trainer_fetch_update(lt_trainer* trainer, int32_t* prefix_words, double* violation);
+
+/* Constrained search: spans the caller already knows to be words.  A constraint of a sentence is (b, e, tag): b, e
+ * syllable offsets in the space-stripped sentence (the coordinates of lt_edge.b / .e), 1 <= e - b <= LT_WINDOW, and
+ * tag a tag id below n_tags other than BOS, EOS and Unk, or LT_NO_TAG for "any word".  A sentence's constraints are
+ * sorted by b and do not overlap (c[i].e <= c[i+1].b); they may cross eojeol boundaries.  The search is beam_search
+ * with three changes to the candidates of end e and begin b (DESIGN.md, "Constrained search"):
+ *   1. (b, e) is blocked when a constraint c overlaps it without being equal to it (b < c.e, c.b < e, (b, e) != (c.b,
+ *      c.e)): no lattice edge and no unknown word.  Positions strictly inside a constrained span keep no hypothesis.
+ *   2. (b, e) == (c.b, c.e): the span's lattice edges with tag0 == c.tag (all of them for LT_NO_TAG), in lattice
+ *      order.  If there is none: with LT_NO_TAG the usual unknown word; with a tag, one LT_EDGE_FORCED word, is_l set
+ *      when b is the first syllable of an eojeol.
+ *   3. An unknown word may follow an unknown word only from the first begin the constraints leave open: the smallest
+ *      b in [max(0, e - LT_WINDOW), e) for which (b, e) is not blocked (without constraints: beam.py:44-45).
+ * Every sentence with status LT_SENT_OK then has a path, and it has a word on each constrained span with its tag.
+ *
+ * lt_constraints_create   constraint set of n_sent sentences: sentence s has cons[cons_off[s] .. cons_off[s+1]),
+ *                         cons_off has n_sent + 1 entries starting at 0.  LT_ERR_INVALID, naming the sentence and the
+ *                         index, for offsets that are not monotone, constraints that are unsorted or overlap, a span
+ *                         outside 1..LT_WINDOW syllables or a tag the search cannot give a word.  A constraint ending
+ *                         beyond its sentence is found by the search: LT_SENT_BAD_CONSTRAINT.
+ * lt_batch_set_constraints binds the set (NULL: none) for the searches that follow on the batch: lt_beam,
+ *                         lt_beam_kbest, lt_tag_batch_host, lt_tag_batch_host_kbest, lt_tag_batch_device, imported
+ *                         lattices included.  The set must outlive its binding and the fetch of those searches'
+ *                         results.  A search of a batch whose n_sent differs from the set's returns LT_ERR_INVALID
+ *                         before any launch.  The statuses lt_paths_fetch / lt_kbest_fetch return are the search's
+ *                         (with LT_SENT_BAD_CONSTRAINT); lt_lattice_status keeps the lattice's.
+ * lt_evaluate and lt_perceptron_delta after a constrained search, and lt_trainer_step on a batch with constraints
+ * bound, return LT_ERR_INVALID: their results are defined on the unconstrained search space. */
+typedef struct lt_constraint {
+    uint16_t b, e;
+    uint8_t  tag;        /* tag id, or LT_NO_TAG */
+    uint8_t  reserved[3];
+} lt_constraint;
+typedef struct lt_constraints lt_constraints;
+int  lt_constraints_create(lt_tables* tables, int32_t n_sent, const lt_constraint* cons, const int64_t* cons_off,
+                           lt_constraints** out);
+void lt_constraints_destroy(lt_constraints* cons);
+int  lt_batch_set_constraints(lt_batch* batch, const lt_constraints* cons);
 
 #ifdef __cplusplus
 }

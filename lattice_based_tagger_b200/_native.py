@@ -13,12 +13,12 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, 'liblt_b200.so')
 
-LT_ABI_VERSION = 7
+LT_ABI_VERSION = 8
 LT_OK = 0
-LT_SENT_OK, LT_SENT_NO_EDGES, LT_SENT_BAD_SPACE, LT_SENT_TOO_LONG, LT_SENT_UNSUPPORTED_CHAR = 0, 1, 2, 3, 4
+LT_SENT_OK, LT_SENT_NO_EDGES, LT_SENT_BAD_SPACE, LT_SENT_TOO_LONG, LT_SENT_UNSUPPORTED_CHAR, LT_SENT_BAD_CONSTRAINT = 0, 1, 2, 3, 4, 5
 LT_NO_TAG = 0xFF
 LT_NO_RULE = 0xFFFFFFFF
-LT_EDGE_IS_L, LT_EDGE_UNK, LT_EDGE_LEMMA, LT_EDGE_SKIP2, LT_EDGE_EXPLICIT = 1, 2, 4, 8, 16
+LT_EDGE_IS_L, LT_EDGE_UNK, LT_EDGE_LEMMA, LT_EDGE_SKIP2, LT_EDGE_EXPLICIT, LT_EDGE_FORCED = 1, 2, 4, 8, 16, 32
 (LT_LOOKUP_MORPHEME, LT_LOOKUP_LR, LT_LOOKUP_LR_ALL, LT_LOOKUP_WORD, LT_LOOKUP_WORD_ALL,
  LT_LOOKUP_EXACT) = range(6)
 LT_FUNC_REG, LT_FUNC_MPREF, LT_FUNC_WPREF, LT_FUNC_TRIGRAM = 1, 2, 3, 4
@@ -37,6 +37,10 @@ LT_MAX_FUNCS = 8
 EDGE_DTYPE = np.dtype([('b', '<u2'), ('e', '<u2'), ('len', '<u2'), ('tag0', 'u1'), ('tag1', 'u1'),
                        ('rule', '<u4'), ('split', '<u2'), ('flags', 'u1'), ('reserved', 'u1')])
 assert EDGE_DTYPE.itemsize == 16
+
+#: numpy view of `lt_constraint` (8 bytes)
+CONSTRAINT_DTYPE = np.dtype([('b', '<u2'), ('e', '<u2'), ('tag', 'u1'), ('reserved', 'u1', (3,))])
+assert CONSTRAINT_DTYPE.itemsize == 8
 
 _p = ctypes.c_void_p
 
@@ -131,6 +135,9 @@ SYMBOLS = {
     'lt_trainer_destroy': (None, [_p]),
     'lt_trainer_set_update': (ctypes.c_int, [_p, ctypes.c_int32]),
     'lt_trainer_fetch_update': (ctypes.c_int, [_p, _p, _p]),
+    'lt_constraints_create': (ctypes.c_int, [_p, ctypes.c_int32, _p, _p, ctypes.POINTER(_p)]),
+    'lt_constraints_destroy': (None, [_p]),
+    'lt_batch_set_constraints': (ctypes.c_int, [_p, _p]),
 }
 
 _lib = None

@@ -39,6 +39,7 @@
 // sentence, once without the code (and the out-of-line calls) that only buckets beyond the edge cache need —
 // see the note at the top of that file.
 #pragma once
+#include "constraints.cuh"
 #include "lattice.cuh"
 #include "tables.cuh"
 
@@ -88,6 +89,7 @@ struct BeamArgs {
     int32_t* kb_len;            // [n_sent * beam] words of survivor r (0 beyond the survivors)
     double* kb_scores;          // [n_sent * beam]
     int32_t* kb_count;          // [n_sent] survivors (1 for an empty sentence: [BOS, EOS])
+    const uint32_t* cdesc;      // constrained search: [n_units] position descriptors (constraints.cuh)
 };
 
 // Prepared edges (shared memory, struct of arrays).  Slots [0, kEdgeRing): dictionary edges at
@@ -410,8 +412,11 @@ __device__ __forceinline__ void prep_edge(const DevTables& T, const SentView& v,
 // KB: 1 = every survivor of the last position is written out as well (lt_beam_kbest); 0 compiles that out of
 // the instantiations the throughput path runs.
 // TS: back-pointers in shared memory (1) or HBM (0) known at compile time; -1 = A.trail_smem.
-template <int MODE, int KT, int UC, int PROG, int KB = 0, int TS = -1>
+// CONS: 1 = constrained search (lt_batch_set_constraints): the position loop reads A.cdesc and A.status is the search's
+// status; only the generic instantiations (KT = UC = PROG = 0) have such a copy.
+template <int MODE, int KT, int UC, int PROG, int KB = 0, int TS = -1, int CONS = 0>
 __global__ void __launch_bounds__(beam_max_threads(KT, UC, PROG, KB), beam_min_blocks(KT, UC, PROG, KB)) beam_kernel(const __grid_constant__ DevTables T, const __grid_constant__ BeamArgs A) {
+    static_assert(CONS == 0 || (KT == 0 && UC == 0 && PROG == 0), "only the generic instantiations have a constrained copy");
     constexpr int KR = (MODE == 0) ? 2 : 1;      // kept entries per lane
     LT_DYN_SMEM(smem_raw);
     const int lane = threadIdx.x & 31;
@@ -594,6 +599,14 @@ __global__ void __launch_bounds__(beam_max_threads(KT, UC, PROG, KB), beam_min_b
                         ed.b = (uint16_t)(e - span); ed.e = (uint16_t)e; ed.len = (uint16_t)span;
                         ed.tag0 = LT_TAG_UNK; ed.tag1 = LT_NO_TAG; ed.rule = LT_NO_RULE; ed.split = 0;
                         ed.flags = LT_EDGE_UNK; ed.reserved = 0;
+                        if constexpr (CONS != 0) {
+                            // at a forced constraint end the only unknown-word slot is the forced word's
+                            const uint32_t d = __ldg(A.cdesc + s0 + e - 1);
+                            if (d & kConsForced) {
+                                ed.tag0 = (uint8_t)((d >> kConsTagShift) & 0xFFu);
+                                ed.flags = (uint8_t)(LT_EDGE_FORCED | ((d & kConsIsL) ? LT_EDGE_IS_L : 0u));
+                            }
+                        }
                     } else {
                         ed = A.edges[eref];
                     }

@@ -17,6 +17,7 @@
 
 #include "../../include/lt_b200.h"
 #include "beam.cuh"
+#include "constraints.cuh"
 #include "evaluate.cuh"
 #include "hash.cuh"
 #include "lattice.cuh"
@@ -472,7 +473,7 @@ struct LatticePlan {
 };
 struct BeamPlan {
     int units = 0, beam = 0;                  // key
-    bool kbest = false, hbm_trail = false;
+    bool kbest = false, hbm_trail = false, constrained = false;
     void (*fn)(const DevTables, const BeamArgs) = nullptr;
     int warps = 0, per_sm = 1;
     size_t smem = 0, warp_smem = 0;
@@ -481,6 +482,13 @@ struct BeamPlan {
 
 // events of a timed batch (lt_batch_timings): host text in, lattice kernels, beam kernel, path packing, results out
 enum { kEvHostIn, kEvLatticeStart, kEvLatticeEnd, kEvBeamStart, kEvBeamEnd, kEvPackEnd, kEvHostOut, kStageEvents };
+
+struct lt_constraints {
+    lt_tables* tables = nullptr;
+    int device = 0;
+    int32_t n_sent = 0;
+    DevBuf cons, off;               // [n_cons] constraints, [n_sent + 1] offsets
+};
 
 struct lt_batch {
     lt_tables* tables = nullptr;
@@ -497,6 +505,9 @@ struct lt_batch {
     DevBuf pth_scores, pth_feat, pth_nfeat;      // lt_pathset_eval results
     DevBuf pc_delta, pc_differs, pc_count;       // lt_perceptron_delta results
     DevBuf ev_image, ev_class, ev_counts, ev_scores, ev_reason;   // lt_evaluate: gold images (scratch), results
+    DevBuf cons_status, cons_desc;               // constrained search: its per-sentence status, position descriptors
+    const lt_constraints* cons = nullptr;        // bound by lt_batch_set_constraints for the searches to come
+    const lt_constraints* search_cons = nullptr; // the set the last search ran with (its reruns run with it too)
     bool imported = false;
     const uint16_t* d_text = nullptr;
     const int32_t* d_sent_off = nullptr;
@@ -724,16 +735,19 @@ static int lattice_plan(lt_batch* b, int lcap, int hcap, bool retry_pass, const 
     return LT_OK;
 }
 
-static int beam_plan(lt_batch* b, int lcap, int beam_size, bool kbest, const BeamPlan** out) {
+static int beam_plan(lt_batch* b, int lcap, int beam_size, bool kbest, bool constrained, const BeamPlan** out) {
     lt_tables* t = b->tables;
     // sentence arrays: common sizes are template parameters of the kernel (for beams 5 and 10); the all-survivors
-    // variant (lt_beam_kbest) exists in the generic instantiations only
-    const int uclass = (!kbest && (beam_size == 5 || beam_size == 10)) ? beam_units_class(lcap) : 0;
+    // variant (lt_beam_kbest) and the constrained search exist in the generic instantiations only
+    const int uclass = (!kbest && !constrained && (beam_size == 5 || beam_size == 10)) ? beam_units_class(lcap) : 0;
     const int units = uclass ? uclass : lcap + 8;
     for (const BeamPlan& p : b->beam_plans)
-        if (p.units == units && p.beam == beam_size && p.kbest == kbest && p.hbm_trail == b->hbm_trail) { *out = &p; return LT_OK; }
+        if (p.units == units && p.beam == beam_size && p.kbest == kbest && p.hbm_trail == b->hbm_trail && p.constrained == constrained) {
+            *out = &p;
+            return LT_OK;
+        }
     const size_t dense_bytes = ((size_t)t->dev.n_tri * dense_block_bytes(t->dev.n_tags) + 15) & ~(size_t)15;
-    const bool reg_tri = t->dev.n_funcs == 2 && t->dev.funcs[0].kind == LT_FUNC_REG && t->dev.funcs[1].kind == LT_FUNC_TRIGRAM;
+    const bool reg_tri = !constrained && t->dev.n_funcs == 2 && t->dev.funcs[0].kind == LT_FUNC_REG && t->dev.funcs[1].kind == LT_FUNC_TRIGRAM;
     const bool prog1 = reg_tri && !kbest;                      // the instantiation specialised for that score program
     const int kvd = beam_kval_doubles(t->dev.n_funcs, prog1);
     // CTA shape: the warps per CTA (1..8) that keep the most warps resident on an SM under the kernel's
@@ -764,13 +778,18 @@ static int beam_plan(lt_batch* b, int lcap, int beam_size, bool kbest, const Bea
     P.beam = beam_size;
     P.kbest = kbest;
     P.hbm_trail = b->hbm_trail;
+    P.constrained = constrained;
     P.trail_smem = !b->hbm_trail && b->trail_smem_ok && w_own > 0 && resident_warps(smem_own_trail, w_own) >= resident_warps(smem_hbm_trail, w_hbm);
     P.warp_smem = P.trail_smem ? smem_own_trail : smem_hbm_trail;
     P.warps = P.trail_smem ? w_own : w_hbm;
     P.smem = dense_bytes + P.warp_smem * P.warps;
     // common beam sizes, sentence-array sizes and the (RegularizationScore, SimpleTrigramFeatureScore)
     // score program get their own instantiation (compile-time array offsets, unrolled scorer loop)
-    if (kbest) P.fn = beam_size <= kRankMaxBeam ? beam_kernel<2, 0, 0, 0, 1> : (beam_size <= 32 ? beam_kernel<1, 0, 0, 0, 1> : beam_kernel<0, 0, 0, 0, 1>);
+    if (constrained && kbest)
+        P.fn = beam_size <= kRankMaxBeam ? beam_kernel<2, 0, 0, 0, 1, -1, 1> : (beam_size <= 32 ? beam_kernel<1, 0, 0, 0, 1, -1, 1> : beam_kernel<0, 0, 0, 0, 1, -1, 1>);
+    else if (constrained)
+        P.fn = beam_size <= kRankMaxBeam ? beam_kernel<2, 0, 0, 0, 0, -1, 1> : (beam_size <= 32 ? beam_kernel<1, 0, 0, 0, 0, -1, 1> : beam_kernel<0, 0, 0, 0, 0, -1, 1>);
+    else if (kbest) P.fn = beam_size <= kRankMaxBeam ? beam_kernel<2, 0, 0, 0, 1> : (beam_size <= 32 ? beam_kernel<1, 0, 0, 0, 1> : beam_kernel<0, 0, 0, 0, 1>);
     // (the specialised kernels also know at compile time where the back-pointers live)
     else if (beam_size == 5 && uclass == 64) P.fn = reg_tri ? (P.trail_smem ? beam_kernel<2, 5, 64, 1, 0, 1> : beam_kernel<2, 5, 64, 1, 0, 0>) : beam_kernel<2, 5, 64, 0>;
     else if (beam_size == 5 && uclass == 128) P.fn = reg_tri ? (P.trail_smem ? beam_kernel<2, 5, 128, 1, 0, 1> : beam_kernel<2, 5, 128, 1, 0, 0>) : beam_kernel<2, 5, 128, 0>;
@@ -786,9 +805,9 @@ static int beam_plan(lt_batch* b, int lcap, int beam_size, bool kbest, const Bea
     CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&P.per_sm, P.fn, P.warps * 32, P.smem));
     P.per_sm = std::max(1, P.per_sm);
     if (b->debug)
-        fprintf(stderr, "[lt] beam kernel: beam %d units %d%s, %zu B/warp, %d warps/CTA, %zu B/CTA, %d CTAs/SM, trail in %s%s%s\n", beam_size,
+        fprintf(stderr, "[lt] beam kernel: beam %d units %d%s, %zu B/warp, %d warps/CTA, %zu B/CTA, %d CTAs/SM, trail in %s%s%s%s\n", beam_size,
                 units, uclass ? " (sized instantiation)" : "", P.warp_smem, P.warps, P.smem, P.per_sm, P.trail_smem ? "shared memory" : "HBM",
-                prog1 ? ", reg+trigram program" : "", kbest ? ", k-best" : "");
+                prog1 ? ", reg+trigram program" : "", kbest ? ", k-best" : "", constrained ? ", constrained" : "");
     b->beam_plans.push_back(P);
     *out = &b->beam_plans.back();
     return LT_OK;
@@ -811,6 +830,9 @@ static void bind_batch(lt_batch* b, const uint16_t* d_text, const int32_t* d_sen
     b->have_lattice = b->have_paths = b->have_kbest = false;
     b->imported = b->resolved = false;
 }
+
+// per-sentence statuses of the last search: the lattice's, or a constrained search's own (LT_SENT_BAD_CONSTRAINT)
+static const void* search_status(const lt_batch* b) { return b->search_cons ? b->cons_status.p : b->status.p; }
 
 // the order in which persistent warps take sentences (longest first), or nullptr: in input order
 static uint32_t* work_order(const lt_batch* b) {
@@ -936,8 +958,9 @@ static int launch_beam(lt_batch* b, cudaStream_t st, bool kbest) {
         if (int rc = ensure(b->kb_count, (size_t)std::max(1, n_sent) * 4)) return rc;
     }
 
+    const lt_constraints* cons = b->search_cons;
     const BeamPlan* P = nullptr;
-    if (int rc = beam_plan(b, b->lcap, beam_size, kbest, &P)) return rc;
+    if (int rc = beam_plan(b, b->lcap, beam_size, kbest, cons != nullptr, &P)) return rc;
     b->last_beam_plan = P;
     if (!P->trail_smem)
         if (int rc = ensure(b->trail, nu * (size_t)beam_size * 8)) return rc;
@@ -970,6 +993,32 @@ static int launch_beam(lt_batch* b, cudaStream_t st, bool kbest) {
     A.kb_len = static_cast<int32_t*>(b->kb_len.p);
     A.kb_scores = static_cast<double*>(b->kb_scores.p);
     A.kb_count = static_cast<int32_t*>(b->kb_count.p);
+    if (cons) {
+        // the search's statuses and the position descriptors of its constraints (constraints.cuh), from the lattice
+        // as it stands: a rerun after a grown lattice prepares them again
+        if (int rc = ensure(b->cons_status, (size_t)std::max(1, n_sent) * 4)) return rc;
+        if (int rc = ensure(b->cons_desc, nu * 4)) return rc;
+        ConstraintArgs C{};
+        C.text = b->d_text;
+        C.sent_off = b->d_sent_off;
+        C.n_sent = n_sent;
+        C.status = static_cast<const int32_t*>(b->status.p);
+        C.flags = ctl + kCtlFlags;
+        C.pos = static_cast<const uint2*>(b->pos.p);
+        C.edges = static_cast<const lt_edge*>(b->edges.p);
+        C.cons = static_cast<const lt_constraint*>(cons->cons.p);
+        C.cons_off = static_cast<const int64_t*>(cons->off.p);
+        C.search_status = static_cast<int32_t*>(b->cons_status.p);
+        C.desc = static_cast<uint32_t*>(b->cons_desc.p);
+        if (n_sent > 0) {
+            const unsigned cgrid = (unsigned)std::min<int64_t>(((int64_t)n_sent + kConsWarps - 1) / kConsWarps, (int64_t)t->sm_count * 8);
+            LT_LAUNCH(constraint_prep_kernel, cgrid, kConsWarps * 32, 0, st, C);
+            CU(cudaGetLastError());
+            b->launches += 1;
+        }
+        A.status = C.search_status;
+        A.cdesc = C.desc;
+    }
 
     const int64_t want_blocks = ((int64_t)n_sent + P->warps - 1) / P->warps;
     const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(want_blocks, (int64_t)t->sm_count * P->per_sm));
@@ -1102,13 +1151,22 @@ extern "C" int lt_lattice(lt_batch* b, const uint16_t* d_text, const int32_t* d_
     return launch_lattice(b, st);
 }
 
+// a search of n_sent sentences against the bound constraint set (checked before anything is launched)
+static int check_constraints(const lt_batch* b, int32_t n_sent) {
+    if (b->cons && b->cons->n_sent != n_sent)
+        return fail(LT_ERR_INVALID, "the bound constraint set has %d sentences, the search %d", b->cons->n_sent, n_sent);
+    return LT_OK;
+}
+
 static int beam_entry(lt_batch* b, int32_t beam_size, void* stream, bool kbest) {
     if (!b || !b->have_lattice) return fail(LT_ERR_INVALID, "lt_beam needs a lattice: call lt_lattice first");
     if (beam_size < 1 || beam_size > LT_MAX_BEAM) return fail(LT_ERR_INVALID, "beam_size must be in 1..%d", LT_MAX_BEAM);
+    if (int rc = check_constraints(b, b->n_sent)) return rc;
     ON_DEVICE(b->tables->device);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     b->last_stream = st;
     b->beam = beam_size;
+    b->search_cons = b->cons;
     return launch_beam(b, st, kbest);
 }
 
@@ -1117,6 +1175,8 @@ extern "C" int lt_beam_kbest(lt_batch* b, int32_t beam_size, void* stream) { ret
 
 extern "C" int lt_tag_batch_device(lt_batch* b, const uint16_t* d_text, const int32_t* d_sent_off, int32_t n_sent,
                                    int64_t n_units, int32_t max_sent_units, int32_t beam_size, void* stream) {
+    if (b)
+        if (int rc = check_constraints(b, n_sent)) return rc;
     if (int rc = lt_lattice(b, d_text, d_sent_off, n_sent, n_units, max_sent_units, stream)) return rc;
     return lt_beam(b, beam_size, stream);
 }
@@ -1194,7 +1254,7 @@ static int fetch_paths(lt_batch* b, int32_t* path_off, lt_edge* path_edges, int6
         CU(cudaMemcpyAsync(ctl, b->ctl.p, kCtlWords * sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
         CU(cudaMemcpyAsync(path_off, b->path_off.p, (size_t)(n + 1) * 4, cudaMemcpyDeviceToHost, st));
         CU(cudaMemcpyAsync(scores, b->scores.p, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(status, b->status.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(status, search_status(b), (size_t)n * 4, cudaMemcpyDeviceToHost, st));
         if (guess > 0) CU(cudaMemcpyAsync(path_edges, b->path_out.p, (size_t)guess * sizeof(lt_edge), cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
         copied = guess;
@@ -1250,7 +1310,7 @@ extern "C" int lt_kbest_fetch(lt_batch* b, int32_t* n_best, int32_t* path_off, l
     CU(cudaMemcpyAsync(path_off, b->kb_off.p, (nk + 1) * 4, cudaMemcpyDeviceToHost, st));
     CU(cudaMemcpyAsync(n_best, b->kb_count.p, n * 4, cudaMemcpyDeviceToHost, st));
     CU(cudaMemcpyAsync(scores, b->kb_scores.p, nk * 8, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(status, b->status.p, n * 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(status, search_status(b), n * 4, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     const int64_t total = path_off[nk];
     if (total > path_cap) return fail(LT_ERR_CAPACITY, "path buffer holds %lld records, need %lld", (long long)path_cap, (long long)total);
@@ -1291,6 +1351,7 @@ extern "C" int lt_tag_batch_host(lt_batch* b, const uint16_t* text, const int32_
                                  int32_t beam_size, int32_t* path_off, lt_edge* path_edges, int64_t path_cap,
                                  double* scores, int32_t* status) {
     if (!b) return fail(LT_ERR_INVALID, "bad argument");
+    if (int rc = check_constraints(b, n_sent)) return rc;
     ON_DEVICE(b->tables->device);
     cudaStream_t st = b->own_stream;
     const bool timed = b->timed;
@@ -1309,6 +1370,7 @@ extern "C" int lt_tag_batch_host(lt_batch* b, const uint16_t* text, const int32_
 extern "C" int lt_tag_batch_host_kbest(lt_batch* b, const uint16_t* text, const int32_t* sent_off, int32_t n_sent,
                                        int32_t beam_size) {
     if (!b) return fail(LT_ERR_INVALID, "bad argument");
+    if (int rc = check_constraints(b, n_sent)) return rc;
     ON_DEVICE(b->tables->device);
     if (int rc = host_lattice(b, text, sent_off, n_sent)) return rc;
     return lt_beam_kbest(b, beam_size, b->own_stream);
@@ -1495,6 +1557,61 @@ extern "C" int lt_batch_timings(lt_batch* b, lt_timings* out) {
 }
 
 // ------------------------------------------------------------------------------------------------
+// constraint sets (constraints.cuh): spans the search must keep as words
+// ------------------------------------------------------------------------------------------------
+extern "C" void lt_constraints_destroy(lt_constraints* c) {
+    if (!c) return;
+    DeviceGuard guard(c->device);      // (the tables may be gone already)
+    delete c;
+}
+
+extern "C" int lt_constraints_create(lt_tables* t, int32_t n_sent, const lt_constraint* cons, const int64_t* cons_off,
+                                     lt_constraints** out) {
+    if (!t || !out || !cons_off || n_sent < 0) return fail(LT_ERR_INVALID, "bad argument");
+    *out = nullptr;
+    if (cons_off[0] != 0) return fail(LT_ERR_INVALID, "cons_off[0] must be 0");
+    for (int32_t s = 0; s < n_sent; ++s)
+        if (cons_off[s + 1] < cons_off[s]) return fail(LT_ERR_INVALID, "cons_off is not monotone at sentence %d", s);
+    const int64_t n_cons = cons_off[n_sent];
+    if (n_cons > 0 && !cons) return fail(LT_ERR_INVALID, "null constraint pointer");
+    const int n_tags = t->dev.n_tags;
+    for (int32_t s = 0; s < n_sent; ++s)
+        for (int64_t i = cons_off[s]; i < cons_off[s + 1]; ++i) {
+            const lt_constraint& c = cons[i];
+            const int64_t k = i - cons_off[s];
+            if (c.e <= c.b || c.e - c.b > LT_WINDOW)
+                return fail(LT_ERR_INVALID, "sentence %d, constraint %lld: span [%d, %d) is not 1..%d syllables", s, (long long)k, c.b, c.e,
+                            LT_WINDOW);
+            if (c.tag != LT_NO_TAG && (c.tag >= n_tags || c.tag == LT_TAG_BOS || c.tag == LT_TAG_EOS || c.tag == LT_TAG_UNK))
+                return fail(LT_ERR_INVALID, "sentence %d, constraint %lld: tag %d is not a word tag of the tables (nor LT_NO_TAG)", s,
+                            (long long)k, c.tag);
+            if (k > 0 && cons[i - 1].e > c.b)
+                return fail(LT_ERR_INVALID, "sentence %d, constraint %lld: begins at %d, before the previous one ends (%d); constraints are "
+                                            "sorted by b and do not overlap", s, (long long)k, c.b, cons[i - 1].e);
+        }
+    ON_DEVICE(t->device);
+    lt_constraints* c = new lt_constraints();
+    c->tables = t;
+    c->device = t->device;
+    c->n_sent = n_sent;
+    int rc = upload_once(c->cons, cons, (size_t)n_cons * sizeof(lt_constraint));
+    if (rc == LT_OK) rc = upload_once(c->off, cons_off, (size_t)(n_sent + 1) * 8);
+    if (rc != LT_OK) {
+        delete c;
+        return rc;
+    }
+    *out = c;
+    return LT_OK;
+}
+
+extern "C" int lt_batch_set_constraints(lt_batch* b, const lt_constraints* c) {
+    if (!b) return fail(LT_ERR_INVALID, "null argument");
+    if (c && c->tables != b->tables) return fail(LT_ERR_INVALID, "the constraint set belongs to other tables");
+    b->cons = c;
+    return LT_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
 // path sets: scoring / featurizing given paths, the perceptron step (paths.cuh)
 // ------------------------------------------------------------------------------------------------
 struct lt_pathset {
@@ -1635,6 +1752,8 @@ extern "C" int lt_pathset_eval(lt_batch* b, const lt_pathset* paths, int32_t fun
 // lt_perceptron_delta / lt_evaluate: the best paths of the last search next to one gold path per sentence
 static int check_gold(const lt_batch* b, const lt_pathset* gold) {
     if (!b->have_paths) return fail(LT_ERR_INVALID, "no paths: run a search (lt_tag_batch_host, lt_beam, ...) first");
+    if (b->search_cons)
+        return fail(LT_ERR_INVALID, "the last search was constrained: its paths are not the ones this compares against gold paths");
     if (gold->tables != b->tables) return fail(LT_ERR_INVALID, "the gold path set belongs to other tables");
     if (gold->n_paths != b->n_sent) return fail(LT_ERR_INVALID, "%d gold paths for %d sentences", gold->n_paths, b->n_sent);
     return LT_OK;
@@ -1875,6 +1994,7 @@ extern "C" int lt_trainer_step(lt_trainer* tr, lt_batch* b, int32_t first, int32
         return fail(LT_ERR_INVALID, "sentences [%d, %lld) are not a non-empty range of the %d corpus sentences", first,
                     (long long)first + count, tr->n_sent);
     if (beam_size < 1 || beam_size > LT_MAX_BEAM) return fail(LT_ERR_INVALID, "beam_size must be in 1..%d", LT_MAX_BEAM);
+    if (b->cons) return fail(LT_ERR_INVALID, "the batch has constraints bound: a trainer step searches without them");
     ON_DEVICE(t->device);
     cudaStream_t st = b->own_stream;
     const int32_t* off = tr->sent_off.data() + first;
@@ -1891,6 +2011,7 @@ extern "C" int lt_trainer_step(lt_trainer* tr, lt_batch* b, int32_t first, int32
     bind_batch(b, static_cast<const uint16_t*>(b->text.p), static_cast<const int32_t*>(b->sent_off.p), count, n_units, max_units, st);
     if (int rc = launch_lattice(b, st)) return rc;
     b->beam = beam_size;
+    b->search_cons = nullptr;
     // (the flag holds through the reruns resolve may launch; later searches of the batch keep the usual trail)
     b->hbm_trail = tr->mode != LT_UPDATE_FULL;
     int rc = launch_beam(b, st, false);

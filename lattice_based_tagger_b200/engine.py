@@ -7,6 +7,7 @@ eojeol-lookup classes (`dictionary/lookup.py`), `MorphemeDictionary.lookup / lem
 `analyze_morphology` and `beam_search` are thin layers over it.
 """
 
+import contextlib
 import ctypes
 from collections.abc import Sequence as _SequenceABC
 
@@ -14,13 +15,14 @@ import numpy as np
 
 from . import _native
 from .compile import CompiledTables, _encode_units
-from .tagset import BOS, EOS
+from .tagset import BOS, EOS, Unk
 
 _STATUS_MESSAGES = {
     _native.LT_SENT_BAD_SPACE: 'sentence %d contains whitespace other than U+0020',
     _native.LT_SENT_TOO_LONG: 'sentence %d is longer than the %d code units the device kernels hold',
     _native.LT_SENT_UNSUPPORTED_CHAR: 'sentence %d contains characters outside the Basic Multilingual Plane, '
                                       'which the device text format (UTF-16 code units) does not support',
+    _native.LT_SENT_BAD_CONSTRAINT: 'sentence %d has a constraint that ends beyond its last syllable',
 }
 
 
@@ -138,9 +140,77 @@ class Engine:
             _native.check(self._lib.lt_batch_set_lookup(self.batch, int(mode)))
             self._mode = mode
 
+    # -- constraints -------------------------------------------------------------------------------
+    def pack_constraints(self, sents, constraints):
+        """Per sentence a list of `(b, e)` / `(b, e, tag_name)` spans the search must keep as words (`None` or `[]`:
+        none) -> (`lt_constraint` records, int64 offsets).  Every malformed list raises `ValueError`: a count that
+        is not one list per sentence, items that are not such tuples, b >= e, spans longer than the window or
+        beyond the sentence's syllables, unsorted or overlapping spans, BOS / EOS / Unknown or a tag the tables do
+        not know."""
+        if len(constraints) != len(sents):
+            raise ValueError('%d constraint lists for %d sentences' % (len(constraints), len(sents)))
+        tag_ids = self.tables.tag_ids
+        rec, off = [], [0]
+        for i, (sent, items) in enumerate(zip(sents, constraints)):
+            n_syl = len(sent.replace(' ', ''))
+            prev_b, prev_e = -1, 0
+            for k, item in enumerate(items or ()):
+                where = 'sentence %d, constraint %d' % (i, k)
+                if not isinstance(item, (tuple, list)) or len(item) not in (2, 3):
+                    raise ValueError('%s: %r is not (b, e) or (b, e, tag)' % (where, item))
+                b, e = item[0], item[1]
+                tag = item[2] if len(item) == 3 else None
+                if not all(isinstance(x, int) and not isinstance(x, bool) for x in (b, e)):
+                    raise ValueError('%s: b and e must be integers, got %r' % (where, item))
+                if not 0 <= b < e:
+                    raise ValueError('%s: needs 0 <= b < e, got (%d, %d)' % (where, b, e))
+                if e - b > _native.LT_WINDOW:
+                    raise ValueError('%s: span (%d, %d) is longer than the %d-syllable window' % (where, b, e, _native.LT_WINDOW))
+                if e > n_syl:
+                    raise ValueError('%s: span (%d, %d) ends beyond the sentence\'s %d syllables' % (where, b, e, n_syl))
+                if b < prev_b:
+                    raise ValueError('%s: constraints must be sorted by b' % where)
+                if b < prev_e:
+                    raise ValueError('%s: span (%d, %d) overlaps the previous one' % (where, b, e))
+                if tag is None:
+                    tag_id = _native.LT_NO_TAG
+                elif tag in (BOS, EOS, Unk):
+                    raise ValueError('%s: %r is not a tag a constraint can ask for' % (where, tag))
+                elif tag not in tag_ids:
+                    raise ValueError('%s: tag %r is unknown to the compiled tables' % (where, tag))
+                else:
+                    tag_id = tag_ids[tag]
+                rec.append((b, e, tag_id, (0, 0, 0)))
+                prev_b, prev_e = b, e
+            off.append(len(rec))
+        cons = np.array(rec, dtype=_native.CONSTRAINT_DTYPE) if rec else np.zeros(1, dtype=_native.CONSTRAINT_DTYPE)
+        return cons, np.array(off, dtype=np.int64)
+
+    @contextlib.contextmanager
+    def constrained(self, sents, constraints):
+        """Within the block the batch's searches keep `constraints` (see `pack_constraints`; `None`: no binding):
+        the set is validated, uploaded and bound here, and unbound and freed on the way out.  Fetch the results
+        inside the block."""
+        if constraints is None:
+            yield
+            return
+        cons, off = self.pack_constraints(sents, constraints)
+        handle = ctypes.c_void_p()
+        _native.check(self._lib.lt_constraints_create(self.tables.handle, len(sents), _native.ptr(cons), _native.ptr(off),
+                                                      ctypes.byref(handle)))
+        try:
+            _native.check(self._lib.lt_batch_set_constraints(self.batch, handle))
+            try:
+                yield
+            finally:
+                self._lib.lt_batch_set_constraints(self.batch, None)
+        finally:
+            self._lib.lt_constraints_destroy(handle)
+
     # -- tagging -----------------------------------------------------------------------------------
-    def tag_packed(self, sents, beam_size):
-        """The C-ABI call alone: (path_off, path_edges, scores, status) numpy arrays."""
+    def tag_packed(self, sents, beam_size, constraints=None):
+        """The C-ABI call alone: (path_off, path_edges, scores, status) numpy arrays.  `constraints`: see
+        `pack_constraints`."""
         if not 1 <= beam_size <= _native.LT_MAX_BEAM:
             raise ValueError('beam_size must be in 1..%d' % _native.LT_MAX_BEAM)
         unsupported = []
@@ -151,35 +221,38 @@ class Engine:
         path_edges = np.empty(cap, dtype=_native.EDGE_DTYPE)
         scores = np.zeros(max(1, n), dtype=np.float64)
         status = np.zeros(max(1, n), dtype=np.int32)
-        _native.check(self._lib.lt_tag_batch_host(
-            self.batch, _native.ptr(text), _native.ptr(offsets), n, int(beam_size),
-            _native.ptr(path_off), _native.ptr(path_edges), cap, _native.ptr(scores), _native.ptr(status)))
+        with self.constrained(sents, constraints):
+            _native.check(self._lib.lt_tag_batch_host(
+                self.batch, _native.ptr(text), _native.ptr(offsets), n, int(beam_size),
+                _native.ptr(path_off), _native.ptr(path_edges), cap, _native.ptr(scores), _native.ptr(status)))
         for i in unsupported:
             status[i] = _native.LT_SENT_UNSUPPORTED_CHAR
         return path_off, path_edges[:int(path_off[n])], scores[:n], status[:n]
 
-    def kbest_packed(self, sents, beam_size, imported=None):
+    def kbest_packed(self, sents, beam_size, imported=None, constraints=None):
         """All survivors: (n_best, path_off, path_edges, scores, status); `path_off` / `scores` are
-        indexed by sentence * beam_size + rank.  With `imported` the lattice is the caller's."""
+        indexed by sentence * beam_size + rank.  With `imported` the lattice is the caller's.
+        `constraints`: see `pack_constraints`."""
         if not 1 <= beam_size <= _native.LT_MAX_BEAM:
             raise ValueError('beam_size must be in 1..%d' % _native.LT_MAX_BEAM)
         n = len(sents)
         unsupported = []
-        if imported is None:
-            text, offsets = pack_sentences(sents, unsupported)
-            _native.check(self._lib.lt_tag_batch_host_kbest(self.batch, _native.ptr(text), _native.ptr(offsets), n, int(beam_size)))
-        else:
-            self.import_lattice(sents, imported)
-            _native.check(self._lib.lt_beam_kbest(self.batch, int(beam_size), None))
-        total = ctypes.c_int64()
-        _native.check(self._lib.lt_kbest_size(self.batch, ctypes.byref(total)))
-        n_best = np.zeros(max(1, n), dtype=np.int32)
-        path_off = np.zeros(n * beam_size + 1, dtype=np.int32)
-        path_edges = np.empty(max(1, total.value), dtype=_native.EDGE_DTYPE)
-        scores = np.zeros(max(1, n * beam_size), dtype=np.float64)
-        status = np.zeros(max(1, n), dtype=np.int32)
-        _native.check(self._lib.lt_kbest_fetch(self.batch, _native.ptr(n_best), _native.ptr(path_off), _native.ptr(path_edges),
-                                               path_edges.size, _native.ptr(scores), _native.ptr(status)))
+        with self.constrained(sents, constraints):
+            if imported is None:
+                text, offsets = pack_sentences(sents, unsupported)
+                _native.check(self._lib.lt_tag_batch_host_kbest(self.batch, _native.ptr(text), _native.ptr(offsets), n, int(beam_size)))
+            else:
+                self.import_lattice(sents, imported)
+                _native.check(self._lib.lt_beam_kbest(self.batch, int(beam_size), None))
+            total = ctypes.c_int64()
+            _native.check(self._lib.lt_kbest_size(self.batch, ctypes.byref(total)))
+            n_best = np.zeros(max(1, n), dtype=np.int32)
+            path_off = np.zeros(n * beam_size + 1, dtype=np.int32)
+            path_edges = np.empty(max(1, total.value), dtype=_native.EDGE_DTYPE)
+            scores = np.zeros(max(1, n * beam_size), dtype=np.float64)
+            status = np.zeros(max(1, n), dtype=np.int32)
+            _native.check(self._lib.lt_kbest_fetch(self.batch, _native.ptr(n_best), _native.ptr(path_off), _native.ptr(path_edges),
+                                                   path_edges.size, _native.ptr(scores), _native.ptr(status)))
         for i in unsupported:
             status[i] = _native.LT_SENT_UNSUPPORTED_CHAR
             n_best[i] = 0

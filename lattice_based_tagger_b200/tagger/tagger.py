@@ -122,13 +122,16 @@ class Tagger:
         return self._engine.tables
 
     # -- the reference's API ---------------------------------------------------------------------------
-    def tag(self, sent, beam_size=5, ensure_normalize=True, debug=False):
+    def tag(self, sent, beam_size=5, ensure_normalize=True, debug=False, constraints=None):
+        """`constraints`: this sentence's list for `tag_batch`'s `constraints=`."""
         if debug:
+            if constraints is not None:
+                raise ValueError('tag(debug=True) does not support constraints')
             self.trace(sent, beam_size)
-        return self.tag_batch([sent], beam_size=beam_size)[0]
+        return self.tag_batch([sent], beam_size=beam_size, constraints=None if constraints is None else [constraints])[0]
 
     # -- batched API -----------------------------------------------------------------------------------
-    def tag_batch(self, sents, beam_size=5, errors='raise', lazy=True):
+    def tag_batch(self, sents, beam_size=5, errors='raise', lazy=True, constraints=None):
         """Tag many sentences in one device pass; returns one `Sequence` per sentence.
 
         A sentence the reference cannot tag — no dictionary edge at all, `IndexError` there
@@ -137,14 +140,23 @@ class Tagger:
         other than U+0020, characters outside the BMP, sentences beyond the device limit:
         `ValueError`).  The result is a `PackedSequences`: a list whose `Sequence` / `Word` objects
         are built when an item is read (`lazy=False`: a plain list, all built at once).
+
+        `constraints`: one list per sentence (`None` or `[]`: none) of `(b, e)` or `(b, e, tag_name)` spans,
+        syllable offsets in the space-stripped sentence, sorted and not overlapping, at most 8 syllables each.  The
+        search keeps each span as one word — a lattice word of that tag, or of any tag for `(b, e)`; where the
+        lattice has none, an unknown word for `(b, e)` and the word `Word(surface, surface, None, tag, None, e - b,
+        b, e, is_l)` for a tag — and no word crosses a span's boundary (DESIGN.md, "Constrained search").  A
+        malformed list raises `ValueError` before anything runs.
         """
         if self.score_funcs is None:
             raise TypeError("'NoneType' object is not callable")      # what beam.py:47 raises
         sents = list(sents)
         if self.eojeol_lookup.flatten:
+            if constraints is not None:
+                raise ValueError('constraints are not supported with a flatten=True lookup')
             best = [None if s is None else s[0] for s in self._kbest_flattened(sents, beam_size, errors)]
             return best
-        packed = self._engine.tag_packed(sents, beam_size)
+        packed = self._engine.tag_packed(sents, beam_size, constraints)
         if errors == 'raise':
             status = packed[3]
             if status.any():
@@ -154,19 +166,23 @@ class Tagger:
             return self._engine.unpack(sents, packed, errors)
         return PackedSequences(self._engine, sents, packed, errors)
 
-    def tag_batch_packed(self, sents, beam_size=5):
+    def tag_batch_packed(self, sents, beam_size=5, constraints=None):
         """The C-ABI call alone: returns (path_off, path_edges, scores, status) numpy arrays."""
-        return self._engine.tag_packed(list(sents), beam_size)
+        if constraints is not None and self.eojeol_lookup.flatten:
+            raise ValueError('constraints are not supported with a flatten=True lookup')
+        return self._engine.tag_packed(list(sents), beam_size, constraints)
 
-    def tag_batch_kbest(self, sents, beam_size=5, errors='raise'):
+    def tag_batch_kbest(self, sents, beam_size=5, errors='raise', constraints=None):
         """Every survivor of the beam per sentence, best first — what the reference's `beam_search`
         returns (`beam/beam.py:59-61`); `tag_batch(...)[i]` is `tag_batch_kbest(...)[i][0]`."""
         if self.score_funcs is None:
             raise TypeError("'NoneType' object is not callable")
         sents = list(sents)
         if self.eojeol_lookup.flatten:
+            if constraints is not None:
+                raise ValueError('constraints are not supported with a flatten=True lookup')
             return self._kbest_flattened(sents, beam_size, errors)
-        packed = self._engine.kbest_packed(sents, beam_size)
+        packed = self._engine.kbest_packed(sents, beam_size, constraints=constraints)
         return self._engine.unpack_kbest(sents, packed, beam_size, errors)
 
     def _kbest_flattened(self, sents, beam_size, errors):
