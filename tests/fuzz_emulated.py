@@ -4,7 +4,9 @@ lattice, best path, fp64 score and work counters compared bit for bit through th
 the beam sizes, sentence lengths, k-best survivors and lookup modes rotating over the seeds.  Every seed
 also scores and featurizes random tilings of its sentences and runs the perceptron step against gold
 paths that include near misses (tests/test_gpu_path_edges.py, `check_path_stage`); the 110- and
-200-syllable sentences give paths of more than one 32-word chunk.
+200-syllable sentences give paths of more than one 32-word chunk.  Every odd seed also runs the constrained
+search (tests/test_gpu_constraint_edges.py, `pattern_constraints`) with its beam sizes against the constrained
+oracle, survivor for survivor.
 
     python tests/fuzz_emulated.py FIRST_SEED LAST_SEED        # prints `ok SEED` / `FAIL SEED` + traceback
     python tests/fuzz_emulated.py FIRST_SEED LAST_SEED knobs  # + the library's debugging knobs rotating over the seeds
@@ -15,6 +17,7 @@ last to first).  LT_SIMT_MEMCHECK=1 in the environment adds the emulator's guard
 """
 
 import os
+import random
 import sys
 import traceback
 
@@ -23,6 +26,9 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import lattice_based_tagger_b200 as pkg                      # noqa: E402
 from oracle import lattice_oracle as lo                      # noqa: E402
 from tests import _cases, _checks, _emu                      # noqa: E402
+from tests import _constrained_oracle as co                  # noqa: E402
+from tests import test_gpu_constraint_edges as constraint_edges  # noqa: E402
+from tests import test_gpu_constraints as constraints        # noqa: E402
 from tests import test_gpu_path_edges as path_edges          # noqa: E402
 
 BEAMS = [(1, 5), (2, 10), (3, 33), (7, 64), (16, 40)]
@@ -53,8 +59,25 @@ def run_seed(seed, knobs=False):
     if seed % 3 == 0:
         _checks.check_kbest(tagger, oracle, case['sentences'], (beams[0], 5))
     path_edges.check_path_stage(case, funcs, tagger, seed, beams[0])
+    if seed % 2:
+        check_constrained(case, tagger, oracle, seed, beams)
     if seed % 7 == 0:
         _checks.check_lookup_modes(case)
+
+
+def check_constrained(case, tagger, oracle, seed, beams):
+    """The constrained search against the constrained oracle: random constraints, every span constrained back to
+    back, and 8-syllable constraints end to end, rotating over the sentences."""
+    rng = random.Random(seed ^ 0xC0)
+    cons = []
+    for i, sent in enumerate(case['sentences']):
+        try:
+            survivor = rng.choice(co.survivors(oracle, sent, 5, [])).words[1:-1]
+        except IndexError:
+            survivor = None
+        kind = ('random', 'back_to_back', 'eight')[i % 3]
+        cons.append(constraint_edges.pattern_constraints(kind, rng, sent, oracle.lattice(sent), case['tags'], survivor))
+    constraints.check_parity(tagger, oracle, case['sentences'], cons, beams)
 
 
 def main(first, last, knobs=False):

@@ -176,6 +176,51 @@ def test_path_kernels(monkeypatch, block_order):
     path_edges.check_after_search('rerun')
 
 
+@pytest.mark.parametrize('block_order', ['forward', 'reverse'])
+def test_constrained_search_across_ctas(monkeypatch, block_order):
+    """The constrained search over a few hundred sentences of mixed statuses on an emulated device of 2 SMs: the
+    constraint preparation and the beam grids take their stride, with the CTAs run in both orders."""
+    import random
+    from lattice_based_tagger_b200 import _native
+    from tests import _constrained_oracle as co
+    from tests.test_gpu_constraint_edges import PATTERNS, pattern_constraints
+    from tests.test_gpu_constraints import _as_items
+    monkeypatch.setenv('LT_SIMT_BLOCK_ORDER', block_order)
+    monkeypatch.setenv('LT_SIMT_SMS', '2')
+    case = _checks.make_case(5400, n_sent=14, max_sent_len=60)
+    dictionary, funcs = _cases.build_objects(case, pkg)
+    tagger = pkg.Tagger(dictionary, score_funcs=funcs)
+    oracle = lo.OracleTagger(dictionary, funcs)
+    bad = ['\U0001F600가', '가\t나', 'x' * (tagger.info()['unit_limit'] + 1)]
+    pool = case['sentences'] + bad
+    sents = [pool[i % len(pool)] for i in range(320)]
+    memo, cons = {}, []
+    for i, sent in enumerate(sents):
+        key = (sent, PATTERNS[i % len(PATTERNS)])
+        if key not in memo:
+            memo[key] = pattern_constraints(key[1], random.Random(i), sent, oracle.lattice(sent), case['tags'])
+        cons.append(memo[key])
+    got = tagger.tag_batch_kbest(sents, 5, errors='none', constraints=[_as_items(c) for c in cons])
+    status = tagger.tag_batch_packed(sents, 5, constraints=[_as_items(c) for c in cons])[3]
+    assert {_native.LT_SENT_UNSUPPORTED_CHAR, _native.LT_SENT_BAD_SPACE, _native.LT_SENT_TOO_LONG,
+            _native.LT_SENT_NO_EDGES} <= set(status.tolist())
+    want = {}
+    for sent, c, seqs in zip(sents, cons, got):
+        if sent in bad:
+            assert seqs is None
+            continue
+        key = (sent, tuple(c))
+        if key not in want:
+            try:
+                want[key] = [(h.words, h.score) for h in co.survivors(oracle, sent, 5, c)]
+            except IndexError:
+                want[key] = None
+        if want[key] is None:
+            assert seqs is None, sent
+        else:
+            assert [([tuple(w) for w in s.sequences], s.score) for s in seqs] == want[key], (sent, c)
+
+
 def test_memcheck_self_test(tmp_path):
     """LT_SIMT_MEMCHECK=1 places device buffers and a launch's dynamic shared memory against guard pages: the
     emulator's own check that an access one element past either is caught (and that a clean kernel is not)."""
